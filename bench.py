@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- SATYR p-d-p hot path on B200: SP edge-updates/s (+ CNFs solved/s), % of HBM roofline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[3], the configuration the metric is quoted on at 1/2/4/8 B200): the
@@ -22,6 +22,9 @@ WalkSAT, solution merge.  Weak scaling: every rank owns its own problems, no dat
            bounded sample of the workload (one smaller problem, few iterations; set-up, loop and WalkSAT timed
            separately and the whole-step figure rebuilt for the workload's T and W).  The C oracle port is the
            fallback when the reference tree is absent (`kind: "port"`).
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what the last step of the `value` leg returned to its caller
+           (prediction, solved, unsat_clauses) as DIR/<name>.npy.  The inputs are a function of the arguments (seeded
+           generator, seeded WalkSAT draws), so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -37,6 +40,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 ALG_BYTES_PER_EDGE_UPDATE = 20.0   # SURVEY.md section 8d: q_u r + eta r + index r + eta' w + q_u' w
+DUMP_BYTES = 60 * 10 ** 6          # --dump-outputs: array bytes in all, under 64 MB with the .npy headers
 
 
 def parse():
@@ -65,7 +69,23 @@ def parse():
     ap.add_argument("--cpu-port", action="store_true", help="time the C oracle port even when the reference is present")
     ap.add_argument("--strong-problems", type=int, default=64, help="problems of the fixed batch of the strong-scaling line (0: skip it)")
     ap.add_argument("--strong-n", type=int, default=0, help="variables per problem of that batch (0: --n)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="B200 arm: write the outputs of the last timed step as DIR/<name>.npy (an output too large for the "
+                         "%d-byte budget is replaced by a fixed, seeded sample of its elements)" % DUMP_BYTES)
     return ap.parse_args()
+
+
+def dump_outputs(out_dir, outputs):
+    """outputs: name -> 1-D float32 / float64 numpy array.  Smallest first, each is written whole while it fits in what is
+    left of DUMP_BYTES; one that does not is cut to the elements at sorted indices drawn by numpy's default_rng(0)."""
+    os.makedirs(out_dir, exist_ok=True)
+    room = DUMP_BYTES
+    for name, x in sorted(outputs.items(), key=lambda kv: kv[1].nbytes):
+        keep = room // x.itemsize
+        if x.size > keep:
+            x = x[np.sort(np.random.default_rng(0).choice(x.size, keep, replace=False))]
+        room -= x.nbytes
+        np.save(os.path.join(out_dir, name + ".npy"), x)
 
 
 def config_of(a):
@@ -289,7 +309,7 @@ def run_b200_arm(a, rank, world, local_rank):
                              edge_feature=ef, meta_data=None, is_training=False, iteration_num=a.iterations,
                              check_termination=termination, batch_replication=1)
         ctx = model.last_problem._ctx
-        solved, _ = ctx.cnf_eval(pred)
+        solved, n_unsat = ctx.cnf_eval(pred)
         if from_host:      # the step's result back to (pinned) host memory, then wait for it
             out_h["pred"].copy_(pred.reshape(-1), non_blocking=True)
             out_h["solved"].copy_(solved.reshape(-1), non_blocking=True)
@@ -307,7 +327,7 @@ def run_b200_arm(a, rank, world, local_rank):
                 stats["loop_ms"] += t.get("sp_run", 0.0)
                 stats["ws_ms"] += t.get("walksat", 0.0)
                 stats["loop_updates"] += upd
-        return pred
+        return {"prediction": pred, "solved": solved, "unsat_clauses": n_unsat}
 
     copy_stream = torch.cuda.Stream(dev)
 
@@ -370,10 +390,12 @@ def run_b200_arm(a, rank, world, local_rank):
                 st.release(i)
         else:
             for _ in range(a.steps):
-                one_step(tensors, False, True)
+                last = one_step(tensors, False, True)
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1)
+        if a.dump_outputs and not from_host and rank == 0:
+            outputs.update({k: v.reshape(-1).cpu().numpy() for k, v in last.items()})
         copy_ms = st.copy_ms() if from_host else 0.0
         if world > 1:
             t = torch.tensor([ms, copy_ms], device=dev, dtype=torch.float64)
@@ -391,9 +413,12 @@ def run_b200_arm(a, rank, world, local_rank):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
+    outputs = {}
     ms, upd, solved, launches, st = timed_region(resident, False)
     ms_e, upd_e, solved_e, _, st_e = timed_region(host, True)
     sampler.stop_flag = True
+    if outputs:
+        dump_outputs(a.dump_outputs, outputs)
 
     strong = None
     if a.strong_problems > 0:
@@ -596,7 +621,7 @@ def run_other_workload(a, rank, world, local_rank):
     spec = other_workload(a)
     if a.impl == "reference":
         if rank == 0:
-            print(json.dumps(other_reference_line(a, spec)))
+            print(json.dumps(other_reference_line(a, spec, a.steps, min(a.warmup, 1))))
         return
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
@@ -620,8 +645,10 @@ def run_other_workload(a, rank, world, local_rank):
                                  meta_data=None, is_training=False, iteration_num=spec["T"], check_termination=termination,
                                  batch_replication=rep)
         from pdp_solver_b200.nn.util import cnf_eval_edges
-        solved, _ = cnf_eval_edges(pred, gm, bvm, bfm, ef, batch_size=B)
-        return pred, solved
+        solved, n_unsat = cnf_eval_edges(pred, gm, bvm, bfm, ef, batch_size=B)
+        return pred, solved, n_unsat
+
+    outputs = {}
 
     def measure(rep, from_host):
         tot = {"solved": 0.0, "updates": 0.0}
@@ -629,12 +656,13 @@ def run_other_workload(a, rank, world, local_rank):
         def step(timed):
             torch.manual_seed(1 + rank)
             tens = [t.to(dev, non_blocking=True) for t in host] if from_host else resident
-            pred, solved = forward(tens, rep)
+            pred, solved, n_unsat = forward(tens, rep)
             if from_host:
                 pred.cpu(); solved.cpu()
             if timed:
                 tot["solved"] += float((solved > 0.5).sum().item())
                 tot["updates"] += float(E) * rep * float(model.last_iterations.reshape(-1)[0].item())
+            return {"prediction": pred, "solved": solved, "unsat_clauses": n_unsat}
         for _ in range(a.warmup):
             step(False)
         torch.cuda.synchronize()
@@ -643,10 +671,12 @@ def run_other_workload(a, rank, world, local_rank):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(a.steps):
-            step(True)
+            last = step(True)
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1)
+        if a.dump_outputs and not from_host and rep == spec["reps"][0] and rank == 0:
+            outputs.update({k: v.reshape(-1).cpu().numpy() for k, v in last.items()})
         if world > 1:
             t = torch.tensor([ms], device=dev, dtype=torch.float64)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -668,6 +698,8 @@ def run_other_workload(a, rank, world, local_rank):
                       "e2e_ms_per_step": ms_e / a.steps, "cnfs_solved_per_step": tot["solved"] / a.steps,
                       "cnfs_per_s": world * B * a.steps / (ms / 1e3), "edge_updates_per_s": tot["updates"] / (ms / 1e3)})
     sampler.stop_flag = True
+    if outputs:
+        dump_outputs(a.dump_outputs, outputs)
     if rank == 0:
         head = sweep[0]
         h2d = sum(int(t.numel() * t.element_size()) for t in host)
@@ -689,30 +721,49 @@ def run_other_workload(a, rank, world, local_rank):
         dist.destroy_process_group()
 
 
-def other_reference_line(a, spec):
-    """the reference's CPU path on a bounded sample of the workload (same model type, fewer / smaller problems, fewer iterations)"""
+def other_reference_line(a, spec, steps=1, warmup=0):
+    """the reference's CPU path on a bounded sample of the workload (same model type, fewer / smaller problems, fewer iterations),
+    `steps` timed forwards after `warmup` untimed ones.  Without the reference tree the C oracle port stands in for p-d-p, as
+    in run_reference_arm; the neural model types have no port."""
     import torch
     from oracle import ref_timing
     from pdp_solver_b200 import cnfgen
     c = spec["cpu"]
-    if not ref_timing.available():
+    if ref_timing.available():
+        kind, what = "reference", "the unmodified reference with use_cuda=False"
+        cores = ref_timing.pin_threads()
+        model = ref_timing.build_model(spec["model"], torch.device("cpu"), c["W"], a.epsilon, a.tolerance, a.t_max)
+    elif spec["model"] == "p-d-p":
+        from oracle import pdp_oracle as po
+        kind, what = "port", "the C oracle port"
+        po.build()
+        po.set_num_threads(os.cpu_count() or 1)
+        cores = po.num_threads()
+    else:
         cb = {"unavailable": "reference tree absent (baseline/_ref)"}
         return {"impl": "reference", "metric": spec["metric"], "unit": spec["unit"], "cpu_baseline": cb}
-    cores = ref_timing.pin_threads()
-    model = ref_timing.build_model(spec["model"], torch.device("cpu"), c["W"], a.epsilon, a.tolerance, a.t_max)
     batch = cnfgen.random_batch(c["B"], c["n"], c["k"], c["alpha"], a.seed + 999)
-    r = ref_timing.timed_forward(model, batch, c["T"], torch.device("cpu"), seed=a.seed)
+
+    def forward():
+        if kind == "reference":
+            return ref_timing.timed_forward(model, batch, c["T"], torch.device("cpu"), seed=a.seed)
+        return port_forward(batch, c["T"], c["W"], a.tolerance, a.t_max, a.epsilon, a.seed)
+    for _ in range(warmup):
+        forward()
+    runs = [forward() for _ in range(steps)]
+    r = {k: sum(x[k] for x in runs) for k in ("total_s", "loop_s", "setup_s", "iterations", "solved")}
+    r["edges"] = runs[0]["edges"]
     if spec["metric"] == "cnfs_solved_per_s":
         value = r["solved"] / r["total_s"]
     else:
         value = r["edges"] * max(r["iterations"], 1) / r["total_s"]
-    cb = {"value": value, "unit": spec["unit"], "cores": cores, "kind": "reference",
-          "sample": "%d problems of random %d-SAT n=%d m/n=%.2f, T=%d, %d WalkSAT iterations: one forward of the unmodified reference with use_cuda=False, %.2f s (%d iterations executed, %d solved)"
-                    % (c["B"], c["k"], c["n"], c["alpha"], c["T"], c["W"], r["total_s"], r["iterations"], r["solved"]),
-          "s_per_iteration": r["loop_s"] / max(r["iterations"], 1), "setup_s": r["setup_s"],
-          "cnfs_per_s": c["B"] / r["total_s"], "edge_updates_per_s": r["edges"] * max(r["iterations"], 1) / r["total_s"]}
-    return {"impl": "reference", "metric": spec["metric"], "value": value, "unit": spec["unit"], "n_gpus": a.gpus, "steps": 1, "warmup": 0,
-            "ms_per_step": 1e3 * r["total_s"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
+    cb = {"value": value, "unit": spec["unit"], "cores": cores, "kind": kind,
+          "sample": "%d problems of random %d-SAT n=%d m/n=%.2f, T=%d, %d WalkSAT iterations: %d forward(s) of %s, %.2f s (%d iterations executed, %d solved)"
+                    % (c["B"], c["k"], c["n"], c["alpha"], c["T"], c["W"], steps, what, r["total_s"], r["iterations"], r["solved"]),
+          "s_per_iteration": r["loop_s"] / max(r["iterations"], 1), "setup_s": r["setup_s"] / steps,
+          "cnfs_per_s": c["B"] * steps / r["total_s"], "edge_updates_per_s": r["edges"] * max(r["iterations"], 1) / r["total_s"]}
+    return {"impl": "reference", "metric": spec["metric"], "value": value, "unit": spec["unit"], "n_gpus": a.gpus, "steps": steps, "warmup": warmup,
+            "ms_per_step": 1e3 * r["total_s"] / steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": spec["name"], "model_type": spec["model"]}, "cpu_baseline": cb,
             "e2e": {"value": value, "unit": spec["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}, "gpu_launches": 0}
 
