@@ -184,6 +184,24 @@ typedef struct {
  * Can be called repeatedly; module state (previous surveys, counters) persists until pdp_reset. */
 int pdp_sp_run(pdp_ctx* ctx, const pdp_sp_params* params, int32_t* d_iters_done, void* stream);
 
+/* SP-inspired decimation (Braunstein, Mezard, Zecchina, Random Structures & Algorithms 27, 2005), generalising the rule of
+ * SequentialDecimator (reference pdp/nn/pdp_decimate.py:152-171, one arg-max variable per problem and step).  With a
+ * fraction f in [0, 1), a problem b selected at a step (converged, active, no NaN coefficient, sum of coefficients > 0)
+ * with A_b active variables takes K_b = max(1, floor((double)f * A_b)) variables:
+ *   K_b == 1: the reference's arg-max rule (first index attaining the max of fl(fl(c - min) + 1));
+ *   K_b >= 2: the first min(K_b, #candidates) of the active variables with c > 0, ordered by c descending, then index
+ *             ascending (exact fp32 comparisons); each gets sign(score).
+ * All variables of a step are fixed together (_set_variable_core, solver.py:205-226), then unit propagation and peeling run.
+ * pdp_set_decimation_fraction: the fraction pdp_sp_run uses; 0 after pdp_create (the reference's rule), kept by pdp_reset;
+ *   PDP_ERR_ARG unless 0 <= f < 1.
+ * pdp_decimation_select: the same rule, stateless, on caller-supplied coefficients d_coeff [V] (>= 0; |score| * active *
+ *   converged in the reference) and scores d_score [V]; d_problem_sel uint8 [B] (NULL = every problem) stands for
+ *   "converged and active"; A_b counts the context's active variables.  d_assignment [V] receives sign(score) on the taken
+ *   variables and 0 elsewhere.  Uses the context's per-step scratch: not concurrently with pdp_sp_run on the context. */
+int pdp_set_decimation_fraction(pdp_ctx* ctx, float fraction);
+int pdp_decimation_select(pdp_ctx* ctx, const float* d_coeff, const float* d_score, const uint8_t* d_problem_sel,
+                          float fraction, float* d_assignment, void* stream);
+
 /* IdentityPredictor.forward(last_call=True), reference pdp/nn/pdp_predict.py:118-128.
  * pdp_count_active_variables syncs the stream.  d_draws holds >= n_active uniform draws that are
  * consumed by the active variables in batch-global variable order (like torch.rand(n_active)). */

@@ -60,6 +60,8 @@ SIGNATURES = {
     "pdp_random_fill": (ctypes.c_int, [P, P, P]),
     "pdp_walksat": (ctypes.c_int, [P, I32, F32, I32, P, P, U64, P, P, P]),
     "pdp_deduplicate": (ctypes.c_int, [P, I32, P, P, P, P]),
+    "pdp_set_decimation_fraction": (ctypes.c_int, [P, F32]),
+    "pdp_decimation_select": (ctypes.c_int, [P, P, P, P, F32, P, P]),
     "pdp_set_trace_buffer": (ctypes.c_int, [P, P, I32]),
     "pdp_trace_length": (ctypes.c_int, [P, ctypes.POINTER(I32), P]),
     "pdp_debug_check_layout": (ctypes.c_int, [P, P, ctypes.POINTER(I32 * 5), P]),

@@ -28,6 +28,7 @@ struct KArgs {
     int32_t* trace;      // optional decimation trace: triples (iteration, variable, sign)
     int32_t trace_cap;
     int32_t stagger_c, stagger_v;   // cycles the second CTA of an SM waits at the start of a clause / variable pass
+    float dec_fraction;             // pdp_set_decimation_fraction (0: the arg-max rule only)
 };
 
 __device__ __forceinline__ int lane_id() { return threadIdx.x & 31; }
@@ -447,8 +448,20 @@ __device__ __forceinline__ void score_phase(const KArgs& A, int w, float pi) {
     red.finish(s);
 }
 
+// decimation coefficient c_i = |score_i| * active_i of the fused loop (pdp_decimate.py:153)
+struct CoefScore {
+    const pdp_state& s;
+    __device__ __forceinline__ float operator()(int64_t i) const { return fabsf(s.score[i]) * (float)s.av[i]; }
+};
+// coefficients handed in by the caller (pdp_decimation_select)
+struct CoefGiven {
+    const float* c;
+    __device__ __forceinline__ float operator()(int64_t i) const { return c[i]; }
+};
+
 // first index attaining max of fl(fl(c - min) + 1)  (util.py:257-265)
-__device__ __forceinline__ void argmax_phase(const KArgs& A) {
+template <typename CF>
+__device__ __forceinline__ void argmax_phase(const KArgs& A, const CF& coef) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
     if (range_scans(g)) {
         for (int b = 0; b < (int)g.B; ++b) {
@@ -458,7 +471,7 @@ __device__ __forceinline__ void argmax_phase(const KArgs& A) {
             const int v1 = g.prob_vptr[b + 1];
 #pragma unroll 4
             for (int i = g.prob_vptr[b] + (int)gtid(); i < v1; i += (int)gthreads()) {
-                const float c = fabsf(s.score[i]) * (float)s.av[i];
+                const float c = coef(i);
                 if (argmax_key(c, m) == kmax) atomicMin(&s.arg_idx[b], i);
             }
         }
@@ -470,7 +483,7 @@ __device__ __forceinline__ void argmax_phase(const KArgs& A) {
         if (!s.conv[b] || s.c_nan[b]) continue;
         const float m = u2f(s.c_min[b]);
         const float kmax = argmax_key(u2f(s.c_max[b]), m);
-        const float c = fabsf(s.score[i]) * (float)s.av[i];
+        const float c = coef(i);
         if (argmax_key(c, m) == kmax) atomicMin(&s.arg_idx[b], (int)i);
     }
 }
@@ -698,6 +711,142 @@ __device__ __forceinline__ void warp_fix_variable(const pdp_graph& g, const pdp_
         mask_edge(g, g.p_vpos[p], g.p_qpos[p]);
     }
     if (lane_id() == 0) { s.av[i] = 0; s.sol[i] = (sg + 1.f) / 2.0f; }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Fractional decimation (SP-inspired decimation, Braunstein, Mezard, Zecchina 2005): the rule of pdp_decimate.py:152-171
+// fixes the arg-max variable of every selected problem; with a fraction f > 0 a problem b with A_b active variables takes
+// K_b = max(1, floor(f * A_b)) variables per step.  K_b == 1 keeps the arg-max rule above unchanged.  K_b >= 2 takes the
+// first min(K_b, #candidates) active variables with c > 0 ordered by c descending, then index ascending: a per-problem
+// radix select, 8 bits per pass from the top, on the unique 64-bit key (float bits of c) << 32 | (0xFFFFFFFF - index)
+// (c >= 0: its bits order like unsigned integers).  A pass stops refining a problem as soon as the bucket holding the K-th
+// key is taken whole; the rule that remains is (key >> sel_sh) >= sel_pref.
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ unsigned long long sel_key(float c, int64_t i) {
+    return ((unsigned long long)__float_as_uint(c) << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)i);
+}
+// K_b in double from the fp32 fraction
+__device__ __forceinline__ int sel_k(float f, int nav) {
+    const double k = floor((double)f * (double)nav);
+    return k < 1.0 ? 1 : (int)k;
+}
+// warp-aggregated histogram increment (all 32 lanes call it): lanes hitting the same bin add once
+__device__ __forceinline__ void sel_count(uint32_t* bin, bool pred) {
+    const unsigned long long a = pred ? (unsigned long long)(uintptr_t)bin : 0ull;
+    const unsigned m = __match_any_sync(0xffffffffu, a);
+    if (pred && lane_id() == __ffs(m) - 1) atomicAdd(bin, (uint32_t)__popc(m));
+}
+// histogram of one variable: `first` = pass 0 (every candidate, plus the active-variable count); otherwise candidates
+// whose key agrees with the bits fixed so far.  All lanes call it; `valid` = the variable belongs to a selecting problem.
+__device__ __forceinline__ void sel_hist_var(const pdp_state& s, bool valid, int b, int64_t i, float c, bool act, bool first) {
+    uint32_t* h = s.sel_hist + (size_t)(valid ? b : 0) * PDP_SEL_BINS;
+    const bool cand = valid && act && c > 0.f;
+    const unsigned long long key = sel_key(c, i);
+    int sh = 56;
+    bool in = cand;
+    if (!first && cand) { sh = s.sel_sh[b]; in = (key >> (sh + 8)) == s.sel_pref[b]; }
+    if (first) sel_count(h + 256, valid && act);
+    sel_count(h + (int)((key >> sh) & 255u), in);
+}
+// is variable i (coefficient c, active) taken by the final rule of its problem
+__device__ __forceinline__ bool sel_taken(const pdp_state& s, int b, int64_t i, float c, bool act) {
+    return act && c > 0.f && (sel_key(c, i) >> s.sel_sh[b]) >= s.sel_pref[b];
+}
+
+// one warp, after a histogram pass of problem b: picks the digit that holds the K-th key, clears the histogram, updates the
+// problem's state.  first: K_b from the active-variable count; a problem with K_b == 1 leaves (sel_need = -1) for the
+// arg-max rule.  Returns -1 (arg-max rule), 0 (final rule) or 1 (another pass), the same in every lane.
+__device__ __forceinline__ int sel_decide(const pdp_state& s, int b, float frac, bool first) {
+    uint32_t* h = s.sel_hist + (size_t)b * PDP_SEL_BINS;
+    const int lane = lane_id();
+    uint32_t v[8], tot = 0;
+#pragma unroll
+    for (int k = 0; k < 8; ++k) { v[k] = h[8 * lane + k]; tot += v[k]; }
+    int need, sh;
+    unsigned long long pref;
+    const int nav = first ? (int)h[256] : 0;
+    __syncwarp();
+#pragma unroll
+    for (int k = 0; k < 8; ++k) h[8 * lane + k] = 0u;
+    if (first && lane == 0) h[256] = 0u;
+    // inclusive suffix sums over the lanes: keys in bins >= 8 * lane
+    uint32_t suf = tot;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const uint32_t y = __shfl_down_sync(0xffffffffu, suf, o); if (lane + o < 32) suf += y; }
+    if (first) {
+        const int K = sel_k(frac, nav);
+        const uint32_t ncand = __shfl_sync(0xffffffffu, suf, 0);
+        if (K < 2) { if (lane == 0) s.sel_need[b] = -1; return -1; }
+        if (ncand <= (uint32_t)K) {   // every candidate is taken
+            if (lane == 0) { s.sel_need[b] = 0; s.sel_sh[b] = 0; s.sel_pref[b] = 0ull; }
+            return 0;
+        }
+        need = K; sh = 56; pref = 0ull;
+    } else {
+        need = s.sel_need[b]; sh = s.sel_sh[b]; pref = s.sel_pref[b];
+    }
+    // the lane whose bins hold the need-th key from the top, then the bin inside it
+    const uint32_t above_lane = suf - tot;
+    const bool mine = above_lane < (uint32_t)need && suf >= (uint32_t)need;
+    const int src = __ffs(__ballot_sync(0xffffffffu, mine)) - 1;
+    int d = 0; uint32_t above = 0, cnt = 0;
+    if (mine) {
+        uint32_t cum = above_lane;
+#pragma unroll
+        for (int k = 7; k >= 0; --k) {
+            if (cum + v[k] >= (uint32_t)need) { d = 8 * lane + k; above = cum; cnt = v[k]; break; }
+            cum += v[k];
+        }
+    }
+    d = __shfl_sync(0xffffffffu, d, src); above = __shfl_sync(0xffffffffu, above, src); cnt = __shfl_sync(0xffffffffu, cnt, src);
+    pref = (pref << 8) | (unsigned long long)d;
+    const bool done = cnt == (uint32_t)need - above;   // the bucket is taken whole (always true at shift 0: keys are unique)
+    if (lane == 0) {
+        s.sel_pref[b] = pref;
+        if (done) { s.sel_need[b] = 0; s.sel_sh[b] = sh; }
+        else { s.sel_need[b] = need - (int)above; s.sel_sh[b] = sh - 8; }
+    }
+    return done ? 0 : 1;
+}
+
+// Grid-wide selection over the problems the arg-max phase left selectable (conv, no NaN coefficient, max c > 0); called by
+// ALL threads after that phase and a barrier, returns after a barrier.  Problems with K_b >= 2 get arg_idx cleared (the
+// arg-max fix skips them) and their final rule in sel_need / sel_sh / sel_pref; every other problem gets sel_need = -1.
+// One histogram pass over the variables, then up to 7 more while some problem is undecided (CTRL_SEL parity slots).
+template <typename CF>
+__device__ __forceinline__ void sel_grid(const KArgs& A, cg::grid_group& grid, const CF& coef, float frac) {
+    const pdp_graph& g = A.g; const pdp_state& s = A.s;
+    for (int pass = 0; pass < 8; ++pass) {
+        if (pass > 0 && !s.ctrl[CTRL_SEL + (pass & 1)]) break;   // uniform: written before the last barrier
+        const bool first = pass == 0;
+        for (int64_t base = gwarp() * 32; base < g.V; base += gwarps() * 32) {
+            const int64_t i = base + lane_id();
+            int b = 0; bool valid = false;
+            if (i < g.V) {
+                b = g.bvm[i];
+                valid = first ? (s.conv[b] && !s.c_nan[b] && u2f(s.c_max[b]) > 0.f) : (s.sel_need[b] > 0);
+            }
+            const float c = valid ? coef(i) : 0.f;
+            sel_hist_var(s, valid, b, i, c, valid && s.av[i], first);
+        }
+        if (gtid() == 0) s.ctrl[CTRL_SEL + ((pass + 1) & 1)] = 0;
+        grid.sync();
+        for (int64_t b = gwarp(); b < g.B; b += gwarps()) {
+            int st = -1;
+            if (first) {
+                if (s.conv[b] && !s.c_nan[b] && u2f(s.c_max[b]) > 0.f) {
+                    st = sel_decide(s, (int)b, frac, true);
+                    if (st >= 0 && lane_id() == 0) s.arg_idx[b] = 0x7fffffff;
+                } else if (lane_id() == 0) {
+                    s.sel_need[b] = -1;
+                }
+            } else if (s.sel_need[b] > 0) {
+                st = sel_decide(s, (int)b, frac, false);
+            }
+            if (st > 0 && lane_id() == 0) s.ctrl[CTRL_SEL + ((pass + 1) & 1)] = 1;
+        }
+        grid.sync();
+    }
 }
 
 __device__ __forceinline__ void fr_find_units(const KArgs& A, int clist, int ulist, int flag_slot) {
@@ -959,7 +1108,88 @@ __device__ __forceinline__ void loc_closure(const KArgs& A, int b, int v0, int v
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// shared-memory tier of the CTA-local decimation.  A problem whose masks, adjacency (16-bit local indices) and
+// scratch fit the group's share of the (idle) sweep buffer is decimated entirely in shared memory: the closure
+// is a chain of dozens of dependent rounds, each a couple of microseconds through global memory and tens of
+// nanoseconds here.  Same rounds, same arithmetic as loc_closure; what changed is written back at the end.
+// ------------------------------------------------------------------------------------------------
+struct TinyView {
+    uint8_t *av, *af, *pure, *single;
+    float *sol, *score;
+    int *cnt, *ev;
+    uint16_t *clp, *cvar, *vp, *vcls;   // local CSR / CSC: pointers, (local index | sign << 15)
+};
+__device__ __forceinline__ size_t tiny_bytes(int n, int m, int E) {
+    return (size_t)n * (1 + 1 + 4 + 4 + 4 + 4) + (size_t)m * 2 + (size_t)(m + 1 + n + 1 + 2 * E) * 2 + 64;
+}
+__device__ __forceinline__ TinyView tiny_carve(unsigned char* base, int n, int m, int E) {
+    TinyView t;
+    float* f = reinterpret_cast<float*>(base);
+    t.sol = f; t.score = f + n;
+    t.cnt = reinterpret_cast<int*>(f + 2 * n); t.ev = t.cnt + n;
+    uint16_t* h = reinterpret_cast<uint16_t*>(t.ev + n);
+    t.clp = h; t.vp = t.clp + (m + 1); t.cvar = t.vp + (n + 1); t.vcls = t.cvar + E;
+    uint8_t* q = reinterpret_cast<uint8_t*>(t.vcls + E);
+    t.av = q; t.pure = q + n; t.af = q + 2 * n; t.single = t.af + m;
+    return t;
+}
+
+__device__ __forceinline__ void tiny_fix(const TinyView& t, int i, float sg) {
+    for (int p = t.vp[i]; p < t.vp[i + 1]; ++p) {
+        const uint32_t w = t.vcls[p];
+        const float lit = (w & 0x8000u) ? -1.f : 1.f;
+        if (lit * sg > 0.f) t.af[w & 0x7fffu] = 0;
+    }
+    t.av[i] = 0;
+    t.sol[i] = (sg + 1.f) / 2.0f;
+}
+
+// the fractional selection of one converged problem inside its CTA group (sel_grid's passes over the problem's own
+// variables, group barriers instead of grid barriers; the histograms stay in global memory: the kernel's shared memory is
+// the sweep buffer's).  Called by the whole group after the scoring loop with !cnan and max c > 0.  score / av: the
+// problem's variables (local index); TINY: fixes go to the shared-memory view.  Returns false for K_b == 1 (the caller
+// applies the arg-max rule); otherwise fixes the taken variables and sets ls.fixed.
+template <bool TINY>
+__device__ __forceinline__ bool loc_select_fix(const KArgs& A, int b, int iter, const float* score, const uint8_t* av, int v0, int n,
+                                            TinyView t, LocSmem& ls, int tid, int nthr, int bar_id) {
+    const pdp_graph& g = A.g; const pdp_state& s = A.s;
+    for (int pass = 0; pass < 8; ++pass) {
+        const bool first = pass == 0;
+        if (!first && s.sel_need[b] <= 0) break;
+        for (int base = 0; base < n; base += nthr) {   // (nthr is a multiple of 32: whole warps take part)
+            const int i = base + tid;
+            const bool valid = i < n;
+            const float c = valid ? fabsf(score[i]) * (float)av[i] : 0.f;
+            sel_hist_var(s, valid, b, v0 + i, c, valid && av[i], first);
+        }
+        bar_sync(bar_id, nthr);
+        if (tid < 32) sel_decide(s, b, A.dec_fraction, first);
+        bar_sync(bar_id, nthr);
+        if (first && s.sel_need[b] < 0) return false;
+    }
+    const int i0 = tid;
+    bool any = false;
+    for (int i = i0; i < n; i += nthr) {
+        const float c = fabsf(score[i]) * (float)av[i];
+        if (!sel_taken(s, b, v0 + i, c, av[i] != 0)) continue;
+        const float sg = sgnf(score[i]);
+        if (TINY) tiny_fix(t, i, sg); else fix_variable(g, s, v0 + i, sg);
+        any = true;
+        if (A.trace) {
+            const int k = atomicAdd(&s.ctrl[CTRL_TRACE_LEN], 1);
+            if (k < A.trace_cap) { A.trace[3 * k] = iter; A.trace[3 * k + 1] = v0 + i; A.trace[3 * k + 2] = (int)sg; }
+        }
+    }
+    if (any) { ls.fixed = 1; s.masked[b] = 1; s.dirty[b] = 1; }
+    bar_sync(bar_id, nthr);
+    if (tid == 0) s.sel_need[b] = -1;
+    return true;
+}
+
+#define LSYNC() bar_sync(bar_id, nthr)
 // one converged problem: pdp_decimate.py:152-171 + solver.py:275-285 + trainer.py:150-162
+template <bool FRAC>
 __device__ __forceinline__ void loc_decimate_problem(const KArgs& A, int b, int iter, int w, float pi, bool check_termination, LocSmem& ls,
                                                      int tid, int nthr, int bar_id) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
@@ -973,7 +1203,9 @@ __device__ __forceinline__ void loc_decimate_problem(const KArgs& A, int b, int 
         if (c != c) ls.cnan = 1u; else { atomicMax(&ls.cmax, f2u(c)); atomicMin(&ls.cmin, f2u(c)); }
     }
     LSYNC();
-    if (!ls.cnan) {   // first index attaining max of fl(fl(c - min) + 1), util.py:257-265
+    const bool topk = FRAC && !ls.cnan && u2f(ls.cmax) > 0.f &&
+                      loc_select_fix<false>(A, b, iter, s.score + v0, s.av + v0, v0, v1 - v0, TinyView{}, ls, tid, nthr, bar_id);
+    if (!topk && !ls.cnan) {   // first index attaining max of fl(fl(c - min) + 1), util.py:257-265
         const float m = u2f(ls.cmin);
         const float kmax = argmax_key(u2f(ls.cmax), m);
         for (int i = v0 + tid; i < v1; i += nthr) {
@@ -982,7 +1214,7 @@ __device__ __forceinline__ void loc_decimate_problem(const KArgs& A, int b, int 
         }
     }
     LSYNC();
-    if (tid == 0 && !ls.cnan && u2f(ls.cmax) > 0.f && ls.arg != 0x7fffffff) {
+    if (!topk && tid == 0 && !ls.cnan && u2f(ls.cmax) > 0.f && ls.arg != 0x7fffffff) {
         const int i = ls.arg;
         const float sg = sgnf(s.score[i]);
         if (sg != 0.f && s.av[i]) {
@@ -1027,44 +1259,7 @@ __device__ __forceinline__ void loc_decimate_problem(const KArgs& A, int b, int 
     LSYNC();
 }
 
-// ------------------------------------------------------------------------------------------------
-// shared-memory tier of the CTA-local decimation.  A problem whose masks, adjacency (16-bit local indices) and
-// scratch fit the group's share of the (idle) sweep buffer is decimated entirely in shared memory: the closure
-// is a chain of dozens of dependent rounds, each a couple of microseconds through global memory and tens of
-// nanoseconds here.  Same rounds, same arithmetic as loc_closure; what changed is written back at the end.
-// ------------------------------------------------------------------------------------------------
-struct TinyView {
-    uint8_t *av, *af, *pure, *single;
-    float *sol, *score;
-    int *cnt, *ev;
-    uint16_t *clp, *cvar, *vp, *vcls;   // local CSR / CSC: pointers, (local index | sign << 15)
-};
-__device__ __forceinline__ size_t tiny_bytes(int n, int m, int E) {
-    return (size_t)n * (1 + 1 + 4 + 4 + 4 + 4) + (size_t)m * 2 + (size_t)(m + 1 + n + 1 + 2 * E) * 2 + 64;
-}
-__device__ __forceinline__ TinyView tiny_carve(unsigned char* base, int n, int m, int E) {
-    TinyView t;
-    float* f = reinterpret_cast<float*>(base);
-    t.sol = f; t.score = f + n;
-    t.cnt = reinterpret_cast<int*>(f + 2 * n); t.ev = t.cnt + n;
-    uint16_t* h = reinterpret_cast<uint16_t*>(t.ev + n);
-    t.clp = h; t.vp = t.clp + (m + 1); t.cvar = t.vp + (n + 1); t.vcls = t.cvar + E;
-    uint8_t* q = reinterpret_cast<uint8_t*>(t.vcls + E);
-    t.av = q; t.pure = q + n; t.af = q + 2 * n; t.single = t.af + m;
-    return t;
-}
-
-__device__ __forceinline__ void tiny_fix(const TinyView& t, int i, float sg) {
-    for (int p = t.vp[i]; p < t.vp[i + 1]; ++p) {
-        const uint32_t w = t.vcls[p];
-        const float lit = (w & 0x8000u) ? -1.f : 1.f;
-        if (lit * sg > 0.f) t.af[w & 0x7fffu] = 0;
-    }
-    t.av[i] = 0;
-    t.sol[i] = (sg + 1.f) / 2.0f;
-}
-
-#define LSYNC() bar_sync(bar_id, nthr)
+template <bool FRAC>
 __device__ __forceinline__ void loc_decimate_tiny(const KArgs& A, int b, int iter, int w, float pi, bool check_termination, LocSmem& ls,
                                                   int tid, int nthr, int bar_id, unsigned char* area, int share) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
@@ -1116,7 +1311,9 @@ __device__ __forceinline__ void loc_decimate_tiny(const KArgs& A, int b, int ite
         if (c != c) ls.cnan = 1u; else { atomicMax(&ls.cmax, f2u(c)); atomicMin(&ls.cmin, f2u(c)); }
     }
     LSYNC();
-    if (!ls.cnan) {
+    const bool topk = FRAC && !ls.cnan && u2f(ls.cmax) > 0.f &&
+                      loc_select_fix<true>(A, b, iter, t.score, t.av, v0, n, t, ls, tid, nthr, bar_id);
+    if (!topk && !ls.cnan) {
         const float mn = u2f(ls.cmin);
         const float kmax = argmax_key(u2f(ls.cmax), mn);
         for (int i = tid; i < n; i += nthr) {
@@ -1125,7 +1322,7 @@ __device__ __forceinline__ void loc_decimate_tiny(const KArgs& A, int b, int ite
         }
     }
     LSYNC();
-    if (tid == 0 && !ls.cnan && u2f(ls.cmax) > 0.f && ls.arg != 0x7fffffff) {
+    if (!topk && tid == 0 && !ls.cnan && u2f(ls.cmax) > 0.f && ls.arg != 0x7fffffff) {
         const int i = ls.arg;
         const float sg = sgnf(t.score[i]);
         if (sg != 0.f && t.av[i]) {
@@ -1259,9 +1456,15 @@ __device__ __forceinline__ bool loc_problem_is_small(const pdp_graph& g, int b) 
 #define PDP_LOCAL_GROUP 128
 // `area` / `area_bytes`: the CTA's dynamic shared memory (the sweep buffer, idle during the decimation), split evenly
 // between the groups; null when the kernel has none
+// (one array for both instances of loc_decimate_all)
+__device__ __forceinline__ LocSmem* loc_smem() {
+    __shared__ LocSmem ls[8];
+    return ls;
+}
+template <bool FRAC>
 __device__ __forceinline__ void loc_decimate_all(const KArgs& A, int iter, int w, float pi, bool check_termination,
                                                  unsigned char* area, int area_bytes) {
-    __shared__ LocSmem ls[8];
+    LocSmem* ls = loc_smem();
     const pdp_state& s = A.s;
     int ngroups = blockDim.x / PDP_LOCAL_GROUP;
     if (ngroups > 8) ngroups = 8;
@@ -1280,9 +1483,9 @@ __device__ __forceinline__ void loc_decimate_all(const KArgs& A, int iter, int w
         const int n = A.g.prob_vptr[b + 1] - A.g.prob_vptr[b], m = A.g.prob_fptr[b + 1] - A.g.prob_fptr[b];
         const int E = A.g.cl_ptr[A.g.prob_fptr[b + 1]] - A.g.cl_ptr[A.g.prob_fptr[b]];
         if (n < 32768 && m < 32768 && E < 65536 && tiny_bytes(n, m, E) <= (size_t)share)
-            loc_decimate_tiny(A, b, iter, w, pi, check_termination, ls[grp], gt, gthr, 8 + grp, area + (size_t)grp * share, share);
+            loc_decimate_tiny<FRAC>(A, b, iter, w, pi, check_termination, ls[grp], gt, gthr, 8 + grp, area + (size_t)grp * share, share);
         else
-            loc_decimate_problem(A, b, iter, w, pi, check_termination, ls[grp], gt, gthr, 8 + grp);
+            loc_decimate_problem<FRAC>(A, b, iter, w, pi, check_termination, ls[grp], gt, gthr, 8 + grp);
     }
 }
 

@@ -131,6 +131,10 @@ void carve(pdp_ctx* c, Carver& k, int64_t E, int64_t V, int64_t F, int64_t B) {
     s.last_d = k.take<float>(B);
     s.stamp_c = k.take<int32_t>(F);
     s.stamp_v = k.take<int32_t>(V);
+    s.sel_hist = k.take<uint32_t>(B * PDP_SEL_BINS);
+    s.sel_pref = k.take<unsigned long long>(B);
+    s.sel_need = k.take<int32_t>(B);
+    s.sel_sh = k.take<int32_t>(B);
     s.ctrl = k.take<int32_t>(CTRL_SIZE);
     s.sm_ctr = k.take<int32_t>(PDP_MAX_SMS);
     s.asg = k.take<int8_t>(V);
@@ -249,6 +253,8 @@ __global__ void k_reset_state(pdp_graph g, pdp_state s, int64_t V, int64_t F, in
             s.nav[i] = 0; s.arg_idx[i] = 0x7fffffff; s.energy[i] = 0; s.want_score[i] = 0; s.have_score[i] = 0; s.last_d[i] = 0.f;
             s.st_max[2 * i] = 0u; s.st_max[2 * i + 1] = 0u; s.st_min[2 * i] = 0x7f800000u; s.st_min[2 * i + 1] = 0x7f800000u;
             s.st_nan[i] = 0u; s.c_max[i] = 0u; s.c_min[i] = 0x7f800000u; s.c_nan[i] = 0u;
+            s.sel_need[i] = -1; s.sel_sh[i] = 0; s.sel_pref[i] = 0ull;
+            for (int j = 0; j < PDP_SEL_BINS; ++j) s.sel_hist[i * PDP_SEL_BINS + j] = 0u;
         }
         if (i < CTRL_SIZE) s.ctrl[i] = (i == CTRL_NUM_ACTIVE) ? (int32_t)B
                                        : ((i == CTRL_ANY_DIRTY || i == CTRL_FR_EPC || i == CTRL_FR_EPV || i == CTRL_NATIVE) ? 1 : 0);

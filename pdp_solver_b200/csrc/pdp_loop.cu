@@ -97,6 +97,47 @@ __device__ __forceinline__ void select_and_fix_phase(const KArgs& A, int iter, b
     }
 }
 
+// the fix step of the fused loop with a fraction: the arg-max fixes (K_b == 1) and the top-K fixes of the other problems,
+// one warp per taken variable (warp_fix_variable, + the frontier lists).  Fixes of one step commute: a clause is
+// de-activated iff it holds a newly true literal (_set_variable_core, solver.py:205-226).
+__device__ __forceinline__ void frac_select_and_fix(const KArgs& A, cg::grid_group& grid, int iter, bool frontier) {
+    const pdp_graph& g = A.g; const pdp_state& s = A.s;
+    sel_grid(A, grid, CoefScore{s}, A.dec_fraction);
+    select_and_fix_phase(A, iter, frontier);
+    const int slot = CTRL_FIX + (iter & 1);
+    const int epc = s.ctrl[CTRL_FR_EPC], epv = s.ctrl[CTRL_FR_EPV];
+    for (int64_t base = gwarp() * 32; base < g.V; base += gwarps() * 32) {
+        const int64_t i = base + lane_id();
+        bool take = false;
+        float sg = 0.f;
+        if (i < g.V) {
+            const int b = g.bvm[i];
+            if (s.sel_need[b] == 0) {
+                take = sel_taken(s, b, i, fabsf(s.score[i]) * (float)s.av[i], s.av[i] != 0);
+                sg = sgnf(s.score[i]);
+            }
+        }
+        unsigned m = __ballot_sync(0xffffffffu, take);
+        while (m) {
+            const int src = __ffs(m) - 1;
+            m &= m - 1;
+            const int vi = (int)__shfl_sync(0xffffffffu, i, src);
+            const float vsg = __shfl_sync(0xffffffffu, sg, src);
+            warp_fix_variable(g, s, vi, vsg, frontier, epc, epv);
+            if (lane_id() == 0) {
+                const int b = g.bvm[vi];
+                s.masked[b] = 1; s.dirty[b] = 1;
+                s.ctrl[slot] = 1; s.ctrl[CTRL_ANY_DIRTY] = 1;
+                if (A.trace) {
+                    const int k = atomicAdd(&s.ctrl[CTRL_TRACE_LEN], 1);
+                    if (k < A.trace_cap) { A.trace[3 * k] = iter; A.trace[3 * k + 1] = vi; A.trace[3 * k + 2] = (int)vsg; }
+                }
+            }
+            __syncwarp();
+        }
+    }
+}
+
 // trainer.py:150-162 on the dirty problems
 __device__ __forceinline__ void termination_phase(const KArgs& A, int iter, int rep) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
@@ -122,8 +163,10 @@ __device__ __forceinline__ void termination_phase(const KArgs& A, int iter, int 
     if (gtid() == 0) s.ctrl[CTRL_ANY_DIRTY] = 0;
 }
 
-// FAST: the blocked shared-memory passes (pi == 0, q_u only); otherwise the generic passes
-template <bool FAST, bool FULL, int CTAS>
+// FAST: the blocked shared-memory passes (pi == 0, q_u only); otherwise the generic passes.
+// FRAC: a decimation fraction is set (pdp_set_decimation_fraction); a separate instance, so that the top-K selection
+// takes nothing from the registers of the instance the reference's rule runs in
+template <bool FAST, bool FULL, int CTAS, bool FRAC>
 __global__ void __launch_bounds__(FAST ? SweepCfg<CTAS>::kThreads : 256, FAST ? CTAS : 1)
 k_sp_run(const __grid_constant__ KArgs A, const __grid_constant__ pdp_sp_params prm, int32_t* d_iters_done) {
     extern __shared__ __align__(128) unsigned char smem_dyn[];
@@ -208,8 +251,8 @@ k_sp_run(const __grid_constant__ KArgs A, const __grid_constant__ pdp_sp_params 
         LOOP_T(20);
         if (local_ok && s.ctrl[CTRL_CONV + (iter & 1)]) {
             // converged problems one CTA can walk: scoring, arg-max, fix, closure, CNF check, termination, CTA-local
-            loc_decimate_all(A, iter, w, prm.pi, prm.check_termination != 0, FAST ? smem_dyn : nullptr,
-                             FAST ? SweepCfg<CTAS>::kSmem : 0);
+            loc_decimate_all<FRAC>(A, iter, w, prm.pi, prm.check_termination != 0, FAST ? smem_dyn : nullptr,
+                                   FAST ? SweepCfg<CTAS>::kSmem : 0);
             LOOP_T(21);
             GRID_SYNC();
             LOOP_T(22);
@@ -219,9 +262,10 @@ k_sp_run(const __grid_constant__ KArgs A, const __grid_constant__ pdp_sp_params 
             score_phase(A, w, prm.pi);
             GRID_SYNC();
             LOOP_T(24);
-            argmax_phase(A);
+            argmax_phase(A, CoefScore{s});
             GRID_SYNC();
-            select_and_fix_phase(A, iter, frontier);
+            if (FRAC) frac_select_and_fix(A, grid, iter, frontier);
+            else select_and_fix_phase(A, iter, frontier);
             GRID_SYNC();
             LOOP_T(25);
             if (s.ctrl[CTRL_FIX + (iter & 1)]) {
@@ -287,6 +331,44 @@ __global__ void __launch_bounds__(256) k_set_variables(const __grid_constant__ K
     if (gtid() == 0) s.ctrl[CTRL_CLOSED] = 1;
 }
 
+// pdp_decimation_select: the decimation rule on caller-supplied coefficients, with the phases of the fused loop
+__global__ void __launch_bounds__(256) k_decimation_select(const __grid_constant__ KArgs A, const float* __restrict__ coeff,
+                                                           const float* __restrict__ score, const uint8_t* __restrict__ psel,
+                                                           float* __restrict__ out) {
+    cg::grid_group grid = cg::this_grid();
+    const pdp_graph& g = A.g; const pdp_state& s = A.s;
+    WARP_STRIDED(i, g.V) { if (i < g.V) out[i] = 0.f; }
+    WARP_STRIDED(b, g.B) { if (b < g.B) s.conv[b] = psel ? (psel[b] != 0) : 1; }
+    grid.sync();
+    KeyedReducer<CoefAcc> red;   // per-problem max / min / NaN of the coefficients (score_phase's statistics)
+    WARP_STRIDED(i, g.V) {
+        if (i >= g.V) continue;
+        const int b = g.bvm[i];
+        if (!s.conv[b]) continue;
+        red.touch(s, b);
+        red.acc.add(coeff[i]);
+    }
+    red.finish(s);
+    grid.sync();
+    argmax_phase(A, CoefGiven{coeff});
+    grid.sync();
+    if (A.dec_fraction > 0.f) sel_grid(A, grid, CoefGiven{coeff}, A.dec_fraction);
+    WARP_STRIDED(i, g.V) {
+        if (i >= g.V) continue;
+        const int b = g.bvm[i];
+        if (A.dec_fraction > 0.f && s.sel_need[b] == 0 && sel_taken(s, b, i, coeff[i], s.av[i] != 0)) out[i] = sgnf(score[i]);
+    }
+    WARP_STRIDED(b, g.B) {
+        if (b >= g.B) continue;
+        if (s.conv[b] && !s.c_nan[b] && u2f(s.c_max[b]) > 0.f && s.arg_idx[b] != 0x7fffffff) out[s.arg_idx[b]] = sgnf(score[s.arg_idx[b]]);
+    }
+    grid.sync();
+    WARP_STRIDED(b, g.B) {   // the per-iteration scratch of the fused loop back to its resting state
+        if (b >= g.B) continue;
+        s.conv[b] = 0; s.c_max[b] = 0u; s.c_min[b] = 0x7f800000u; s.c_nan[b] = 0u; s.arg_idx[b] = 0x7fffffff; s.sel_need[b] = -1;
+    }
+}
+
 template <typename K>
 int coop_blocks(pdp_ctx* ctx, K kernel) {
     int per_sm = 0;
@@ -316,6 +398,7 @@ static KArgs make_args(pdp_ctx* ctx) {
     KArgs A;
     A.g = ctx->g; A.s = ctx->s; A.trace = ctx->trace; A.trace_cap = ctx->trace_cap;
     A.stagger_c = PDP_STAGGER_C; A.stagger_v = PDP_STAGGER_V;
+    A.dec_fraction = ctx->dec_fraction;
     if (const char* e = getenv("PDP_B200_STAGGER_C")) A.stagger_c = atoi(e);
     if (const char* e = getenv("PDP_B200_STAGGER_V")) A.stagger_v = atoi(e);
     return A;
@@ -332,11 +415,13 @@ extern "C" int pdp_sp_run(pdp_ctx* ctx, const pdp_sp_params* params, int32_t* d_
     ctx->full_state_tracked = prm.full_state ? 1 : 0;
     ctx->last_pi = prm.pi;
     void* args[] = {&A, &prm, &d_iters_done};
+    const bool frac = ctx->dec_fraction > 0.f;
     const bool fast = ctx->g.blocked_ok && !prm.full_state && prm.pi == 0.f && !(prm.flags & 1);
     if (fast) {
         // one or two CTAs per SM holding the whole shared memory: co-residency of the cooperative grid is guaranteed
         const int two = (ctx->g.ctas == 2) ? 1 : 0;
-        void* kern = two ? (void*)k_sp_run<true, false, 2> : (void*)k_sp_run<true, false, 1>;
+        void* kern = frac ? (two ? (void*)k_sp_run<true, false, 2, true> : (void*)k_sp_run<true, false, 1, true>)
+                          : (two ? (void*)k_sp_run<true, false, 2, false> : (void*)k_sp_run<true, false, 1, false>);
         const int smem = two ? SweepCfg<2>::kSmem : SweepCfg<1>::kSmem;
         const int threads = two ? SweepCfg<2>::kThreads : SweepCfg<1>::kThreads;
         // (set on every launch: a per-device "already set" table would be shared, unsynchronised, by the worker threads of the
@@ -344,14 +429,12 @@ extern "C" int pdp_sp_run(pdp_ctx* ctx, const pdp_sp_params* params, int32_t* d_
         PDP_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         if (two) PDP_CUDA_CHECK(cudaMemsetAsync(ctx->s.sm_ctr, 0, sizeof(int32_t) * PDP_MAX_SMS, stream));
         PDP_CUDA_CHECK(cudaLaunchCooperativeKernel(kern, dim3(ctx->num_sms * (two ? 2 : 1)), dim3(threads), args, smem, stream));
-    } else if (prm.full_state) {
-        int blocks = coop_blocks(ctx, k_sp_run<false, true, 1>);
-        if (blocks < 1) { pdp_set_error("pdp_sp_run: occupancy query failed"); return PDP_ERR_CUDA; }
-        PDP_CUDA_CHECK(cudaLaunchCooperativeKernel((void*)k_sp_run<false, true, 1>, dim3(blocks), dim3(256), args, 0, stream));
     } else {
-        int blocks = coop_blocks(ctx, k_sp_run<false, false, 1>);
+        void* kern = prm.full_state ? (frac ? (void*)k_sp_run<false, true, 1, true> : (void*)k_sp_run<false, true, 1, false>)
+                                    : (frac ? (void*)k_sp_run<false, false, 1, true> : (void*)k_sp_run<false, false, 1, false>);
+        int blocks = coop_blocks(ctx, kern);
         if (blocks < 1) { pdp_set_error("pdp_sp_run: occupancy query failed"); return PDP_ERR_CUDA; }
-        PDP_CUDA_CHECK(cudaLaunchCooperativeKernel((void*)k_sp_run<false, false, 1>, dim3(blocks), dim3(256), args, 0, stream));
+        PDP_CUDA_CHECK(cudaLaunchCooperativeKernel(kern, dim3(blocks), dim3(256), args, 0, stream));
     }
     PDP_LAUNCH_CHECK(ctx);
     return PDP_OK;
@@ -375,6 +458,30 @@ extern "C" int pdp_set_variables(pdp_ctx* ctx, const float* d_assignment, void* 
     int blocks = coop_blocks(ctx, k_set_variables);
     if (blocks < 1) { pdp_set_error("pdp_set_variables: occupancy query failed"); return PDP_ERR_CUDA; }
     PDP_CUDA_CHECK(cudaLaunchCooperativeKernel((void*)k_set_variables, dim3(blocks), dim3(256), args, 0, (cudaStream_t)stream_));
+    PDP_LAUNCH_CHECK(ctx);
+    return PDP_OK;
+}
+
+static bool valid_fraction(float f) { return f == f && f >= 0.f && f < 1.f; }
+
+// SP-inspired decimation (pdp_b200.h): the fraction of each problem's active variables the fused loop fixes per step
+extern "C" int pdp_set_decimation_fraction(pdp_ctx* ctx, float fraction) {
+    if (!ctx) { pdp_set_error("pdp_set_decimation_fraction: null context"); return PDP_ERR_ARG; }
+    if (!valid_fraction(fraction)) { pdp_set_error("pdp_set_decimation_fraction: fraction %g not in [0, 1)", (double)fraction); return PDP_ERR_ARG; }
+    ctx->dec_fraction = fraction;
+    return PDP_OK;
+}
+
+extern "C" int pdp_decimation_select(pdp_ctx* ctx, const float* d_coeff, const float* d_score, const uint8_t* d_problem_sel,
+                                     float fraction, float* d_assignment, void* stream_) {
+    if (!ctx || (ctx->g.V > 0 && (!d_coeff || !d_score || !d_assignment))) { pdp_set_error("pdp_decimation_select: null argument"); return PDP_ERR_ARG; }
+    if (!valid_fraction(fraction)) { pdp_set_error("pdp_decimation_select: fraction %g not in [0, 1)", (double)fraction); return PDP_ERR_ARG; }
+    KArgs A = make_args(ctx);
+    A.dec_fraction = fraction;
+    void* args[] = {&A, &d_coeff, &d_score, &d_problem_sel, &d_assignment};
+    int blocks = coop_blocks(ctx, k_decimation_select);
+    if (blocks < 1) { pdp_set_error("pdp_decimation_select: occupancy query failed"); return PDP_ERR_CUDA; }
+    PDP_CUDA_CHECK(cudaLaunchCooperativeKernel((void*)k_decimation_select, dim3(blocks), dim3(256), args, 0, (cudaStream_t)stream_));
     PDP_LAUNCH_CHECK(ctx);
     return PDP_OK;
 }

@@ -520,7 +520,7 @@ extern "C" int pdp_walksat(pdp_ctx* ctx, int32_t W, float epsilon, int32_t batch
     const int rep = batch_replication > 1 ? batch_replication : 1;
     if (ctx->g.B % rep != 0) { pdp_set_error("pdp_walksat: batch size not divisible by replication"); return PDP_ERR_ARG; }
     KArgs A;
-    A.g = ctx->g; A.s = ctx->s; A.trace = nullptr; A.trace_cap = 0; A.stagger_c = 0; A.stagger_v = 0;
+    A.g = ctx->g; A.s = ctx->s; A.trace = nullptr; A.trace_cap = 0; A.stagger_c = 0; A.stagger_v = 0; A.dec_fraction = 0.f;
 #ifdef PDP_PHASE_TIMING
     A.trace = ctx->trace;
 #endif

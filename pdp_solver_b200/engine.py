@@ -243,6 +243,23 @@ class Context(object):
         a = _f32(assignment, self.device).reshape(-1)
         self._check(self._L.pdp_set_variables(self._h, _ptr(a), _stream()), "pdp_set_variables")
 
+    def set_decimation_fraction(self, fraction):
+        """SP-inspired decimation in sp_run: every selected problem fixes max(1, floor(fraction * active variables)) of its
+        most biased variables per decimation step; 0 (the default) is the reference's one arg-max variable.  The value
+        stays until the next call (pdp_reset keeps it)."""
+        self._check(self._L.pdp_set_decimation_fraction(self._h, float(fraction)), "pdp_set_decimation_fraction")
+
+    def decimation_select(self, coeff, score, fraction, problem_sel=None):
+        """The decimation rule (arg-max for K_b == 1, top-K_b otherwise) on given coefficients [V] (>= 0) and scores [V]:
+        returns the assignment [V] with sign(score) on the taken variables and 0 elsewhere.  problem_sel [B] (nonzero =
+        converged and active; None = every problem); K_b counts the context's active variables."""
+        c, sc = _f32(coeff, self.device).reshape(-1), _f32(score, self.device).reshape(-1)
+        ps = None if problem_sel is None else problem_sel.to(device=self.device, dtype=torch.uint8).reshape(-1).contiguous()
+        out = self._new(self.V)
+        self._check(self._L.pdp_decimation_select(self._h, _ptr(c), _ptr(sc), _ptr(ps), float(fraction), _ptr(out), _stream()),
+                    "pdp_decimation_select")
+        return out
+
     def enable_trace(self, capacity=1 << 16):
         self._trace = torch.zeros(capacity, 3, dtype=torch.int32, device=self.device)
         self._check(self._L.pdp_set_trace_buffer(self._h, _ptr(self._trace), capacity), "pdp_set_trace_buffer")

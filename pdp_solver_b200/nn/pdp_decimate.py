@@ -1,4 +1,6 @@
 """Decimators of the PDP framework, B200-native (reference src/pdp/nn/pdp_decimate.py)."""
+import math
+
 import torch
 import torch.nn as nn
 
@@ -34,6 +36,17 @@ def problem_argmax(x, bvm, B):
     mx = torch.zeros(B, dtype=x.dtype, device=x.device).scatter_reduce(0, idx, y, "amax", include_self=True)
     pos = torch.where(y == mx[idx], torch.arange(V, device=x.device), torch.full((1,), V, device=x.device))
     return torch.full((B,), V, dtype=torch.int64, device=x.device).scatter_reduce(0, idx, pos, "amin", include_self=True)
+
+
+def check_decimation_fraction(fraction):
+    """the fraction of SP-inspired decimation: a finite float with 0 <= f < 1 (0 = one arg-max variable per step)"""
+    try:
+        f = float(fraction)
+    except (TypeError, ValueError):
+        raise ValueError("decimation_fraction must be a number, got %r" % (fraction,))
+    if not math.isfinite(f) or not 0.0 <= f < 1.0:
+        raise ValueError("decimation_fraction must be finite with 0 <= f < 1, got %r" % (fraction,))
+    return f
 
 
 class NeuralDecimator(nn.Module):
@@ -106,13 +119,18 @@ class SequentialDecimator(nn.Module):
     one variable per problem and iteration is fixed, once that problem's surveys have converged
     (max smooth-max |delta eta| < tolerance) or its counter reached t_max.
 
+    decimation_fraction f > 0 turns it into SP-inspired decimation: a selected problem with A active variables fixes
+    the max(1, floor(f * A)) variables with the largest |score| at once (include/pdp_b200.h, pdp_decimation_select).
+    It is a plain attribute, not a buffer: state dicts of the reference load unchanged.
+
     Its statistics, per-problem decisions, scoring, arg-max, variable fixing and the following unit
     propagation / peeling closure all live inside the persistent kernel launched by
     PropagatorDecimatorSolverBase.forward (pdp_sp_run); the module keeps the hyper-parameters and the
     initial-state contract."""
 
-    def __init__(self, device, message_dimension, scorer, tolerance, t_max):
+    def __init__(self, device, message_dimension, scorer, tolerance, t_max, decimation_fraction=0.0):
         super(SequentialDecimator, self).__init__()
+        self._decimation_fraction = check_decimation_fraction(decimation_fraction)
         self._device = device
         self._tolerance = tolerance
         self._scorer = scorer
@@ -151,7 +169,14 @@ class SequentialDecimator(nn.Module):
             if bool((conv_v.sum() > 0).item()):
                 score = self._scorer(message_state, sat_problem)[0][:, 0]
                 coeff = score.abs() * av * conv_v
-                if bool((coeff.sum() > 0).item()):
+                if bool((coeff.sum() > 0).item()) and self._decimation_fraction > 0.0:
+                    sel = None if active_mask is None else active_mask[:, 0]
+                    assignment = ctx.decimation_select(coeff, score, self._decimation_fraction, sel)
+                    ind = torch.nonzero(assignment).reshape(-1)
+                    if ind.numel() > 0:
+                        sat_problem.set_variables(assignment)
+                        self.decimation_log.append((ind, assignment[ind].clone()))
+                elif bool((coeff.sum() > 0).item()):
                     max_ind = problem_argmax(coeff, bvm, B)
                     norm = torch.zeros(B, device=ctx.device).index_add_(0, idx, coeff)
                     sel = norm != 0

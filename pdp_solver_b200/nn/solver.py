@@ -263,6 +263,7 @@ class PropagatorDecimatorSolverBase(nn.Module):
         else:
             ctx.load_state(init_propagator_state, init_decimator_state[:2])
         b = sat_problem._batch_replication
+        ctx.set_decimation_fraction(dec._decimation_fraction)
         if check_termination is None or _is_standard_termination(check_termination):
             self.last_iterations = ctx.sp_run(iteration_num, dec._tolerance, dec._t_max,
                                               check_termination is not None, b, self._propagator.pi_value())
@@ -373,14 +374,14 @@ class PropagatorDecimatorSolverBase(nn.Module):
 class SurveyPropagatorSolver(PropagatorDecimatorSolverBase):
     "The classical SP-guided decimation solver, model type `p-d-p` (reference solver.py:567-578)."
 
-    def __init__(self, device, name, tolerance, t_max, local_search_iterations=0, epsilon=0.05):
+    def __init__(self, device, name, tolerance, t_max, local_search_iterations=0, epsilon=0.05, decimation_fraction=0.0):
         super(SurveyPropagatorSolver, self).__init__(
             device=device, name=name,
             propagator=pdp_propagate.SurveyPropagator(device, decimator_dimension=1, include_adaptors=False),
             decimator=pdp_decimate.SequentialDecimator(
                 device, message_dimension=(3, 1),
                 scorer=pdp_predict.SurveyScorer(device, message_dimension=1, include_adaptors=False),
-                tolerance=tolerance, t_max=t_max),
+                tolerance=tolerance, t_max=t_max, decimation_fraction=decimation_fraction),
             predictor=pdp_predict.IdentityPredictor(device=device, random_fill=True),
             local_search_iterations=local_search_iterations, epsilon=epsilon)
 
@@ -458,7 +459,7 @@ class NeuralSequentialDecimatorSolver(PropagatorDecimatorSolverBase):
 
     def __init__(self, device, name, edge_dimension, meta_data_dimension, propagator_dimension, decimator_dimension,
                  mem_hidden_dimension, agg_hidden_dimension, mem_agg_hidden_dimension, classifier_dimension, dropout,
-                 tolerance, t_max, local_search_iterations=0, epsilon=0.05):
+                 tolerance, t_max, local_search_iterations=0, epsilon=0.05, decimation_fraction=0.0):
         super(NeuralSequentialDecimatorSolver, self).__init__(
             device=device, name=name,
             propagator=pdp_propagate.NeuralMessagePasser(device, edge_dimension, decimator_dimension, meta_data_dimension,
@@ -471,7 +472,7 @@ class NeuralSequentialDecimatorSolver(PropagatorDecimatorSolverBase):
                                                    variable_classifier=util.PerceptronTanh(decimator_dimension,
                                                                                            classifier_dimension, 1),
                                                    function_classifier=None),
-                tolerance=tolerance, t_max=t_max),
+                tolerance=tolerance, t_max=t_max, decimation_fraction=decimation_fraction),
             predictor=pdp_predict.IdentityPredictor(device=device, random_fill=True),
             local_search_iterations=local_search_iterations, epsilon=epsilon)
         self.to(device)

@@ -5,7 +5,7 @@ import torch
 import torch.nn as nn
 
 from .factorgraph import FactorGraphTrainerBase
-from .nn import solver, util
+from .nn import pdp_decimate, solver, util
 
 
 class Perceptron(nn.Module):
@@ -46,6 +46,10 @@ class SatFactorGraphTrainer(FactorGraphTrainerBase):
         "reference trainer.py:48-99"
         t = config["model_type"]
         w, eps = config["local_search_iteration"], config["epsilon"]
+        # SP-inspired decimation (optional key): only the model types with a sequential decimator fix variables
+        frac = pdp_decimate.check_decimation_fraction(config.get("decimation_fraction", 0.0))
+        if frac != 0.0 and t not in ("p-d-p", "np-d-np"):
+            raise ValueError("decimation_fraction applies to model types p-d-p and np-d-np only, not %r" % (t,))
         neural = dict(edge_dimension=config.get("edge_feature_dim"), meta_data_dimension=config.get("meta_feature_dim"),
                       mem_hidden_dimension=config.get("mem_hidden_dim"), agg_hidden_dimension=config.get("agg_hidden_dim"),
                       mem_agg_hidden_dimension=config.get("mem_agg_hidden_dim"), dropout=config.get("dropout", 0),
@@ -66,11 +70,11 @@ class SatFactorGraphTrainer(FactorGraphTrainerBase):
             model = solver.NeuralSequentialDecimatorSolver(
                 device=self._device, name=config["model_name"], propagator_dimension=config["hidden_dim"],
                 decimator_dimension=config["hidden_dim"], classifier_dimension=config["classifier_dim"],
-                tolerance=config["tolerance"], t_max=config["t_max"], **neural)
+                tolerance=config["tolerance"], t_max=config["t_max"], decimation_fraction=frac, **neural)
         elif t == "p-d-p":
             model = solver.SurveyPropagatorSolver(device=self._device, name=config["model_name"],
                                                   tolerance=config["tolerance"], t_max=config["t_max"],
-                                                  local_search_iterations=w, epsilon=eps)
+                                                  local_search_iterations=w, epsilon=eps, decimation_fraction=frac)
         elif t == "walk-sat":
             model = solver.WalkSATSolver(device=self._device, name=config["model_name"], iteration_num=w, epsilon=eps)
         elif t == "reinforce":
