@@ -47,6 +47,7 @@ typedef struct pdp_ctx pdp_ctx;
 #define PDP_FLAG_SOLVED 2u         /* a satisfying assignment was found (trainer.py:150-162)      */
 #define PDP_FLAG_CONTRADICTION 4u  /* NaN surveys: SP contradiction (pdp_propagate.py:215-216)    */
 #define PDP_FLAG_UP_CONFLICT 8u    /* unit propagation conflict (solver.py:247-261)               */
+#define PDP_FLAG_ROLLED_BACK 16u   /* a decimation step was undone (pdp_set_conflict_rollback)    */
 
 const char* pdp_version(void);
 const char* pdp_last_error(void);
@@ -202,6 +203,27 @@ int pdp_set_decimation_fraction(pdp_ctx* ctx, float fraction);
 int pdp_decimation_select(pdp_ctx* ctx, const float* d_coeff, const float* d_score, const uint8_t* d_problem_sel,
                           float fraction, float* d_assignment, void* stream);
 
+/* Conflict rollback for SP-inspired decimation.  One unit-propagation conflict ends a problem (the `== 1` quirk of
+ * solver.py:257,261 wipes it, any count sets PDP_FLAG_UP_CONFLICT), so a step that fixes too many variables at once throws
+ * away every step before it.  With rollback on, each problem b carries a halving exponent h_b and a rollback count r_b
+ * (both 0 after pdp_reset) and pdp_sp_run decimates with
+ *   K_b = max(1, floor((double)f * A_b) >> h_b)      (h_b = 0: the rule of pdp_set_decimation_fraction; same selection).
+ * When a step of b with K_b >= 2 fixes its variables and the UP + peel closure that follows sets PDP_FLAG_UP_CONFLICT,
+ * which was clear before the step, b's active variables, active clauses, solution and is_sat go back to their values just
+ * before the fix (the edge mask with them), the conflict bit is cleared, PDP_FLAG_ROLLED_BACK is set, and h_b and r_b grow
+ * by one.  Messages, previous surveys and counters are untouched: the step changed none of them.  A K_b = 1 step that
+ * conflicts stands (retrying it would pick the same variable from the same surveys).  h_b never decreases before
+ * pdp_reset.  The decimation trace keeps the fixes of a rolled-back step.
+ * pdp_rollback_scratch_bytes: bytes of the snapshot buffer (the state of the problems a step decimates, taken before the fix).
+ * pdp_set_conflict_rollback: d_scratch (device, 16-byte aligned, >= pdp_rollback_scratch_bytes) turns rollback on, NULL
+ *   turns it off; off after pdp_create, kept by pdp_reset.  The buffer belongs to the caller and must outlive its use.
+ *   Rollback acts only when a decimation fraction is set.
+ * pdp_get_rollbacks: d_count int32 [B] receives r_b, d_last_iter int32 [B] the iteration (1-based, counted since
+ *   pdp_reset) of b's last rollback, 0 when none; NULL = skip. */
+size_t pdp_rollback_scratch_bytes(int64_t V, int64_t F, int64_t B);
+int pdp_set_conflict_rollback(pdp_ctx* ctx, void* d_scratch, size_t bytes);
+int pdp_get_rollbacks(pdp_ctx* ctx, int32_t* d_count, int32_t* d_last_iter, void* stream);
+
 /* IdentityPredictor.forward(last_call=True), reference pdp/nn/pdp_predict.py:118-128.
  * pdp_count_active_variables syncs the stream.  d_draws holds >= n_active uniform draws that are
  * consumed by the active variables in batch-global variable order (like torch.rand(n_active)). */
@@ -231,6 +253,9 @@ int pdp_trace_length(pdp_ctx* ctx, int32_t* host_out, void* stream);
  * blocked layout is on); host_info int32[5] (nullable) = {blocked, variable blocks, clause blocks,
  * variable block stride, clause block stride} */
 int pdp_debug_check_layout(pdp_ctx* ctx, int32_t* d_errs, int32_t* host_info, void* stream);
+/* self-check of the edge-mask bits the sweeps read (tests): d_errs device int32[2] receives the number of edges whose bit in
+ * the variable-side / clause-side layout differs from "variable or clause inactive" under the current node masks */
+int pdp_debug_check_edge_mask(pdp_ctx* ctx, int32_t* d_errs, void* stream);
 
 /* ---- host-side ingest helpers (no device work; SURVEY.md section 8f rank 1) ---------------------------
  * pdp_host_parse_ints: scans `text[0..len)` for decimal integers (optional leading '-', any other byte is a

@@ -62,6 +62,10 @@ SIGNATURES = {
     "pdp_deduplicate": (ctypes.c_int, [P, I32, P, P, P, P]),
     "pdp_set_decimation_fraction": (ctypes.c_int, [P, F32]),
     "pdp_decimation_select": (ctypes.c_int, [P, P, P, P, F32, P, P]),
+    "pdp_rollback_scratch_bytes": (ctypes.c_size_t, [I64, I64, I64]),
+    "pdp_set_conflict_rollback": (ctypes.c_int, [P, P, ctypes.c_size_t]),
+    "pdp_get_rollbacks": (ctypes.c_int, [P, P, P, P]),
+    "pdp_debug_check_edge_mask": (ctypes.c_int, [P, P, P]),
     "pdp_set_trace_buffer": (ctypes.c_int, [P, P, I32]),
     "pdp_trace_length": (ctypes.c_int, [P, ctypes.POINTER(I32), P]),
     "pdp_debug_check_layout": (ctypes.c_int, [P, P, ctypes.POINTER(I32 * 5), P]),

@@ -29,6 +29,9 @@ struct KArgs {
     int32_t trace_cap;
     int32_t stagger_c, stagger_v;   // cycles the second CTA of an SM waits at the start of a clause / variable pass
     float dec_fraction;             // pdp_set_decimation_fraction (0: the arg-max rule only)
+    // conflict rollback (pdp_set_conflict_rollback): the snapshot of the problems a step decimates, indexed like the state
+    // (all null: rollback off)
+    struct { float* sol; float* is_sat; uint8_t* av; uint8_t* af; } rb;
 };
 
 __device__ __forceinline__ int lane_id() { return threadIdx.x & 31; }
@@ -501,6 +504,52 @@ __device__ __forceinline__ void fix_variable(const pdp_graph& g, const pdp_state
     s.sol[i] = (sg + 1.f) / 2.0f;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Conflict rollback (pdp_set_conflict_rollback).  A decimation step of problem b with K_b >= 2 and a clear conflict bit
+// first copies b's node masks, solution and is_sat to the caller's snapshot buffer (one byte per node mask, indexed like the
+// state: neighbouring problems never write the same byte, so their copies need no atomics).  When the closure after the fix
+// sets b's conflict bit, the nodes go back to the snapshot and the edge-mask bits of b's edges are rebuilt from the restored
+// node masks; the messages, previous surveys and counters are not touched, the step changed none of them.
+// A restored state is one the library itself produced and closed under UP + peeling before this step: the precondition of
+// the frontier closure (CTRL_CLOSED) and that of the CNF count (CTRL_NATIVE, only the library changed the masks) still hold.
+// ------------------------------------------------------------------------------------------------
+// (the conflict marking of the grid-wide closure) b's top-K step conflicted: flag it for rb_restore_grid
+__device__ __forceinline__ void rb_mark(const KArgs& A, int b) {
+    const pdp_state& s = A.s;
+    if (A.rb.av && s.rb_snap[b]) { s.rb_snap[b] = 2; s.ctrl[CTRL_RB] = 1; }
+}
+__device__ __forceinline__ void rb_save_var(const KArgs& A, int i) { A.rb.av[i] = A.s.av[i]; A.rb.sol[i] = A.s.sol[i]; }
+__device__ __forceinline__ void rb_save_clause(const KArgs& A, int a) { A.rb.af[a] = A.s.af[a]; }
+// one edge-mask bit; atomic because a mask word holds edges of other nodes and problems
+__device__ __forceinline__ void rb_edge_bit(uint32_t* words, int pos, bool masked) {
+    const uint32_t bit = 1u << (pos & 31);
+    const bool now = (__ldcg(words + (pos >> 5)) & bit) != 0u;
+    if (masked && !now) atomicOr(words + (pos >> 5), bit);
+    else if (!masked && now) atomicAnd(words + (pos >> 5), ~bit);
+}
+// variable i back to the snapshot, with the mask bits of its edges (taken from the snapshot's masks, so the clause restores
+// need not be complete)
+__device__ __forceinline__ void rb_restore_var(const KArgs& A, int i) {
+    const pdp_graph& g = A.g; const pdp_state& s = A.s;
+    const uint8_t v = A.rb.av[i];
+    s.av[i] = v;
+    s.sol[i] = A.rb.sol[i];
+    for (int p = g.var_ptr[i]; p < g.var_ptr[i + 1]; ++p) {
+        const bool masked = !(v && A.rb.af[g.v_cls[p]]);
+        rb_edge_bit(g.vmask, g.p_vpos[p], masked);
+        rb_edge_bit(g.qmask, g.p_qpos[p], masked);
+    }
+}
+__device__ __forceinline__ void rb_restore_clause(const KArgs& A, int a) { A.s.af[a] = A.rb.af[a]; }
+// the per-problem part of a rollback (one thread)
+__device__ __forceinline__ void rb_commit(const KArgs& A, int b, int iter) {
+    const pdp_state& s = A.s;
+    s.is_sat[b] = A.rb.is_sat[b];
+    s.flags[b] = (s.flags[b] & ~PDP_FLAG_UP_CONFLICT) | PDP_FLAG_ROLLED_BACK;
+    s.rb_h[b] += 1;
+    s.rb_count[b] += 1;
+    s.rb_last[b] = iter;
+}
 
 // ------------------------------------------------------------------------------------------------
 // unit propagation round (solver.py:228-273), split at its data dependencies
@@ -538,7 +587,8 @@ __device__ __forceinline__ void up_find_conflicts(const KArgs& A) {
 }
 
 // quirk kept from the reference (solver.py:257,261): the problem is wiped only when its conflict
-// COUNT equals exactly one
+// COUNT equals exactly one.  RB: conflict rollback of the fused loop's grid-wide step (rb_mark)
+template <bool RB>
 __device__ __forceinline__ void up_apply_conflicts(const KArgs& A) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
     const int64_t n = g.V > g.F ? g.V : g.F;
@@ -551,7 +601,7 @@ __device__ __forceinline__ void up_apply_conflicts(const KArgs& A) {
             if (s.av[i] && s.conflicts[g.bvm[i]] == 1) deactivate_variable(g, s, (int)i);
         }
         if (i < g.B) {
-            if (s.conflicts[i] >= 1) { s.is_sat[i] = 0.f; s.flags[i] |= PDP_FLAG_UP_CONFLICT; s.masked[i] = 1; }
+            if (s.conflicts[i] >= 1) { s.is_sat[i] = 0.f; s.flags[i] |= PDP_FLAG_UP_CONFLICT; s.masked[i] = 1; if (RB) rb_mark(A, (int)i); }
         }
     }
 }
@@ -617,6 +667,7 @@ __device__ __forceinline__ void peel_apply(const KArgs& A) {
 
 // UP closure then peel closure for the dirty problems.  Called by ALL threads of the cooperative grid.
 // Flag slots alternate by round parity so a flag is never reset while it can still be read.
+template <bool RB = false>
 __device__ PDP_COLD void closure(const KArgs& A, cg::grid_group& grid) {
     const pdp_state& s = A.s;
     int round = 0;
@@ -629,7 +680,7 @@ __device__ PDP_COLD void closure(const KArgs& A, cg::grid_group& grid) {
         if (!s.ctrl[slot]) break;
         up_find_conflicts(A);
         grid.sync();
-        up_apply_conflicts(A);
+        up_apply_conflicts<RB>(A);
         grid.sync();
         up_assign(A);
         up_clear_conflicts(A);
@@ -725,10 +776,11 @@ __device__ __forceinline__ void warp_fix_variable(const pdp_graph& g, const pdp_
 __device__ __forceinline__ unsigned long long sel_key(float c, int64_t i) {
     return ((unsigned long long)__float_as_uint(c) << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)i);
 }
-// K_b in double from the fp32 fraction
-__device__ __forceinline__ int sel_k(float f, int nav) {
+// K_b in double from the fp32 fraction, halved h times (conflict rollback)
+__device__ __forceinline__ int sel_k(float f, int nav, int h) {
     const double k = floor((double)f * (double)nav);
-    return k < 1.0 ? 1 : (int)k;
+    const int64_t q = (int64_t)k >> (h < 62 ? h : 62);
+    return q < 1 ? 1 : (int)q;
 }
 // warp-aggregated histogram increment (all 32 lanes call it): lanes hitting the same bin add once
 __device__ __forceinline__ void sel_count(uint32_t* bin, bool pred) {
@@ -754,9 +806,10 @@ __device__ __forceinline__ bool sel_taken(const pdp_state& s, int b, int64_t i, 
 }
 
 // one warp, after a histogram pass of problem b: picks the digit that holds the K-th key, clears the histogram, updates the
-// problem's state.  first: K_b from the active-variable count; a problem with K_b == 1 leaves (sel_need = -1) for the
-// arg-max rule.  Returns -1 (arg-max rule), 0 (final rule) or 1 (another pass), the same in every lane.
-__device__ __forceinline__ int sel_decide(const pdp_state& s, int b, float frac, bool first) {
+// problem's state.  first: K_b from the active-variable count (halve: shifted right by the problem's rb_h); a problem with
+// K_b == 1 leaves (sel_need = -1) for the arg-max rule.  Returns -1 (arg-max rule), 0 (final rule) or 1 (another pass), the
+// same in every lane.
+__device__ __forceinline__ int sel_decide(const pdp_state& s, int b, float frac, bool first, bool halve) {
     uint32_t* h = s.sel_hist + (size_t)b * PDP_SEL_BINS;
     const int lane = lane_id();
     uint32_t v[8], tot = 0;
@@ -774,7 +827,7 @@ __device__ __forceinline__ int sel_decide(const pdp_state& s, int b, float frac,
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) { const uint32_t y = __shfl_down_sync(0xffffffffu, suf, o); if (lane + o < 32) suf += y; }
     if (first) {
-        const int K = sel_k(frac, nav);
+        const int K = sel_k(frac, nav, halve ? s.rb_h[b] : 0);
         const uint32_t ncand = __shfl_sync(0xffffffffu, suf, 0);
         if (K < 2) { if (lane == 0) s.sel_need[b] = -1; return -1; }
         if (ncand <= (uint32_t)K) {   // every candidate is taken
@@ -809,12 +862,52 @@ __device__ __forceinline__ int sel_decide(const pdp_state& s, int b, float frac,
     return done ? 0 : 1;
 }
 
+// grid-wide step with rollback on, by ALL threads after sel_grid (sel_need is final): the problems taking a top-K step with a
+// clear conflict bit are snapshotted (rb_snap = 1; every other problem gets 0).  A barrier must follow before their fixes.
+__device__ __forceinline__ bool rb_takes(const pdp_state& s, int b) {
+    return s.sel_need[b] == 0 && !(s.flags[b] & PDP_FLAG_UP_CONFLICT);
+}
+__device__ __forceinline__ void rb_snapshot_grid(const KArgs& A) {
+    const pdp_graph& g = A.g; const pdp_state& s = A.s;
+    WARP_STRIDED(b, g.B) {
+        if (b >= g.B) continue;
+        const bool t = rb_takes(s, (int)b);
+        s.rb_snap[b] = t ? 1 : 0;
+        if (t) A.rb.is_sat[b] = s.is_sat[b];
+    }
+    if (range_scans(g)) {   // few contiguous problems: their node ranges
+        for (int b = 0; b < (int)g.B; ++b) {
+            if (!rb_takes(s, b)) continue;
+            for (int i = g.prob_vptr[b] + (int)gtid(); i < g.prob_vptr[b + 1]; i += (int)gthreads()) rb_save_var(A, i);
+            for (int a = g.prob_fptr[b] + (int)gtid(); a < g.prob_fptr[b + 1]; a += (int)gthreads()) rb_save_clause(A, a);
+        }
+        return;
+    }
+    WARP_STRIDED(i, g.V) { if (i < g.V && rb_takes(s, g.bvm[i])) rb_save_var(A, (int)i); }
+    WARP_STRIDED(a, g.F) { if (a < g.F && rb_takes(s, g.bfm[a])) rb_save_clause(A, (int)a); }
+}
+// by ALL threads after the closure when CTRL_RB is set: the problems rb_mark flagged (rb_snap == 2) go back to the snapshot
+__device__ __forceinline__ void rb_restore_grid(const KArgs& A, int iter) {
+    const pdp_graph& g = A.g; const pdp_state& s = A.s;
+    WARP_STRIDED(b, g.B) { if (b < g.B && s.rb_snap[b] == 2) rb_commit(A, (int)b, iter); }
+    if (range_scans(g)) {
+        for (int b = 0; b < (int)g.B; ++b) {
+            if (s.rb_snap[b] != 2) continue;
+            for (int i = g.prob_vptr[b] + (int)gtid(); i < g.prob_vptr[b + 1]; i += (int)gthreads()) rb_restore_var(A, i);
+            for (int a = g.prob_fptr[b] + (int)gtid(); a < g.prob_fptr[b + 1]; a += (int)gthreads()) rb_restore_clause(A, a);
+        }
+        return;
+    }
+    WARP_STRIDED(i, g.V) { if (i < g.V && s.rb_snap[g.bvm[i]] == 2) rb_restore_var(A, (int)i); }
+    WARP_STRIDED(a, g.F) { if (a < g.F && s.rb_snap[g.bfm[a]] == 2) rb_restore_clause(A, (int)a); }
+}
+
 // Grid-wide selection over the problems the arg-max phase left selectable (conv, no NaN coefficient, max c > 0); called by
 // ALL threads after that phase and a barrier, returns after a barrier.  Problems with K_b >= 2 get arg_idx cleared (the
 // arg-max fix skips them) and their final rule in sel_need / sel_sh / sel_pref; every other problem gets sel_need = -1.
 // One histogram pass over the variables, then up to 7 more while some problem is undecided (CTRL_SEL parity slots).
 template <typename CF>
-__device__ __forceinline__ void sel_grid(const KArgs& A, cg::grid_group& grid, const CF& coef, float frac) {
+__device__ __forceinline__ void sel_grid(const KArgs& A, cg::grid_group& grid, const CF& coef, float frac, bool halve) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
     for (int pass = 0; pass < 8; ++pass) {
         if (pass > 0 && !s.ctrl[CTRL_SEL + (pass & 1)]) break;   // uniform: written before the last barrier
@@ -835,13 +928,13 @@ __device__ __forceinline__ void sel_grid(const KArgs& A, cg::grid_group& grid, c
             int st = -1;
             if (first) {
                 if (s.conv[b] && !s.c_nan[b] && u2f(s.c_max[b]) > 0.f) {
-                    st = sel_decide(s, (int)b, frac, true);
+                    st = sel_decide(s, (int)b, frac, true, halve);
                     if (st >= 0 && lane_id() == 0) s.arg_idx[b] = 0x7fffffff;
                 } else if (lane_id() == 0) {
                     s.sel_need[b] = -1;
                 }
             } else if (s.sel_need[b] > 0) {
-                st = sel_decide(s, (int)b, frac, false);
+                st = sel_decide(s, (int)b, frac, false, halve);
             }
             if (st > 0 && lane_id() == 0) s.ctrl[CTRL_SEL + ((pass + 1) & 1)] = 1;
         }
@@ -887,6 +980,7 @@ __device__ __forceinline__ void fr_find_conflicts(const KArgs& A, int ulist) {
     }
 }
 // up_apply_conflicts over the lists; the wipe of single-conflict problems scans their nodes (rare)
+template <bool RB>
 __device__ __forceinline__ void fr_apply_conflicts(const KArgs& A, int clist, int vlist, int epv) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
     const int n = fr_len(s, CTRL_FR_N + clist);
@@ -903,7 +997,7 @@ __device__ __forceinline__ void fr_apply_conflicts(const KArgs& A, int clist, in
         }
     }
     WARP_STRIDED(b, g.B) {
-        if (b < g.B && s.conflicts[b] >= 1) { s.is_sat[b] = 0.f; s.flags[b] |= PDP_FLAG_UP_CONFLICT; s.masked[b] = 1; }
+        if (b < g.B && s.conflicts[b] >= 1) { s.is_sat[b] = 0.f; s.flags[b] |= PDP_FLAG_UP_CONFLICT; s.masked[b] = 1; if (RB) rb_mark(A, (int)b); }
     }
 }
 __device__ __forceinline__ void fr_assign(const KArgs& A, int ulist, int clist_next, int epc, int vlist, int epv) {
@@ -959,6 +1053,7 @@ __device__ __forceinline__ void fr_peel_apply(const KArgs& A, int vlist, int vli
 
 // Called by ALL threads of the cooperative grid after select_and_fix_phase<frontier> and a grid barrier: clause list 0
 // and variable list 2 hold what the fixes touched (epochs epc0 / epv0, both already stored in the control block).
+template <bool RB = false>
 __device__ PDP_COLD void closure_frontier(const KArgs& A, cg::grid_group& grid) {
     const pdp_state& s = A.s;
     int epc = s.ctrl[CTRL_FR_EPC], epv = s.ctrl[CTRL_FR_EPV];
@@ -974,7 +1069,7 @@ __device__ PDP_COLD void closure_frontier(const KArgs& A, cg::grid_group& grid) 
         if (!s.ctrl[slot]) break;
         fr_find_conflicts(A, ul);
         grid.sync();
-        fr_apply_conflicts(A, cur, 2, epv);
+        fr_apply_conflicts<RB>(A, cur, 2, epv);
         grid.sync();
         ++epc;
         fr_assign(A, ul, cur ^ 1, epc, 2, epv);
@@ -1012,7 +1107,7 @@ __device__ PDP_COLD void closure_frontier(const KArgs& A, cg::grid_group& grid) 
         // per-round scratch is clean at a round boundary; the full scans finish the closure from the current masks
         if (gtid() == 0) { s.ctrl[CTRL_FLAG_A] = 0; s.ctrl[CTRL_FLAG_A + 1] = 0; s.ctrl[CTRL_FLAG_C] = 0; s.ctrl[CTRL_FLAG_C + 1] = 0; }
         grid.sync();
-        closure(A, grid);
+        closure<RB>(A, grid);
     }
 }
 
@@ -1149,7 +1244,9 @@ __device__ __forceinline__ void tiny_fix(const TinyView& t, int i, float sg) {
 // variables, group barriers instead of grid barriers; the histograms stay in global memory: the kernel's shared memory is
 // the sweep buffer's).  Called by the whole group after the scoring loop with !cnan and max c > 0.  score / av: the
 // problem's variables (local index); TINY: fixes go to the shared-memory view.  Returns false for K_b == 1 (the caller
-// applies the arg-max rule); otherwise fixes the taken variables and sets ls.fixed.
+// applies the arg-max rule); otherwise fixes the taken variables and sets ls.fixed (2: with rollback on, the state before
+// the fix is in the snapshot; the shared-memory tier leaves global memory as it was until its write-back, so it saves
+// is_sat only).
 template <bool TINY>
 __device__ __forceinline__ bool loc_select_fix(const KArgs& A, int b, int iter, const float* score, const uint8_t* av, int v0, int n,
                                             TinyView t, LocSmem& ls, int tid, int nthr, int bar_id) {
@@ -1164,9 +1261,18 @@ __device__ __forceinline__ bool loc_select_fix(const KArgs& A, int b, int iter, 
             sel_hist_var(s, valid, b, v0 + i, c, valid && av[i], first);
         }
         bar_sync(bar_id, nthr);
-        if (tid < 32) sel_decide(s, b, A.dec_fraction, first);
+        if (tid < 32) sel_decide(s, b, A.dec_fraction, first, A.rb.av != nullptr);
         bar_sync(bar_id, nthr);
         if (first && s.sel_need[b] < 0) return false;
+    }
+    const bool snap = A.rb.av != nullptr && !(s.flags[b] & PDP_FLAG_UP_CONFLICT);
+    if (snap) {
+        if (!TINY) {
+            for (int i = tid; i < n; i += nthr) rb_save_var(A, v0 + i);
+            for (int a = g.prob_fptr[b] + tid; a < g.prob_fptr[b + 1]; a += nthr) rb_save_clause(A, a);
+        }
+        if (tid == 0) A.rb.is_sat[b] = s.is_sat[b];
+        bar_sync(bar_id, nthr);
     }
     const int i0 = tid;
     bool any = false;
@@ -1181,7 +1287,7 @@ __device__ __forceinline__ bool loc_select_fix(const KArgs& A, int b, int iter, 
             if (k < A.trace_cap) { A.trace[3 * k] = iter; A.trace[3 * k + 1] = v0 + i; A.trace[3 * k + 2] = (int)sg; }
         }
     }
-    if (any) { ls.fixed = 1; s.masked[b] = 1; s.dirty[b] = 1; }
+    if (any) { ls.fixed = snap ? 2 : 1; s.masked[b] = 1; s.dirty[b] = 1; }
     bar_sync(bar_id, nthr);
     if (tid == 0) s.sel_need[b] = -1;
     return true;
@@ -1230,6 +1336,12 @@ __device__ __forceinline__ void loc_decimate_problem(const KArgs& A, int b, int 
     LSYNC();
     if (ls.fixed) loc_closure(A, b, v0, v1, f0, f1, ls, tid, nthr, bar_id);
     LSYNC();
+    if (FRAC && ls.fixed == 2 && (s.flags[b] & PDP_FLAG_UP_CONFLICT)) {   // conflict rollback
+        for (int a = f0 + tid; a < f1; a += nthr) rb_restore_clause(A, a);
+        for (int i = v0 + tid; i < v1; i += nthr) rb_restore_var(A, i);
+        LSYNC();   // everybody has read the conflict bit before it is cleared
+        if (tid == 0) rb_commit(A, b, iter);
+    }
     if (s.dirty[b]) {
         if (check_termination) {   // SatCNFEvaluator on _solution over the full formula, then trainer.py:150-162
             int n = 0;
@@ -1408,13 +1520,19 @@ __device__ __forceinline__ void loc_decimate_tiny(const KArgs& A, int b, int ite
             }
             if (tid == 0) s.masked[b] = 1;
         }
-        // ---- write back what changed: masks (+ edge-mask bits), solutions
-        for (int i = tid; i < n; i += nthr) {
-            if (!t.av[i] && s.av[v0 + i]) deactivate_variable(g, s, v0 + i);
-            s.sol[v0 + i] = t.sol[i];
+        if (FRAC && ls.fixed == 2 && (s.flags[b] & PDP_FLAG_UP_CONFLICT)) {
+            // conflict rollback: nothing is written back, global memory holds the state before the step
+            LSYNC();   // everybody has read the conflict bit before it is cleared
+            if (tid == 0) rb_commit(A, b, iter);
+        } else {
+            // ---- write back what changed: masks (+ edge-mask bits), solutions
+            for (int i = tid; i < n; i += nthr) {
+                if (!t.av[i] && s.av[v0 + i]) deactivate_variable(g, s, v0 + i);
+                s.sol[v0 + i] = t.sol[i];
+            }
+            for (int a = tid; a < m; a += nthr)
+                if (!t.af[a] && s.af[f0 + a]) deactivate_clause(g, s, f0 + a);
         }
-        for (int a = tid; a < m; a += nthr)
-            if (!t.af[a] && s.af[f0 + a]) deactivate_clause(g, s, f0 + a);
     }
     LSYNC();
     if (s.dirty[b]) {

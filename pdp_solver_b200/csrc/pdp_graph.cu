@@ -135,6 +135,10 @@ void carve(pdp_ctx* c, Carver& k, int64_t E, int64_t V, int64_t F, int64_t B) {
     s.sel_pref = k.take<unsigned long long>(B);
     s.sel_need = k.take<int32_t>(B);
     s.sel_sh = k.take<int32_t>(B);
+    s.rb_h = k.take<int32_t>(B);
+    s.rb_count = k.take<int32_t>(B);
+    s.rb_last = k.take<int32_t>(B);
+    s.rb_snap = k.take<uint8_t>(B);
     s.ctrl = k.take<int32_t>(CTRL_SIZE);
     s.sm_ctr = k.take<int32_t>(PDP_MAX_SMS);
     s.asg = k.take<int8_t>(V);
@@ -254,6 +258,7 @@ __global__ void k_reset_state(pdp_graph g, pdp_state s, int64_t V, int64_t F, in
             s.st_max[2 * i] = 0u; s.st_max[2 * i + 1] = 0u; s.st_min[2 * i] = 0x7f800000u; s.st_min[2 * i + 1] = 0x7f800000u;
             s.st_nan[i] = 0u; s.c_max[i] = 0u; s.c_min[i] = 0x7f800000u; s.c_nan[i] = 0u;
             s.sel_need[i] = -1; s.sel_sh[i] = 0; s.sel_pref[i] = 0ull;
+            s.rb_h[i] = 0; s.rb_count[i] = 0; s.rb_last[i] = 0; s.rb_snap[i] = 0;
             for (int j = 0; j < PDP_SEL_BINS; ++j) s.sel_hist[i * PDP_SEL_BINS + j] = 0u;
         }
         if (i < CTRL_SIZE) s.ctrl[i] = (i == CTRL_NUM_ACTIVE) ? (int32_t)B

@@ -102,8 +102,11 @@ __device__ __forceinline__ void select_and_fix_phase(const KArgs& A, int iter, b
 // de-activated iff it holds a newly true literal (_set_variable_core, solver.py:205-226).
 __device__ __forceinline__ void frac_select_and_fix(const KArgs& A, cg::grid_group& grid, int iter, bool frontier) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    sel_grid(A, grid, CoefScore{s}, A.dec_fraction);
+    const bool rb = A.rb.av != nullptr;
+    sel_grid(A, grid, CoefScore{s}, A.dec_fraction, rb);
+    if (rb) rb_snapshot_grid(A);
     select_and_fix_phase(A, iter, frontier);
+    if (rb) grid.sync();   // the snapshots are complete before the top-K fixes
     const int slot = CTRL_FIX + (iter & 1);
     const int epc = s.ctrl[CTRL_FR_EPC], epv = s.ctrl[CTRL_FR_EPV];
     for (int64_t base = gwarp() * 32; base < g.V; base += gwarps() * 32) {
@@ -269,8 +272,13 @@ k_sp_run(const __grid_constant__ KArgs A, const __grid_constant__ pdp_sp_params 
             GRID_SYNC();
             LOOP_T(25);
             if (s.ctrl[CTRL_FIX + (iter & 1)]) {
-                if (frontier) closure_frontier(A, grid);
-                else closure(A, grid);
+                if (frontier) closure_frontier<FRAC>(A, grid);
+                else closure<FRAC>(A, grid);
+            }
+            if (FRAC && s.ctrl[CTRL_RB]) {   // conflict rollback: some top-K step ended in a conflict
+                rb_restore_grid(A, iter);
+                GRID_SYNC();
+                if (gtid() == 0) s.ctrl[CTRL_RB] = 0;   // (read by everybody before the barrier)
             }
             LOOP_T(26);
         }
@@ -352,7 +360,7 @@ __global__ void __launch_bounds__(256) k_decimation_select(const __grid_constant
     grid.sync();
     argmax_phase(A, CoefGiven{coeff});
     grid.sync();
-    if (A.dec_fraction > 0.f) sel_grid(A, grid, CoefGiven{coeff}, A.dec_fraction);
+    if (A.dec_fraction > 0.f) sel_grid(A, grid, CoefGiven{coeff}, A.dec_fraction, false);
     WARP_STRIDED(i, g.V) {
         if (i >= g.V) continue;
         const int b = g.bvm[i];
@@ -366,6 +374,19 @@ __global__ void __launch_bounds__(256) k_decimation_select(const __grid_constant
     WARP_STRIDED(b, g.B) {   // the per-iteration scratch of the fused loop back to its resting state
         if (b >= g.B) continue;
         s.conv[b] = 0; s.c_max[b] = 0u; s.c_min[b] = 0x7f800000u; s.c_nan[b] = 0u; s.arg_idx[b] = 0x7fffffff; s.sel_need[b] = -1;
+    }
+}
+
+// pdp_debug_check_edge_mask: edges whose mask bit disagrees with the node masks, per layout
+__global__ void __launch_bounds__(256) k_check_edge_mask(const __grid_constant__ KArgs A, int32_t* errs) {
+    const pdp_graph& g = A.g; const pdp_state& s = A.s;
+    WARP_STRIDED(i, g.V) {
+        if (i >= g.V) continue;
+        for (int p = g.var_ptr[i]; p < g.var_ptr[i + 1]; ++p) {
+            const bool masked = !(s.av[i] && s.af[g.v_cls[p]]);
+            if (mbit(g.vmask, g.p_vpos[p]) != masked) atomicAdd(&errs[0], 1);
+            if (mbit(g.qmask, g.p_qpos[p]) != masked) atomicAdd(&errs[1], 1);
+        }
     }
 }
 
@@ -394,11 +415,27 @@ extern "C" int pdp_set_trace_buffer(pdp_ctx* ctx, int32_t* d_trace, int32_t capa
 #ifndef PDP_STAGGER_V
 #define PDP_STAGGER_V 0
 #endif
+// the snapshot buffer of the conflict rollback: sol [V], is_sat [B] (fp32), av [V], af [F] (bytes)
+struct RbLayout { size_t is_sat, av, af, total; };
+static RbLayout rb_layout(int64_t V, int64_t F, int64_t B) {
+    auto up = [](int64_t x) { return ((size_t)(x > 0 ? x : 0) + 255) & ~(size_t)255; };
+    RbLayout l;
+    l.is_sat = up(4 * V); l.av = l.is_sat + up(4 * B); l.af = l.av + up(V); l.total = l.af + up(F);
+    return l;
+}
+
 static KArgs make_args(pdp_ctx* ctx) {
     KArgs A;
     A.g = ctx->g; A.s = ctx->s; A.trace = ctx->trace; A.trace_cap = ctx->trace_cap;
     A.stagger_c = PDP_STAGGER_C; A.stagger_v = PDP_STAGGER_V;
     A.dec_fraction = ctx->dec_fraction;
+    A.rb.sol = nullptr; A.rb.is_sat = nullptr; A.rb.av = nullptr; A.rb.af = nullptr;
+    if (ctx->rb_scratch) {
+        const RbLayout l = rb_layout(ctx->g.V, ctx->g.F, ctx->g.B);
+        unsigned char* base = (unsigned char*)ctx->rb_scratch;
+        A.rb.sol = (float*)base; A.rb.is_sat = (float*)(base + l.is_sat);
+        A.rb.av = base + l.av; A.rb.af = base + l.af;
+    }
     if (const char* e = getenv("PDP_B200_STAGGER_C")) A.stagger_c = atoi(e);
     if (const char* e = getenv("PDP_B200_STAGGER_V")) A.stagger_v = atoi(e);
     return A;
@@ -482,6 +519,45 @@ extern "C" int pdp_decimation_select(pdp_ctx* ctx, const float* d_coeff, const f
     int blocks = coop_blocks(ctx, k_decimation_select);
     if (blocks < 1) { pdp_set_error("pdp_decimation_select: occupancy query failed"); return PDP_ERR_CUDA; }
     PDP_CUDA_CHECK(cudaLaunchCooperativeKernel((void*)k_decimation_select, dim3(blocks), dim3(256), args, 0, (cudaStream_t)stream_));
+    PDP_LAUNCH_CHECK(ctx);
+    return PDP_OK;
+}
+
+// conflict rollback (pdp_b200.h)
+extern "C" size_t pdp_rollback_scratch_bytes(int64_t V, int64_t F, int64_t B) {
+    if (V < 0 || F < 0 || B < 0) return 0;
+    return rb_layout(V, F, B).total;
+}
+
+extern "C" int pdp_set_conflict_rollback(pdp_ctx* ctx, void* d_scratch, size_t bytes) {
+    if (!ctx) { pdp_set_error("pdp_set_conflict_rollback: null context"); return PDP_ERR_ARG; }
+    if (d_scratch) {
+        const size_t need = rb_layout(ctx->g.V, ctx->g.F, ctx->g.B).total;
+        if (bytes < need) {
+            pdp_set_error("pdp_set_conflict_rollback: scratch of %zu bytes, %zu needed", bytes, need);
+            return PDP_ERR_WORKSPACE;
+        }
+        if ((uintptr_t)d_scratch % 16) { pdp_set_error("pdp_set_conflict_rollback: scratch not 16-byte aligned"); return PDP_ERR_ARG; }
+    }
+    ctx->rb_scratch = d_scratch;
+    return PDP_OK;
+}
+
+extern "C" int pdp_get_rollbacks(pdp_ctx* ctx, int32_t* d_count, int32_t* d_last_iter, void* stream_) {
+    if (!ctx) { pdp_set_error("pdp_get_rollbacks: null context"); return PDP_ERR_ARG; }
+    cudaStream_t stream = (cudaStream_t)stream_;
+    const size_t n = sizeof(int32_t) * (size_t)ctx->g.B;
+    if (d_count && n) PDP_CUDA_CHECK(cudaMemcpyAsync(d_count, ctx->s.rb_count, n, cudaMemcpyDeviceToDevice, stream));
+    if (d_last_iter && n) PDP_CUDA_CHECK(cudaMemcpyAsync(d_last_iter, ctx->s.rb_last, n, cudaMemcpyDeviceToDevice, stream));
+    return PDP_OK;
+}
+
+extern "C" int pdp_debug_check_edge_mask(pdp_ctx* ctx, int32_t* d_errs, void* stream_) {
+    if (!ctx || !d_errs) { pdp_set_error("pdp_debug_check_edge_mask: null argument"); return PDP_ERR_ARG; }
+    cudaStream_t stream = (cudaStream_t)stream_;
+    PDP_CUDA_CHECK(cudaMemsetAsync(d_errs, 0, 2 * sizeof(int32_t), stream));
+    KArgs A = make_args(ctx);
+    k_check_edge_mask<<<pdp_grid(ctx->g.V, 256, ctx->num_sms), 256, 0, stream>>>(A, d_errs);
     PDP_LAUNCH_CHECK(ctx);
     return PDP_OK;
 }

@@ -131,6 +131,12 @@ class Context(object):
         self._check(self._L.pdp_debug_check_layout(self._h, _ptr(errs), ctypes.byref(info), _stream()), "pdp_debug_check_layout")
         return errs.cpu().tolist(), dict(blocked=int(info[0]) & 15, ctas=int(info[0]) >> 4, nvb=int(info[1]), ncb=int(info[2]), sv=int(info[3]), sc=int(info[4]))
 
+    def check_edge_mask(self):
+        """[variable-side, clause-side] counts of edge-mask bits that disagree with the node masks (tests)"""
+        errs = self._new(2, dtype=torch.int32)
+        self._check(self._L.pdp_debug_check_edge_mask(self._h, _ptr(errs), _stream()), "pdp_debug_check_edge_mask")
+        return errs.cpu().tolist()
+
     def launch_count(self):
         return int(self._L.pdp_launch_count(self._h))
 
@@ -259,6 +265,25 @@ class Context(object):
         self._check(self._L.pdp_decimation_select(self._h, _ptr(c), _ptr(sc), _ptr(ps), float(fraction), _ptr(out), _stream()),
                     "pdp_decimation_select")
         return out
+
+    def enable_conflict_rollback(self, on=True):
+        """Conflict rollback for SP-inspired decimation in sp_run (include/pdp_b200.h, pdp_set_conflict_rollback): a step of
+        K_b >= 2 variables that ends in a unit-propagation conflict is undone and the problem's later steps are halved.  The
+        context allocates the snapshot buffer; on=False turns rollback off and frees it.  pdp_reset keeps the setting."""
+        if not on:
+            self._check(self._L.pdp_set_conflict_rollback(self._h, None, 0), "pdp_set_conflict_rollback")
+            self._rb_scratch = None
+            return
+        nbytes = int(self._L.pdp_rollback_scratch_bytes(self.V, self.F, self.B))
+        scratch = self._new(max(nbytes, 1), dtype=torch.uint8)
+        self._check(self._L.pdp_set_conflict_rollback(self._h, _ptr(scratch), nbytes), "pdp_set_conflict_rollback")
+        self._rb_scratch = scratch
+
+    def rollbacks(self):
+        """(count int32 [B], iteration of the last rollback int32 [B], 0 = none) since pdp_reset"""
+        count, last = self._new(self.B, dtype=torch.int32), self._new(self.B, dtype=torch.int32)
+        self._check(self._L.pdp_get_rollbacks(self._h, _ptr(count), _ptr(last), _stream()), "pdp_get_rollbacks")
+        return count, last
 
     def enable_trace(self, capacity=1 << 16):
         self._trace = torch.zeros(capacity, 3, dtype=torch.int32, device=self.device)

@@ -49,6 +49,15 @@ def check_decimation_fraction(fraction):
     return f
 
 
+def check_conflict_rollback(conflict_rollback, fraction):
+    """conflict rollback of SP-inspired decimation: a bool, and True only with a decimation fraction > 0"""
+    if not isinstance(conflict_rollback, bool):
+        raise ValueError("conflict_rollback must be True or False, got %r" % (conflict_rollback,))
+    if conflict_rollback and fraction == 0.0:
+        raise ValueError("conflict_rollback needs a decimation_fraction > 0 (one variable per step is never rolled back)")
+    return conflict_rollback
+
+
 class NeuralDecimator(nn.Module):
     """The neural (non-greedy) decimator of `p-nd-np` / `np-nd-np` (reference pdp_decimate.py:21-100): one GRU
     cell per message direction over the edges; same sub-module names (state-dict compatible).  The GRU cells run on the
@@ -121,16 +130,19 @@ class SequentialDecimator(nn.Module):
 
     decimation_fraction f > 0 turns it into SP-inspired decimation: a selected problem with A active variables fixes
     the max(1, floor(f * A)) variables with the largest |score| at once (include/pdp_b200.h, pdp_decimation_select).
-    It is a plain attribute, not a buffer: state dicts of the reference load unchanged.
+    conflict_rollback (needs f > 0) undoes a step of two or more variables that ends in a unit-propagation conflict and
+    halves the problem's later steps (pdp_set_conflict_rollback).  Both are plain attributes, not buffers: state dicts of
+    the reference load unchanged.
 
     Its statistics, per-problem decisions, scoring, arg-max, variable fixing and the following unit
     propagation / peeling closure all live inside the persistent kernel launched by
     PropagatorDecimatorSolverBase.forward (pdp_sp_run); the module keeps the hyper-parameters and the
     initial-state contract."""
 
-    def __init__(self, device, message_dimension, scorer, tolerance, t_max, decimation_fraction=0.0):
+    def __init__(self, device, message_dimension, scorer, tolerance, t_max, decimation_fraction=0.0, conflict_rollback=False):
         super(SequentialDecimator, self).__init__()
         self._decimation_fraction = check_decimation_fraction(decimation_fraction)
+        self._conflict_rollback = check_conflict_rollback(conflict_rollback, self._decimation_fraction)
         self._device = device
         self._tolerance = tolerance
         self._scorer = scorer

@@ -264,6 +264,8 @@ class PropagatorDecimatorSolverBase(nn.Module):
             ctx.load_state(init_propagator_state, init_decimator_state[:2])
         b = sat_problem._batch_replication
         ctx.set_decimation_fraction(dec._decimation_fraction)
+        if dec._conflict_rollback:
+            ctx.enable_conflict_rollback()
         if check_termination is None or _is_standard_termination(check_termination):
             self.last_iterations = ctx.sp_run(iteration_num, dec._tolerance, dec._t_max,
                                               check_termination is not None, b, self._propagator.pi_value())
@@ -374,14 +376,16 @@ class PropagatorDecimatorSolverBase(nn.Module):
 class SurveyPropagatorSolver(PropagatorDecimatorSolverBase):
     "The classical SP-guided decimation solver, model type `p-d-p` (reference solver.py:567-578)."
 
-    def __init__(self, device, name, tolerance, t_max, local_search_iterations=0, epsilon=0.05, decimation_fraction=0.0):
+    def __init__(self, device, name, tolerance, t_max, local_search_iterations=0, epsilon=0.05, decimation_fraction=0.0,
+                 conflict_rollback=False):
         super(SurveyPropagatorSolver, self).__init__(
             device=device, name=name,
             propagator=pdp_propagate.SurveyPropagator(device, decimator_dimension=1, include_adaptors=False),
             decimator=pdp_decimate.SequentialDecimator(
                 device, message_dimension=(3, 1),
                 scorer=pdp_predict.SurveyScorer(device, message_dimension=1, include_adaptors=False),
-                tolerance=tolerance, t_max=t_max, decimation_fraction=decimation_fraction),
+                tolerance=tolerance, t_max=t_max, decimation_fraction=decimation_fraction,
+                conflict_rollback=conflict_rollback),
             predictor=pdp_predict.IdentityPredictor(device=device, random_fill=True),
             local_search_iterations=local_search_iterations, epsilon=epsilon)
 

@@ -50,6 +50,11 @@ class SatFactorGraphTrainer(FactorGraphTrainerBase):
         frac = pdp_decimate.check_decimation_fraction(config.get("decimation_fraction", 0.0))
         if frac != 0.0 and t not in ("p-d-p", "np-d-np"):
             raise ValueError("decimation_fraction applies to model types p-d-p and np-d-np only, not %r" % (t,))
+        # conflict rollback of SP-inspired decimation (optional key): p-d-p only (np-d-np decimates step-wise on the host)
+        rollback = config.get("conflict_rollback", False)
+        if rollback is not False and t != "p-d-p":
+            raise ValueError("conflict_rollback applies to model type p-d-p only, not %r" % (t,))
+        rollback = pdp_decimate.check_conflict_rollback(rollback, frac)
         neural = dict(edge_dimension=config.get("edge_feature_dim"), meta_data_dimension=config.get("meta_feature_dim"),
                       mem_hidden_dimension=config.get("mem_hidden_dim"), agg_hidden_dimension=config.get("agg_hidden_dim"),
                       mem_agg_hidden_dimension=config.get("mem_agg_hidden_dim"), dropout=config.get("dropout", 0),
@@ -74,7 +79,8 @@ class SatFactorGraphTrainer(FactorGraphTrainerBase):
         elif t == "p-d-p":
             model = solver.SurveyPropagatorSolver(device=self._device, name=config["model_name"],
                                                   tolerance=config["tolerance"], t_max=config["t_max"],
-                                                  local_search_iterations=w, epsilon=eps, decimation_fraction=frac)
+                                                  local_search_iterations=w, epsilon=eps, decimation_fraction=frac,
+                                                  conflict_rollback=rollback)
         elif t == "walk-sat":
             model = solver.WalkSATSolver(device=self._device, name=config["model_name"], iteration_num=w, epsilon=eps)
         elif t == "reinforce":
