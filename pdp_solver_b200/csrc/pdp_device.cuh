@@ -504,6 +504,13 @@ __device__ __forceinline__ void fix_variable(const pdp_graph& g, const pdp_state
     s.sol[i] = (sg + 1.f) / 2.0f;
 }
 
+// one event (iteration, variable, sign) of the optional decimation trace
+__device__ __forceinline__ void record_fix(const KArgs& A, int iter, int i, float sg) {
+    if (!A.trace) return;
+    const int k = atomicAdd(&A.s.ctrl[CTRL_TRACE_LEN], 1);
+    if (k < A.trace_cap) { A.trace[3 * k] = iter; A.trace[3 * k + 1] = i; A.trace[3 * k + 2] = (int)sg; }
+}
+
 // ------------------------------------------------------------------------------------------------
 // Conflict rollback (pdp_set_conflict_rollback).  A decimation step of problem b with K_b >= 2 and a clear conflict bit
 // first copies b's node masks, solution and is_sat to the caller's snapshot buffer (one byte per node mask, indexed like the
@@ -552,6 +559,47 @@ __device__ __forceinline__ void rb_commit(const KArgs& A, int b, int iter) {
 }
 
 // ------------------------------------------------------------------------------------------------
+// clause and variable tests of the closures and the CNF check.  A clause -> variable CSR word W is the variable's index
+// with the literal's sign in the top bit: 32 bits in g.c_var, 16 bits (local indices) in the shared-memory tier.
+// ------------------------------------------------------------------------------------------------
+// literal of sign sgn (+-1) true under the solution value p (SatCNFEvaluator, util.py:210-236)
+__device__ __forceinline__ bool literal_true(float sgn, float p) {
+    float ev = sgn * p;
+    ev = ev + (1.f - sgn) / 2.f;
+    return ev > 0.5f;
+}
+// clause [beg, end) of the CSR holds a true literal under sol
+template <typename W>
+__device__ __forceinline__ bool clause_satisfied(const W* cvar, int beg, int end, const float* sol) {
+    constexpr uint32_t sign = 1u << (8 * sizeof(W) - 1);
+    for (int c = beg; c < end; ++c) {
+        const uint32_t w = cvar[c];
+        if (literal_true((w & sign) ? -1.f : 1.f, sol[w & (sign - 1u)])) return true;
+    }
+    return false;
+}
+// clause [beg, end) of the CSR has exactly one active variable: j, and whether it occurs negated
+template <typename W>
+__device__ __forceinline__ bool clause_unit(const W* cvar, int beg, int end, const uint8_t* av, int& j, bool& neg) {
+    constexpr uint32_t sign = 1u << (8 * sizeof(W) - 1);
+    int deg = 0; uint32_t hit = 0;
+    for (int c = beg; c < end; ++c) {
+        const uint32_t w = cvar[c];
+        if (av[w & (sign - 1u)]) { ++deg; hit = w; }
+    }
+    j = (int)(hit & (sign - 1u)); neg = (hit & sign) != 0u;
+    return deg == 1;
+}
+// variable i occurs in the active clauses with one sign only, or in none: val = the solution value peeling gives it
+__device__ __forceinline__ bool var_pure(const pdp_graph& g, const uint8_t* af, int i, float& val) {
+    int deg = 0, sdeg = 0;
+    for (int p = g.var_ptr[i]; p < g.var_ptr[i + 1]; ++p)
+        if (af[g.v_cls[p]]) { ++deg; sdeg += (g.v_cedge[p] & PDP_SIGN_BIT) ? -1 : 1; }
+    val = ((sdeg > 0 ? 1.f : (sdeg < 0 ? -1.f : 0.f)) + 1.f) / 2.0f;
+    return deg == abs(sdeg);
+}
+
+// ------------------------------------------------------------------------------------------------
 // unit propagation round (solver.py:228-273), split at its data dependencies
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void up_find_units(const KArgs& A, int flag_slot) {
@@ -561,17 +609,11 @@ __device__ __forceinline__ void up_find_units(const KArgs& A, int flag_slot) {
         if (!s.af[a]) continue;
         const int b = g.bfm[a];
         if (!s.dirty[b]) continue;
-        const int beg = g.cl_ptr[a], end = g.cl_ptr[a + 1];
-        int deg = 0; uint32_t hit = 0;
-        for (int c = beg; c < end; ++c) {
-            const uint32_t w = g.c_var[c];
-            if (s.av[w & PDP_IDX_MASK]) { ++deg; hit = w; }
-        }
-        if (deg == 1) {
+        int j; bool neg;
+        if (clause_unit(g.c_var, g.cl_ptr[a], g.cl_ptr[a + 1], s.av, j, neg)) {
             s.single[a] = 1;
-            const int j = (int)(hit & PDP_IDX_MASK);
             atomicAdd(&s.up_cnt[j], 1);
-            atomicAdd(&s.up_ev[j], (hit & PDP_SIGN_BIT) ? -1 : 1);
+            atomicAdd(&s.up_ev[j], neg ? -1 : 1);
             s.ctrl[flag_slot] = 1;
         }
     }
@@ -636,14 +678,10 @@ __device__ __forceinline__ void peel_find(const KArgs& A, int flag_slot) {
         if (!s.av[i]) continue;
         const int b = g.bvm[i];
         if (!s.dirty[b]) continue;
-        const int beg = g.var_ptr[i], end = g.var_ptr[i + 1];
-        int deg = 0, sdeg = 0;
-        for (int p = beg; p < end; ++p) {
-            if (s.af[g.v_cls[p]]) { ++deg; sdeg += (g.v_cedge[p] & PDP_SIGN_BIT) ? -1 : 1; }
-        }
-        if (deg == abs(sdeg)) {
+        float val;
+        if (var_pure(g, s.af, (int)i, val)) {
             s.pure[i] = 1;
-            s.sol[i] = ((sdeg > 0 ? 1.f : (sdeg < 0 ? -1.f : 0.f)) + 1.f) / 2.0f;
+            s.sol[i] = val;
             s.ctrl[flag_slot] = 1;
         }
     }
@@ -949,20 +987,14 @@ __device__ __forceinline__ void fr_find_units(const KArgs& A, int clist, int uli
         if (x >= n) continue;
         const int a = s.fr_list[clist][x];
         if (!s.af[a]) continue;
-        const int beg = g.cl_ptr[a], end = g.cl_ptr[a + 1];
-        int deg = 0; uint32_t hit = 0;
-        for (int c = beg; c < end; ++c) {
-            const uint32_t w = g.c_var[c];
-            if (s.av[w & PDP_IDX_MASK]) { ++deg; hit = w; }
-        }
-        if (deg == 1) {
+        int j; bool neg;
+        if (clause_unit(g.c_var, g.cl_ptr[a], g.cl_ptr[a + 1], s.av, j, neg)) {
             s.single[a] = 1;
-            const int j = (int)(hit & PDP_IDX_MASK);
             if (atomicAdd(&s.up_cnt[j], 1) == 0) {
                 const int k = atomicAdd(&s.ctrl[CTRL_FR_NU + ulist], 1);
                 if (k < s.fr_cap) s.fr_unit[ulist][k] = j; else s.ctrl[CTRL_FR_OVER] = 1;
             }
-            atomicAdd(&s.up_ev[j], (hit & PDP_SIGN_BIT) ? -1 : 1);
+            atomicAdd(&s.up_ev[j], neg ? -1 : 1);
             s.ctrl[flag_slot] = 1;
         }
     }
@@ -1021,14 +1053,10 @@ __device__ __forceinline__ void fr_peel_find(const KArgs& A, int vlist, int flag
         if (x >= n) continue;
         const int i = s.fr_list[vlist][x];
         if (!s.av[i]) continue;
-        const int beg = g.var_ptr[i], end = g.var_ptr[i + 1];
-        int deg = 0, sdeg = 0;
-        for (int p = beg; p < end; ++p) {
-            if (s.af[g.v_cls[p]]) { ++deg; sdeg += (g.v_cedge[p] & PDP_SIGN_BIT) ? -1 : 1; }
-        }
-        if (deg == abs(sdeg)) {
+        float val;
+        if (var_pure(g, s.af, i, val)) {
             s.pure[i] = 1;
-            s.sol[i] = ((sdeg > 0 ? 1.f : (sdeg < 0 ? -1.f : 0.f)) + 1.f) / 2.0f;
+            s.sol[i] = val;
             s.ctrl[flag_slot] = 1;
         }
     }
@@ -1118,276 +1146,143 @@ __device__ PDP_COLD void closure_frontier(const KArgs& A, cg::grid_group& grid) 
 // n ~ 100 problems per batch) a CTA does all of it with block barriers, where the grid-wide phases above need a
 // few dozen grid barriers per iteration.  Same arithmetic and the same synchronous rounds as the grid-wide
 // phases (which stay for large problems and batch replication).
+// One body, loc_decimate, runs on a view of the problem (local indices i in [0, n), a in [0, m)): LocGlobal works in place
+// on the state in global memory, TinyView on a copy staged in shared memory.  A view holds the node arrays and provides the
+// clause and variable tests, the fixes, de-activations and scores, and the conflict rollback's save (before a top-K fix),
+// restore (after a step that conflicted) and write_back (after any other step).
 // ------------------------------------------------------------------------------------------------
 struct LocSmem {
     uint32_t cmax, cmin, cnan;
     int arg, flag, conflicts, nunsat, fixed;
 };
 
-__device__ __forceinline__ bool literal_true(float sgn, float p);
+// what both views hold: problem b (nodes [v0, v0 + n), [f0, f0 + m)), the surveys eta[w], and the node arrays
+struct LocNodes {
+    const KArgs& A;
+    int b, v0, f0, n, m, w;
+    float pi;
+    uint8_t *av, *af, *pure, *single;
+    float *sol, *score;
+    int *cnt, *ev;      // unit clauses pointing at the variable, signed sum of those
+};
 
-#define LSYNC() bar_sync(bar_id, nthr)
-__device__ __forceinline__ void loc_closure(const KArgs& A, int b, int v0, int v1, int f0, int f1, LocSmem& ls, int tid, int nthr, int bar_id) {
+// the problem in place: slices of the state, the global CSR / CSC; de-activations set the edge-mask bits
+struct LocGlobal : LocNodes {
+    __device__ __forceinline__ float score_of(int i) const { return score_variable(A.g, A.s, A.s.eta[w], v0 + i, pi); }
+    __device__ __forceinline__ bool is_unit(int a, int& j, bool& neg) const {
+        const bool u = clause_unit(A.g.c_var, A.g.cl_ptr[f0 + a], A.g.cl_ptr[f0 + a + 1], A.s.av, j, neg);
+        j -= v0;
+        return u;
+    }
+    __device__ __forceinline__ bool is_pure(int i, float& val) const { return var_pure(A.g, A.s.af, v0 + i, val); }
+    __device__ __forceinline__ bool satisfied(int a) const {
+        return clause_satisfied(A.g.c_var, A.g.cl_ptr[f0 + a], A.g.cl_ptr[f0 + a + 1], A.s.sol);
+    }
+    __device__ __forceinline__ void fix(int i, float sg) const { fix_variable(A.g, A.s, v0 + i, sg); }
+    __device__ __forceinline__ void drop_clause(int a) const { deactivate_clause(A.g, A.s, f0 + a); }
+    __device__ __forceinline__ void drop_var(int i) const { deactivate_variable(A.g, A.s, v0 + i); }
+    __device__ __forceinline__ void save(int tid, int nthr) const {
+        for (int i = tid; i < n; i += nthr) rb_save_var(A, v0 + i);
+        for (int a = tid; a < m; a += nthr) rb_save_clause(A, f0 + a);
+    }
+    __device__ __forceinline__ void restore(int tid, int nthr) const {
+        for (int a = tid; a < m; a += nthr) rb_restore_clause(A, f0 + a);
+        for (int i = tid; i < n; i += nthr) rb_restore_var(A, v0 + i);
+    }
+    __device__ __forceinline__ void write_back(int, int) const {}
+};
+__device__ __forceinline__ LocGlobal loc_global(const KArgs& A, int b, int w, float pi) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    for (;;) {   // unit propagation rounds, solver.py:234-273
-        if (tid == 0) { ls.flag = 0; ls.conflicts = 0; }
-        LSYNC();
-        for (int a = f0 + tid; a < f1; a += nthr) {
-            if (!s.af[a]) continue;
-            int deg = 0; uint32_t hit = 0;
-            for (int c = g.cl_ptr[a]; c < g.cl_ptr[a + 1]; ++c) {
-                const uint32_t w = g.c_var[c];
-                if (s.av[w & PDP_IDX_MASK]) { ++deg; hit = w; }
-            }
-            if (deg == 1) {
-                s.single[a] = 1;
-                const int j = (int)(hit & PDP_IDX_MASK);
-                atomicAdd(&s.up_cnt[j], 1);
-                atomicAdd(&s.up_ev[j], (hit & PDP_SIGN_BIT) ? -1 : 1);
-                ls.flag = 1;
-            }
-        }
-        LSYNC();
-        if (!ls.flag) break;
-        for (int i = v0 + tid; i < v1; i += nthr) {
-            const int cnt = s.up_cnt[i];
-            if (cnt > 0 && abs(s.up_ev[i]) != cnt) atomicAdd(&ls.conflicts, 1);
-        }
-        LSYNC();
-        const int nc = ls.conflicts;   // the `== 1` quirk of solver.py:257,261
-        for (int a = f0 + tid; a < f1; a += nthr) {
-            if (s.single[a]) { deactivate_clause(g, s, a); s.single[a] = 0; s.masked[b] = 1; }
-            else if (s.af[a] && nc == 1) deactivate_clause(g, s, a);
-        }
-        for (int i = v0 + tid; i < v1; i += nthr)
-            if (s.av[i] && nc == 1) deactivate_variable(g, s, i);
-        if (tid == 0 && nc >= 1) { s.is_sat[b] = 0.f; s.flags[b] |= PDP_FLAG_UP_CONFLICT; s.masked[b] = 1; }
-        LSYNC();
-        for (int i = v0 + tid; i < v1; i += nthr) {
-            const int cnt = s.up_cnt[i];
-            if (cnt > 0) {
-                const int ev = s.up_ev[i];
-                s.up_cnt[i] = 0; s.up_ev[i] = 0;
-                if (s.av[i] && abs(ev) == cnt) fix_variable(g, s, i, ev > 0 ? 1.f : -1.f);
-            }
-        }
-        LSYNC();
-    }
-    for (;;) {   // pure-literal peeling rounds, solver.py:188-203
-        LSYNC();
-        if (tid == 0) ls.flag = 0;
-        LSYNC();
-        for (int i = v0 + tid; i < v1; i += nthr) {
-            if (!s.av[i]) continue;
-            int deg = 0, sdeg = 0;
-            for (int p = g.var_ptr[i]; p < g.var_ptr[i + 1]; ++p)
-                if (s.af[g.v_cls[p]]) { ++deg; sdeg += (g.v_cedge[p] & PDP_SIGN_BIT) ? -1 : 1; }
-            if (deg == abs(sdeg)) {
-                s.pure[i] = 1;
-                s.sol[i] = ((sdeg > 0 ? 1.f : (sdeg < 0 ? -1.f : 0.f)) + 1.f) / 2.0f;
-                ls.flag = 1;
-            }
-        }
-        LSYNC();
-        if (!ls.flag) break;
-        for (int i = v0 + tid; i < v1; i += nthr) {
-            if (!s.pure[i]) continue;
-            s.pure[i] = 0;
-            for (int p = g.var_ptr[i]; p < g.var_ptr[i + 1]; ++p) {
-                const int a = g.v_cls[p];
-                if (s.af[a]) deactivate_clause(g, s, a);
-            }
-            deactivate_variable(g, s, i);
-            s.masked[b] = 1;
-        }
-    }
+    const int v0 = g.prob_vptr[b], f0 = g.prob_fptr[b];
+    return LocGlobal{{A, b, v0, f0, g.prob_vptr[b + 1] - v0, g.prob_fptr[b + 1] - f0, w, pi, s.av + v0, s.af + f0, s.pure + v0,
+                      s.single + f0, s.sol + v0, s.score + v0, s.up_cnt + v0, s.up_ev + v0}};
 }
 
 // ------------------------------------------------------------------------------------------------
 // shared-memory tier of the CTA-local decimation.  A problem whose masks, adjacency (16-bit local indices) and
 // scratch fit the group's share of the (idle) sweep buffer is decimated entirely in shared memory: the closure
 // is a chain of dozens of dependent rounds, each a couple of microseconds through global memory and tens of
-// nanoseconds here.  Same rounds, same arithmetic as loc_closure; what changed is written back at the end.
+// nanoseconds here.  Global memory keeps the problem as it was until the write-back at the end.
 // ------------------------------------------------------------------------------------------------
-struct TinyView {
-    uint8_t *av, *af, *pure, *single;
-    float *sol, *score;
-    int *cnt, *ev;
+struct TinyView : LocNodes {
     uint16_t *clp, *cvar, *vp, *vcls;   // local CSR / CSC: pointers, (local index | sign << 15)
+    const float* eta_s;                 // the problem's surveys in variable-major order (null: not staged)
+    __device__ __forceinline__ float score_of(int i) const {
+        if (!eta_s) return score_variable(A.g, A.s, A.s.eta[w], v0 + i, pi);
+        float ps = 0.f, ns = 0.f, as = 0.f;   // score_variable on the staged copies (same order, same operations)
+        for (int p = vp[i]; p < vp[i + 1]; ++p) {
+            const uint32_t cw = vcls[p];
+            const float f = L10(1.f - eta_s[p]) * (float)af[cw & 0x7fffu];
+            const bool neg = (cw & 0x8000u) != 0u;
+            ps += (neg ? 0.f : 1.f) * f;
+            ns += (neg ? 1.f : 0.f) * f;
+            as += f;
+        }
+        return sp_score_tail(ps, ns, as, 0.f, 0.f);
+    }
+    __device__ __forceinline__ bool is_unit(int a, int& j, bool& neg) const { return clause_unit(cvar, clp[a], clp[a + 1], av, j, neg); }
+    __device__ __forceinline__ bool is_pure(int i, float& val) const {
+        int deg = 0, sdeg = 0;
+        for (int p = vp[i]; p < vp[i + 1]; ++p) {
+            const uint32_t cw = vcls[p];
+            if (af[cw & 0x7fffu]) { ++deg; sdeg += (cw & 0x8000u) ? -1 : 1; }
+        }
+        val = ((sdeg > 0 ? 1.f : (sdeg < 0 ? -1.f : 0.f)) + 1.f) / 2.0f;
+        return deg == abs(sdeg);
+    }
+    __device__ __forceinline__ bool satisfied(int a) const { return clause_satisfied(cvar, clp[a], clp[a + 1], sol); }
+    __device__ __forceinline__ void fix(int i, float sg) const {
+        for (int p = vp[i]; p < vp[i + 1]; ++p) {
+            const uint32_t w = vcls[p];
+            const float lit = (w & 0x8000u) ? -1.f : 1.f;
+            if (lit * sg > 0.f) af[w & 0x7fffu] = 0;
+        }
+        av[i] = 0;
+        sol[i] = (sg + 1.f) / 2.0f;
+    }
+    __device__ __forceinline__ void drop_clause(int a) const { af[a] = 0; }
+    __device__ __forceinline__ void drop_var(int i) const { av[i] = 0; }
+    __device__ __forceinline__ void save(int, int) const {}
+    // the step wrote nothing to global memory: the solution before it is still there
+    __device__ __forceinline__ void restore(int tid, int nthr) const {
+        for (int i = tid; i < n; i += nthr) sol[i] = A.s.sol[v0 + i];
+    }
+    // what changed: masks (+ edge-mask bits), solutions
+    __device__ __forceinline__ void write_back(int tid, int nthr) const {
+        const pdp_graph& g = A.g; const pdp_state& s = A.s;
+        for (int i = tid; i < n; i += nthr) {
+            if (!av[i] && s.av[v0 + i]) deactivate_variable(g, s, v0 + i);
+            s.sol[v0 + i] = sol[i];
+        }
+        for (int a = tid; a < m; a += nthr)
+            if (!af[a] && s.af[f0 + a]) deactivate_clause(g, s, f0 + a);
+    }
 };
 __device__ __forceinline__ size_t tiny_bytes(int n, int m, int E) {
     return (size_t)n * (1 + 1 + 4 + 4 + 4 + 4) + (size_t)m * 2 + (size_t)(m + 1 + n + 1 + 2 * E) * 2 + 64;
 }
-__device__ __forceinline__ TinyView tiny_carve(unsigned char* base, int n, int m, int E) {
-    TinyView t;
-    float* f = reinterpret_cast<float*>(base);
+// problem b staged by its group into `area` (share bytes, at least tiny_bytes of the problem); a barrier must follow
+__device__ __forceinline__ TinyView tiny_stage(const KArgs& A, int b, int w, float pi, unsigned char* area, int share, int tid, int nthr) {
+    const pdp_graph& g = A.g; const pdp_state& s = A.s;
+    const int v0 = g.prob_vptr[b], v1 = g.prob_vptr[b + 1], f0 = g.prob_fptr[b], f1 = g.prob_fptr[b + 1];
+    const int n = v1 - v0, m = f1 - f0;
+    const int ec0 = g.cl_ptr[f0], ep0 = g.var_ptr[v0], E = g.cl_ptr[f1] - ec0;
+    TinyView t{{A, b, v0, f0, n, m, w, pi}};
+    float* f = reinterpret_cast<float*>(area);
     t.sol = f; t.score = f + n;
     t.cnt = reinterpret_cast<int*>(f + 2 * n); t.ev = t.cnt + n;
     uint16_t* h = reinterpret_cast<uint16_t*>(t.ev + n);
     t.clp = h; t.vp = t.clp + (m + 1); t.cvar = t.vp + (n + 1); t.vcls = t.cvar + E;
     uint8_t* q = reinterpret_cast<uint8_t*>(t.vcls + E);
     t.av = q; t.pure = q + n; t.af = q + 2 * n; t.single = t.af + m;
-    return t;
-}
-
-__device__ __forceinline__ void tiny_fix(const TinyView& t, int i, float sg) {
-    for (int p = t.vp[i]; p < t.vp[i + 1]; ++p) {
-        const uint32_t w = t.vcls[p];
-        const float lit = (w & 0x8000u) ? -1.f : 1.f;
-        if (lit * sg > 0.f) t.af[w & 0x7fffu] = 0;
-    }
-    t.av[i] = 0;
-    t.sol[i] = (sg + 1.f) / 2.0f;
-}
-
-// the fractional selection of one converged problem inside its CTA group (sel_grid's passes over the problem's own
-// variables, group barriers instead of grid barriers; the histograms stay in global memory: the kernel's shared memory is
-// the sweep buffer's).  Called by the whole group after the scoring loop with !cnan and max c > 0.  score / av: the
-// problem's variables (local index); TINY: fixes go to the shared-memory view.  Returns false for K_b == 1 (the caller
-// applies the arg-max rule); otherwise fixes the taken variables and sets ls.fixed (2: with rollback on, the state before
-// the fix is in the snapshot; the shared-memory tier leaves global memory as it was until its write-back, so it saves
-// is_sat only).
-template <bool TINY>
-__device__ __forceinline__ bool loc_select_fix(const KArgs& A, int b, int iter, const float* score, const uint8_t* av, int v0, int n,
-                                            TinyView t, LocSmem& ls, int tid, int nthr, int bar_id) {
-    const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    for (int pass = 0; pass < 8; ++pass) {
-        const bool first = pass == 0;
-        if (!first && s.sel_need[b] <= 0) break;
-        for (int base = 0; base < n; base += nthr) {   // (nthr is a multiple of 32: whole warps take part)
-            const int i = base + tid;
-            const bool valid = i < n;
-            const float c = valid ? fabsf(score[i]) * (float)av[i] : 0.f;
-            sel_hist_var(s, valid, b, v0 + i, c, valid && av[i], first);
-        }
-        bar_sync(bar_id, nthr);
-        if (tid < 32) sel_decide(s, b, A.dec_fraction, first, A.rb.av != nullptr);
-        bar_sync(bar_id, nthr);
-        if (first && s.sel_need[b] < 0) return false;
-    }
-    const bool snap = A.rb.av != nullptr && !(s.flags[b] & PDP_FLAG_UP_CONFLICT);
-    if (snap) {
-        if (!TINY) {
-            for (int i = tid; i < n; i += nthr) rb_save_var(A, v0 + i);
-            for (int a = g.prob_fptr[b] + tid; a < g.prob_fptr[b + 1]; a += nthr) rb_save_clause(A, a);
-        }
-        if (tid == 0) A.rb.is_sat[b] = s.is_sat[b];
-        bar_sync(bar_id, nthr);
-    }
-    const int i0 = tid;
-    bool any = false;
-    for (int i = i0; i < n; i += nthr) {
-        const float c = fabsf(score[i]) * (float)av[i];
-        if (!sel_taken(s, b, v0 + i, c, av[i] != 0)) continue;
-        const float sg = sgnf(score[i]);
-        if (TINY) tiny_fix(t, i, sg); else fix_variable(g, s, v0 + i, sg);
-        any = true;
-        if (A.trace) {
-            const int k = atomicAdd(&s.ctrl[CTRL_TRACE_LEN], 1);
-            if (k < A.trace_cap) { A.trace[3 * k] = iter; A.trace[3 * k + 1] = v0 + i; A.trace[3 * k + 2] = (int)sg; }
-        }
-    }
-    if (any) { ls.fixed = snap ? 2 : 1; s.masked[b] = 1; s.dirty[b] = 1; }
-    bar_sync(bar_id, nthr);
-    if (tid == 0) s.sel_need[b] = -1;
-    return true;
-}
-
-#define LSYNC() bar_sync(bar_id, nthr)
-// one converged problem: pdp_decimate.py:152-171 + solver.py:275-285 + trainer.py:150-162
-template <bool FRAC>
-__device__ __forceinline__ void loc_decimate_problem(const KArgs& A, int b, int iter, int w, float pi, bool check_termination, LocSmem& ls,
-                                                     int tid, int nthr, int bar_id) {
-    const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    const int v0 = g.prob_vptr[b], v1 = g.prob_vptr[b + 1], f0 = g.prob_fptr[b], f1 = g.prob_fptr[b + 1];
-    if (tid == 0) { ls.cmax = 0u; ls.cmin = 0x7f800000u; ls.cnan = 0u; ls.arg = 0x7fffffff; ls.fixed = 0; ls.nunsat = 0; }
-    LSYNC();
-    for (int i = v0 + tid; i < v1; i += nthr) {
-        const float sc = score_variable(g, s, s.eta[w], i, pi);
-        s.score[i] = sc;
-        const float c = fabsf(sc) * (float)s.av[i];
-        if (c != c) ls.cnan = 1u; else { atomicMax(&ls.cmax, f2u(c)); atomicMin(&ls.cmin, f2u(c)); }
-    }
-    LSYNC();
-    const bool topk = FRAC && !ls.cnan && u2f(ls.cmax) > 0.f &&
-                      loc_select_fix<false>(A, b, iter, s.score + v0, s.av + v0, v0, v1 - v0, TinyView{}, ls, tid, nthr, bar_id);
-    if (!topk && !ls.cnan) {   // first index attaining max of fl(fl(c - min) + 1), util.py:257-265
-        const float m = u2f(ls.cmin);
-        const float kmax = argmax_key(u2f(ls.cmax), m);
-        for (int i = v0 + tid; i < v1; i += nthr) {
-            const float c = fabsf(s.score[i]) * (float)s.av[i];
-            if (argmax_key(c, m) == kmax) atomicMin(&ls.arg, i);
-        }
-    }
-    LSYNC();
-    if (!topk && tid == 0 && !ls.cnan && u2f(ls.cmax) > 0.f && ls.arg != 0x7fffffff) {
-        const int i = ls.arg;
-        const float sg = sgnf(s.score[i]);
-        if (sg != 0.f && s.av[i]) {
-            fix_variable(g, s, i, sg);
-            s.masked[b] = 1; s.dirty[b] = 1;
-            ls.fixed = 1;
-            if (A.trace) {
-                const int k = atomicAdd(&s.ctrl[CTRL_TRACE_LEN], 1);
-                if (k < A.trace_cap) { A.trace[3 * k] = iter; A.trace[3 * k + 1] = i; A.trace[3 * k + 2] = (int)sg; }
-            }
-        }
-    }
-    LSYNC();
-    if (ls.fixed) loc_closure(A, b, v0, v1, f0, f1, ls, tid, nthr, bar_id);
-    LSYNC();
-    if (FRAC && ls.fixed == 2 && (s.flags[b] & PDP_FLAG_UP_CONFLICT)) {   // conflict rollback
-        for (int a = f0 + tid; a < f1; a += nthr) rb_restore_clause(A, a);
-        for (int i = v0 + tid; i < v1; i += nthr) rb_restore_var(A, i);
-        LSYNC();   // everybody has read the conflict bit before it is cleared
-        if (tid == 0) rb_commit(A, b, iter);
-    }
-    if (s.dirty[b]) {
-        if (check_termination) {   // SatCNFEvaluator on _solution over the full formula, then trainer.py:150-162
-            int n = 0;
-            for (int a = f0 + tid; a < f1; a += nthr) {
-                bool sat = false;
-                for (int c = g.cl_ptr[a]; c < g.cl_ptr[a + 1]; ++c) {
-                    const uint32_t wv = g.c_var[c];
-                    if (literal_true((wv & PDP_SIGN_BIT) ? -1.f : 1.f, s.sol[wv & PDP_IDX_MASK])) { sat = true; break; }
-                }
-                n += sat ? 0 : 1;
-            }
-            n = __reduce_add_sync(0xffffffffu, n);
-            if ((tid & 31) == 0 && n) atomicAdd(&ls.nunsat, n);
-            LSYNC();
-            if (tid == 0) {
-                if (ls.nunsat == 0) {
-                    if (s.active[b]) { s.active[b] = 0; s.freeze_iter[b] = iter; atomicSub(&s.ctrl[CTRL_NUM_ACTIVE], 1); }
-                    s.flags[b] |= PDP_FLAG_SOLVED;
-                }
-                s.dirty[b] = 0; s.n_unsat[b] = 0;
-            }
-        } else if (tid == 0) {
-            s.ctrl[CTRL_ANY_DIRTY] = 1;
-        }
-    }
-    if (tid == 0) s.conv[b] = 0;
-    LSYNC();
-}
-
-template <bool FRAC>
-__device__ __forceinline__ void loc_decimate_tiny(const KArgs& A, int b, int iter, int w, float pi, bool check_termination, LocSmem& ls,
-                                                  int tid, int nthr, int bar_id, unsigned char* area, int share) {
-    const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    const int v0 = g.prob_vptr[b], v1 = g.prob_vptr[b + 1], f0 = g.prob_fptr[b], f1 = g.prob_fptr[b + 1];
-    const int n = v1 - v0, m = f1 - f0;
-    const int ec0 = g.cl_ptr[f0], ep0 = g.var_ptr[v0], E = g.cl_ptr[f1] - ec0;
-    const TinyView t = tiny_carve(area, n, m, E);
     // the surveys of the problem in variable-major order, when they fit too (pi == 0: the external force column drops out)
     const size_t eta_off = (tiny_bytes(n, m, E) + 15) & ~(size_t)15;
-    const bool stage_eta = (pi == 0.f) && (eta_off + (size_t)E * 4 <= (size_t)share);
-    float* eta_s = reinterpret_cast<float*>(area + eta_off);
-    if (stage_eta) {
+    if ((pi == 0.f) && (eta_off + (size_t)E * 4 <= (size_t)share)) {
+        float* eta_s = reinterpret_cast<float*>(area + eta_off);
         const float* __restrict__ eta = s.eta[w];
         for (int e = tid; e < E; e += nthr) eta_s[e] = eta[g.p_vpos[ep0 + e]];
+        t.eta_s = eta_s;
     }
-    // ---- stage
     for (int i = tid; i < n; i += nthr) {
         t.av[i] = s.av[v0 + i]; t.pure[i] = 0; t.sol[i] = s.sol[v0 + i]; t.cnt[i] = 0; t.ev[i] = 0;
     }
@@ -1399,153 +1294,169 @@ __device__ __forceinline__ void loc_decimate_tiny(const KArgs& A, int b, int ite
         t.cvar[e] = (uint16_t)(((cw & PDP_IDX_MASK) - v0) | ((cw & PDP_SIGN_BIT) ? 0x8000u : 0u));
         t.vcls[e] = (uint16_t)((g.v_cls[ep0 + e] - f0) | ((g.v_cedge[ep0 + e] & PDP_SIGN_BIT) ? 0x8000u : 0u));
     }
+    return t;
+}
+
+#define LSYNC() bar_sync(bar_id, nthr)
+// the fractional selection of one converged problem inside its CTA group (sel_grid's passes over the problem's own
+// variables, group barriers instead of grid barriers; the histograms stay in global memory: the kernel's shared memory is
+// the sweep buffer's).  Called by the whole group after the scoring loop with !cnan and max c > 0.  Returns false for
+// K_b == 1 (the caller applies the arg-max rule); otherwise fixes the taken variables and sets ls.fixed (2: with rollback
+// on, the view has saved the state before the fix, and the snapshot holds is_sat).
+template <typename View>
+__device__ __forceinline__ bool loc_select_fix(const View& V, int iter, LocSmem& ls, int tid, int nthr, int bar_id) {
+    const KArgs& A = V.A; const pdp_state& s = A.s;
+    const int b = V.b;
+    for (int pass = 0; pass < 8; ++pass) {
+        const bool first = pass == 0;
+        if (!first && s.sel_need[b] <= 0) break;
+        for (int base = 0; base < V.n; base += nthr) {   // (nthr is a multiple of 32: whole warps take part)
+            const int i = base + tid;
+            const bool valid = i < V.n;
+            const float c = valid ? fabsf(V.score[i]) * (float)V.av[i] : 0.f;
+            sel_hist_var(s, valid, b, V.v0 + i, c, valid && V.av[i], first);
+        }
+        LSYNC();
+        if (tid < 32) sel_decide(s, b, A.dec_fraction, first, A.rb.av != nullptr);
+        LSYNC();
+        if (first && s.sel_need[b] < 0) return false;
+    }
+    const bool snap = A.rb.av != nullptr && !(s.flags[b] & PDP_FLAG_UP_CONFLICT);
+    if (snap) {
+        V.save(tid, nthr);
+        if (tid == 0) A.rb.is_sat[b] = s.is_sat[b];
+        LSYNC();
+    }
+    bool any = false;
+    for (int i = tid; i < V.n; i += nthr) {
+        const float c = fabsf(V.score[i]) * (float)V.av[i];
+        if (!sel_taken(s, b, V.v0 + i, c, V.av[i] != 0)) continue;
+        const float sg = sgnf(V.score[i]);
+        V.fix(i, sg);
+        any = true;
+        record_fix(A, iter, V.v0 + i, sg);
+    }
+    if (any) { ls.fixed = snap ? 2 : 1; s.masked[b] = 1; s.dirty[b] = 1; }
+    LSYNC();
+    if (tid == 0) s.sel_need[b] = -1;
+    return true;
+}
+
+template <typename View>
+__device__ __forceinline__ void loc_closure(const View& V, LocSmem& ls, int tid, int nthr, int bar_id) {
+    const pdp_state& s = V.A.s;
+    const int b = V.b;
+    for (;;) {   // unit propagation rounds, solver.py:234-273
+        if (tid == 0) { ls.flag = 0; ls.conflicts = 0; }
+        LSYNC();
+        for (int a = tid; a < V.m; a += nthr) {
+            int j; bool neg;
+            if (!V.af[a] || !V.is_unit(a, j, neg)) continue;
+            V.single[a] = 1;
+            atomicAdd(&V.cnt[j], 1);
+            atomicAdd(&V.ev[j], neg ? -1 : 1);
+            ls.flag = 1;
+        }
+        LSYNC();
+        if (!ls.flag) break;
+        for (int i = tid; i < V.n; i += nthr) {
+            const int cnt = V.cnt[i];
+            if (cnt > 0 && abs(V.ev[i]) != cnt) atomicAdd(&ls.conflicts, 1);
+        }
+        LSYNC();
+        const int nc = ls.conflicts;   // the `== 1` quirk of solver.py:257,261
+        for (int a = tid; a < V.m; a += nthr) {
+            if (V.single[a]) { V.drop_clause(a); V.single[a] = 0; }
+            else if (V.af[a] && nc == 1) V.drop_clause(a);
+        }
+        for (int i = tid; i < V.n; i += nthr)
+            if (V.av[i] && nc == 1) V.drop_var(i);
+        if (tid == 0) { s.masked[b] = 1; if (nc >= 1) { s.is_sat[b] = 0.f; s.flags[b] |= PDP_FLAG_UP_CONFLICT; } }
+        LSYNC();
+        for (int i = tid; i < V.n; i += nthr) {
+            const int cnt = V.cnt[i];
+            if (cnt > 0) {
+                const int ev = V.ev[i];
+                V.cnt[i] = 0; V.ev[i] = 0;
+                if (V.av[i] && abs(ev) == cnt) V.fix(i, ev > 0 ? 1.f : -1.f);
+            }
+        }
+        LSYNC();
+    }
+    for (;;) {   // pure-literal peeling rounds, solver.py:188-203
+        LSYNC();
+        if (tid == 0) ls.flag = 0;
+        LSYNC();
+        for (int i = tid; i < V.n; i += nthr) {
+            float val;
+            if (!V.av[i] || !V.is_pure(i, val)) continue;
+            V.pure[i] = 1;
+            V.sol[i] = val;
+            ls.flag = 1;
+        }
+        LSYNC();
+        if (!ls.flag) break;
+        // a pure variable is fixed to the value the round gave it: every active clause holding it is satisfied
+        // (none holds it: sol 0.5, sign 0, and it only leaves the problem)
+        for (int i = tid; i < V.n; i += nthr) {
+            if (!V.pure[i]) continue;
+            V.pure[i] = 0;
+            V.fix(i, 2.f * V.sol[i] - 1.f);
+        }
+        if (tid == 0) s.masked[b] = 1;
+    }
+}
+
+// one converged problem: pdp_decimate.py:152-171 + solver.py:275-285 + trainer.py:150-162
+template <bool FRAC, typename View>
+__device__ __forceinline__ void loc_decimate(const View& V, int iter, bool check_termination, LocSmem& ls, int tid, int nthr, int bar_id) {
+    const KArgs& A = V.A; const pdp_state& s = A.s;
+    const int b = V.b;
     if (tid == 0) { ls.cmax = 0u; ls.cmin = 0x7f800000u; ls.cnan = 0u; ls.arg = 0x7fffffff; ls.fixed = 0; ls.nunsat = 0; }
     LSYNC();
-    // ---- score, arg-max, fix (pdp_decimate.py:152-171)
-    for (int i = tid; i < n; i += nthr) {
-        float sc;
-        if (stage_eta) {   // score_variable on the staged copies (same order, same operations)
-            float ps = 0.f, ns = 0.f, as = 0.f;
-            for (int p = t.vp[i]; p < t.vp[i + 1]; ++p) {
-                const uint32_t cw = t.vcls[p];
-                const float f = L10(1.f - eta_s[p]) * (float)t.af[cw & 0x7fffu];
-                const bool neg = (cw & 0x8000u) != 0u;
-                ps += (neg ? 0.f : 1.f) * f;
-                ns += (neg ? 1.f : 0.f) * f;
-                as += f;
-            }
-            sc = sp_score_tail(ps, ns, as, 0.f, 0.f);
-        } else {
-            sc = score_variable(g, s, s.eta[w], v0 + i, pi);
-        }
-        t.score[i] = sc;
-        const float c = fabsf(sc) * (float)t.av[i];
+    for (int i = tid; i < V.n; i += nthr) {
+        const float sc = V.score_of(i);
+        V.score[i] = sc;
+        const float c = fabsf(sc) * (float)V.av[i];
         if (c != c) ls.cnan = 1u; else { atomicMax(&ls.cmax, f2u(c)); atomicMin(&ls.cmin, f2u(c)); }
     }
     LSYNC();
-    const bool topk = FRAC && !ls.cnan && u2f(ls.cmax) > 0.f &&
-                      loc_select_fix<true>(A, b, iter, t.score, t.av, v0, n, t, ls, tid, nthr, bar_id);
-    if (!topk && !ls.cnan) {
+    const bool topk = FRAC && !ls.cnan && u2f(ls.cmax) > 0.f && loc_select_fix(V, iter, ls, tid, nthr, bar_id);
+    if (!topk && !ls.cnan) {   // first index attaining max of fl(fl(c - min) + 1), util.py:257-265
         const float mn = u2f(ls.cmin);
         const float kmax = argmax_key(u2f(ls.cmax), mn);
-        for (int i = tid; i < n; i += nthr) {
-            const float c = fabsf(t.score[i]) * (float)t.av[i];
+        for (int i = tid; i < V.n; i += nthr) {
+            const float c = fabsf(V.score[i]) * (float)V.av[i];
             if (argmax_key(c, mn) == kmax) atomicMin(&ls.arg, i);
         }
     }
     LSYNC();
     if (!topk && tid == 0 && !ls.cnan && u2f(ls.cmax) > 0.f && ls.arg != 0x7fffffff) {
         const int i = ls.arg;
-        const float sg = sgnf(t.score[i]);
-        if (sg != 0.f && t.av[i]) {
-            tiny_fix(t, i, sg);
+        const float sg = sgnf(V.score[i]);
+        if (sg != 0.f && V.av[i]) {
+            V.fix(i, sg);
             s.masked[b] = 1; s.dirty[b] = 1;
             ls.fixed = 1;
-            if (A.trace) {
-                const int k = atomicAdd(&s.ctrl[CTRL_TRACE_LEN], 1);
-                if (k < A.trace_cap) { A.trace[3 * k] = iter; A.trace[3 * k + 1] = v0 + i; A.trace[3 * k + 2] = (int)sg; }
-            }
+            record_fix(A, iter, V.v0 + i, sg);
         }
     }
     LSYNC();
     if (ls.fixed) {
-        for (;;) {   // unit propagation rounds, solver.py:234-273
-            if (tid == 0) { ls.flag = 0; ls.conflicts = 0; }
-            LSYNC();
-            for (int a = tid; a < m; a += nthr) {
-                if (!t.af[a]) continue;
-                int deg = 0; uint32_t hit = 0;
-                for (int c = t.clp[a]; c < t.clp[a + 1]; ++c) {
-                    const uint32_t cw = t.cvar[c];
-                    if (t.av[cw & 0x7fffu]) { ++deg; hit = cw; }
-                }
-                if (deg == 1) {
-                    t.single[a] = 1;
-                    const int j = (int)(hit & 0x7fffu);
-                    atomicAdd(&t.cnt[j], 1);
-                    atomicAdd(&t.ev[j], (hit & 0x8000u) ? -1 : 1);
-                    ls.flag = 1;
-                }
-            }
-            LSYNC();
-            if (!ls.flag) break;
-            for (int i = tid; i < n; i += nthr) {
-                const int cnt = t.cnt[i];
-                if (cnt > 0 && abs(t.ev[i]) != cnt) atomicAdd(&ls.conflicts, 1);
-            }
-            LSYNC();
-            const int nc = ls.conflicts;   // the `== 1` quirk of solver.py:257,261
-            for (int a = tid; a < m; a += nthr) {
-                if (t.single[a]) { t.af[a] = 0; t.single[a] = 0; }
-                else if (t.af[a] && nc == 1) t.af[a] = 0;
-            }
-            for (int i = tid; i < n; i += nthr)
-                if (t.av[i] && nc == 1) t.av[i] = 0;
-            if (tid == 0) { s.masked[b] = 1; if (nc >= 1) { s.is_sat[b] = 0.f; s.flags[b] |= PDP_FLAG_UP_CONFLICT; } }
-            LSYNC();
-            for (int i = tid; i < n; i += nthr) {
-                const int cnt = t.cnt[i];
-                if (cnt > 0) {
-                    const int ev = t.ev[i];
-                    t.cnt[i] = 0; t.ev[i] = 0;
-                    if (t.av[i] && abs(ev) == cnt) tiny_fix(t, i, ev > 0 ? 1.f : -1.f);
-                }
-            }
-            LSYNC();
-        }
-        for (;;) {   // pure-literal peeling rounds, solver.py:188-203
-            LSYNC();
-            if (tid == 0) ls.flag = 0;
-            LSYNC();
-            for (int i = tid; i < n; i += nthr) {
-                if (!t.av[i]) continue;
-                int deg = 0, sdeg = 0;
-                for (int p = t.vp[i]; p < t.vp[i + 1]; ++p) {
-                    const uint32_t cw = t.vcls[p];
-                    if (t.af[cw & 0x7fffu]) { ++deg; sdeg += (cw & 0x8000u) ? -1 : 1; }
-                }
-                if (deg == abs(sdeg)) {
-                    t.pure[i] = 1;
-                    t.sol[i] = ((sdeg > 0 ? 1.f : (sdeg < 0 ? -1.f : 0.f)) + 1.f) / 2.0f;
-                    ls.flag = 1;
-                }
-            }
-            LSYNC();
-            if (!ls.flag) break;
-            for (int i = tid; i < n; i += nthr) {
-                if (!t.pure[i]) continue;
-                t.pure[i] = 0;
-                for (int p = t.vp[i]; p < t.vp[i + 1]; ++p) t.af[t.vcls[p] & 0x7fffu] = 0;
-                t.av[i] = 0;
-            }
-            if (tid == 0) s.masked[b] = 1;
-        }
-        if (FRAC && ls.fixed == 2 && (s.flags[b] & PDP_FLAG_UP_CONFLICT)) {
-            // conflict rollback: nothing is written back, global memory holds the state before the step
+        loc_closure(V, ls, tid, nthr, bar_id);
+        if (FRAC && ls.fixed == 2 && (s.flags[b] & PDP_FLAG_UP_CONFLICT)) {   // conflict rollback
+            V.restore(tid, nthr);
             LSYNC();   // everybody has read the conflict bit before it is cleared
             if (tid == 0) rb_commit(A, b, iter);
         } else {
-            // ---- write back what changed: masks (+ edge-mask bits), solutions
-            for (int i = tid; i < n; i += nthr) {
-                if (!t.av[i] && s.av[v0 + i]) deactivate_variable(g, s, v0 + i);
-                s.sol[v0 + i] = t.sol[i];
-            }
-            for (int a = tid; a < m; a += nthr)
-                if (!t.af[a] && s.af[f0 + a]) deactivate_clause(g, s, f0 + a);
+            V.write_back(tid, nthr);
         }
     }
     LSYNC();
     if (s.dirty[b]) {
         if (check_termination) {   // SatCNFEvaluator on _solution over the full formula, then trainer.py:150-162
             int nun = 0;
-            for (int a = tid; a < m; a += nthr) {
-                bool sat = false;
-                for (int c = t.clp[a]; c < t.clp[a + 1]; ++c) {
-                    const uint32_t cw = t.cvar[c];
-                    if (literal_true((cw & 0x8000u) ? -1.f : 1.f, t.sol[cw & 0x7fffu])) { sat = true; break; }
-                }
-                nun += sat ? 0 : 1;
-            }
+            for (int a = tid; a < V.m; a += nthr) nun += V.satisfied(a) ? 0 : 1;
             nun = __reduce_add_sync(0xffffffffu, nun);
             if ((tid & 31) == 0 && nun) atomicAdd(&ls.nunsat, nun);
             LSYNC();
@@ -1569,7 +1480,6 @@ __device__ __forceinline__ bool loc_problem_is_small(const pdp_graph& g, int b) 
     return (g.prob_vptr[b + 1] - g.prob_vptr[b] <= PDP_LOCAL_MAX_V) && (g.prob_fptr[b + 1] - g.prob_fptr[b] <= PDP_LOCAL_MAX_F);
 }
 
-#undef LSYNC
 // groups of PDP_LOCAL_GROUP threads (named barriers 8..15) take one problem each
 #define PDP_LOCAL_GROUP 128
 // `area` / `area_bytes`: the CTA's dynamic shared memory (the sweep buffer, idle during the decimation), split evenly
@@ -1601,21 +1511,16 @@ __device__ __forceinline__ void loc_decimate_all(const KArgs& A, int iter, int w
         const int n = A.g.prob_vptr[b + 1] - A.g.prob_vptr[b], m = A.g.prob_fptr[b + 1] - A.g.prob_fptr[b];
         const int E = A.g.cl_ptr[A.g.prob_fptr[b + 1]] - A.g.cl_ptr[A.g.prob_fptr[b]];
         if (n < 32768 && m < 32768 && E < 65536 && tiny_bytes(n, m, E) <= (size_t)share)
-            loc_decimate_tiny<FRAC>(A, b, iter, w, pi, check_termination, ls[grp], gt, gthr, 8 + grp, area + (size_t)grp * share, share);
+            loc_decimate<FRAC>(tiny_stage(A, b, w, pi, area + (size_t)grp * share, share, gt, gthr), iter, check_termination,
+                               ls[grp], gt, gthr, 8 + grp);
         else
-            loc_decimate_problem<FRAC>(A, b, iter, w, pi, check_termination, ls[grp], gt, gthr, 8 + grp);
+            loc_decimate<FRAC>(loc_global(A, b, w, pi), iter, check_termination, ls[grp], gt, gthr, 8 + grp);
     }
 }
 
 // ------------------------------------------------------------------------------------------------
 // full-formula satisfaction count (SatCNFEvaluator on _solution, util.py:210-236) for dirty problems
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ bool literal_true(float sgn, float p) {
-    float ev = sgn * p;
-    ev = ev + (1.f - sgn) / 2.f;
-    return ev > 0.5f;
-}
-
 __device__ __forceinline__ void cnf_count_dirty(const KArgs& A) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
     KeyedReducer<CountAcc> red;
@@ -1627,12 +1532,7 @@ __device__ __forceinline__ void cnf_count_dirty(const KArgs& A) {
             red.touch(s, b);
             for (int a = g.prob_fptr[b] + (int)gtid(); a < f1; a += (int)gthreads()) {
                 if (native && s.af[a]) { red.acc.n += 1; continue; }
-                bool sat = false;
-                for (int c = g.cl_ptr[a]; c < g.cl_ptr[a + 1]; ++c) {
-                    const uint32_t w = g.c_var[c];
-                    if (literal_true((w & PDP_SIGN_BIT) ? -1.f : 1.f, s.sol[w & PDP_IDX_MASK])) { sat = true; break; }
-                }
-                red.acc.n += sat ? 0 : 1;
+                red.acc.n += clause_satisfied(g.c_var, g.cl_ptr[a], g.cl_ptr[a + 1], s.sol) ? 0 : 1;
             }
             red.finish(s);
         }
@@ -1644,13 +1544,7 @@ __device__ __forceinline__ void cnf_count_dirty(const KArgs& A) {
         if (!s.dirty[b]) continue;
         red.touch(s, b);
         if (native && s.af[a]) { red.acc.n += 1; continue; }   // an active clause holds no true literal (CTRL_NATIVE)
-        const int beg = g.cl_ptr[a], end = g.cl_ptr[a + 1];
-        bool sat = false;
-        for (int c = beg; c < end; ++c) {
-            const uint32_t w = g.c_var[c];
-            if (literal_true((w & PDP_SIGN_BIT) ? -1.f : 1.f, s.sol[w & PDP_IDX_MASK])) { sat = true; break; }
-        }
-        red.acc.n += sat ? 0 : 1;
+        red.acc.n += clause_satisfied(g.c_var, g.cl_ptr[a], g.cl_ptr[a + 1], s.sol) ? 0 : 1;
     }
     red.finish(s);
 }

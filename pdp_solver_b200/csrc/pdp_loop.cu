@@ -85,10 +85,7 @@ __device__ __forceinline__ void select_and_fix_phase(const KArgs& A, int iter, b
                 if (lane_id() == 0) {
                     s.masked[b] = 1; s.dirty[b] = 1;
                     s.ctrl[slot] = 1; s.ctrl[CTRL_ANY_DIRTY] = 1;
-                    if (A.trace) {
-                        int k = atomicAdd(&s.ctrl[CTRL_TRACE_LEN], 1);
-                        if (k < A.trace_cap) { A.trace[3 * k] = iter; A.trace[3 * k + 1] = i; A.trace[3 * k + 2] = (int)sg; }
-                    }
+                    record_fix(A, iter, i, sg);
                 }
             }
         }
@@ -131,10 +128,7 @@ __device__ __forceinline__ void frac_select_and_fix(const KArgs& A, cg::grid_gro
                 const int b = g.bvm[vi];
                 s.masked[b] = 1; s.dirty[b] = 1;
                 s.ctrl[slot] = 1; s.ctrl[CTRL_ANY_DIRTY] = 1;
-                if (A.trace) {
-                    const int k = atomicAdd(&s.ctrl[CTRL_TRACE_LEN], 1);
-                    if (k < A.trace_cap) { A.trace[3 * k] = iter; A.trace[3 * k + 1] = vi; A.trace[3 * k + 2] = (int)vsg; }
-                }
+                record_fix(A, iter, vi, vsg);
             }
             __syncwarp();
         }

@@ -19,12 +19,7 @@ __global__ void k_cnf_eval_count(pdp_graph g, pdp_state s, const float* __restri
             if (last_b >= 0) { atomicAdd(&s.conflicts[last_b], n_all); atomicAdd(&s.energy[last_b], n_sat); }
             last_b = b; n_all = 0; n_sat = 0;
         }
-        bool sat = false;
-        for (int c = g.cl_ptr[a]; c < g.cl_ptr[a + 1]; ++c) {
-            const uint32_t w = g.c_var[c];
-            if (literal_true((w & PDP_SIGN_BIT) ? -1.f : 1.f, pred[w & PDP_IDX_MASK])) { sat = true; break; }
-        }
-        n_all += 1; n_sat += sat ? 1 : 0;
+        n_all += 1; n_sat += clause_satisfied(g.c_var, g.cl_ptr[a], g.cl_ptr[a + 1], pred) ? 1 : 0;
     }
     if (last_b >= 0) { atomicAdd(&s.conflicts[last_b], n_all); atomicAdd(&s.energy[last_b], n_sat); }
 }
