@@ -229,9 +229,38 @@ __device__ __forceinline__ void deactivate_variable(const pdp_graph& g, const pd
     s.av[i] = 0;
     for (int p = g.var_ptr[i]; p < g.var_ptr[i + 1]; ++p) mask_edge(g, g.p_vpos[p], g.p_qpos[p]);
 }
-__device__ __forceinline__ void deactivate_clause(const pdp_graph& g, const pdp_state& s, int a) {
+
+// entry `id` appended to the list whose length is s.ctrl[slot]; a full list raises CTRL_FR_OVER
+__device__ __forceinline__ void fr_append(const pdp_state& s, int slot, int32_t* list, int id) {
+    const int k = atomicAdd(&s.ctrl[slot], 1);
+    if (k < s.fr_cap) list[k] = id; else s.ctrl[CTRL_FR_OVER] = 1;
+}
+// node `id` put on node list `list` of the frontier closure, once per epoch
+__device__ __forceinline__ void fr_push(const pdp_state& s, int list, int32_t* stamp, int id, int epoch) {
+    if (atomicExch(&stamp[id], epoch) == epoch) return;
+    fr_append(s, CTRL_FR_N + list, s.fr_list[list], id);
+}
+// Where fixes and clause de-activations queue the nodes they touch.  NoQueue: nowhere (the full scans look at every node).
+// ListQueue: the lists of the frontier closure -- the still-active clauses of a fixed variable that its value does not
+// satisfy go to clause list clist at epoch epc (unit test; clist < 0: none), the still-active variables of a de-activated
+// clause go to variable list vlist at epoch epv (purity test).
+struct NoQueue {
+    __device__ __forceinline__ void clause(const pdp_state&, int) const {}
+    __device__ __forceinline__ void var(const pdp_state&, int) const {}
+};
+struct ListQueue {
+    int clist, epc, vlist, epv;
+    __device__ __forceinline__ void clause(const pdp_state& s, int a) const { if (clist >= 0 && s.af[a]) fr_push(s, clist, s.stamp_c, a, epc); }
+    __device__ __forceinline__ void var(const pdp_state& s, int j) const { if (s.av[j]) fr_push(s, vlist, s.stamp_v, j, epv); }
+};
+
+template <typename Q = NoQueue>
+__device__ __forceinline__ void deactivate_clause(const pdp_graph& g, const pdp_state& s, int a, const Q& q = Q()) {
     s.af[a] = 0;
-    for (int c = g.cl_ptr[a]; c < g.cl_ptr[a + 1]; ++c) mask_edge(g, cvpos(g, c), cqpos(g, c));
+    for (int c = g.cl_ptr[a]; c < g.cl_ptr[a + 1]; ++c) {
+        mask_edge(g, cvpos(g, c), cqpos(g, c));
+        q.var(s, (int)(g.c_var[c] & PDP_IDX_MASK));
+    }
 }
 // the words change between passes: read around L1
 __device__ __forceinline__ bool mbit(const uint32_t* words, int pos) { return (__ldcg(words + (pos >> 5)) >> (pos & 31)) & 1u; }
@@ -492,16 +521,20 @@ __device__ __forceinline__ void argmax_phase(const KArgs& A, const CF& coef) {
 }
 
 // fixing one variable (the per-variable form of _set_variable_core, solver.py:205-226): clauses
-// holding a now-true occurrence are de-activated, the variable is de-activated, solution updated
-__device__ __forceinline__ void fix_variable(const pdp_graph& g, const pdp_state& s, int i, float sg) {
-    const int beg = g.var_ptr[i], end = g.var_ptr[i + 1];
-    for (int p = beg; p < end; ++p) {
+// holding a now-true occurrence are de-activated, the variable is de-activated, solution updated.
+// STRIDE 1: by one thread; 32: by the lanes of a warp, over the variable's edges, once all of them have read av[i] (the
+// decimation fix of a large problem: one thread walking its ~40 dependent global updates was 0.4 ms)
+template <int STRIDE = 1, typename Q = NoQueue>
+__device__ __forceinline__ void fix_variable(const pdp_graph& g, const pdp_state& s, int i, float sg, const Q& q = Q()) {
+    const int lane = STRIDE == 1 ? 0 : lane_id();
+    for (int p = g.var_ptr[i] + lane; p < g.var_ptr[i + 1]; p += STRIDE) {
         const float lit = (g.v_cedge[p] & PDP_SIGN_BIT) ? -1.f : 1.f;
         const int a = g.v_cls[p];
-        if (lit * sg > 0.f && s.af[a]) deactivate_clause(g, s, a);
+        if (lit * sg > 0.f) { if (s.af[a]) deactivate_clause(g, s, a, q); }
+        else q.clause(s, a);
+        mask_edge(g, g.p_vpos[p], g.p_qpos[p]);
     }
-    deactivate_variable(g, s, i);
-    s.sol[i] = (sg + 1.f) / 2.0f;
+    if (lane == 0) { s.av[i] = 0; s.sol[i] = (sg + 1.f) / 2.0f; }
 }
 
 // one event (iteration, variable, sign) of the optional decimation trace
@@ -600,206 +633,224 @@ __device__ __forceinline__ bool var_pure(const pdp_graph& g, const uint8_t* af, 
 }
 
 // ------------------------------------------------------------------------------------------------
+// Grid-wide closure: unit propagation rounds, then pure-literal peeling rounds, to the fixed point of the dirty problems
+// (solver.py:180-273), for large problems, batch replication, simplify() and set_variables().  One body, closure_rounds,
+// runs the synchronous rounds -- every phase reads only what the barrier before it published -- over a node source: the
+// nodes a round looks at, and the queue its fixes and de-activations put the nodes they touch on.
+//  * FullScan: every node (of the dirty problems); queues nothing, never overflows.  The closure of simplify() and set_variables(), the
+//    fallback of the frontier, and the reference of the tests (flags bit 2).
+//  * Frontier: lists of the nodes touched since the round before.  Once every problem is closed under unit propagation
+//    and peeling (after simplify()), fixing a variable can only create unit clauses among the clauses that hold a
+//    variable de-activated in the previous round, and pure literals among the variables of clauses de-activated since:
+//    the same rounds over those lists instead of over all F clauses and V variables (8.9 -> 1.9 ms per decimation
+//    iteration at 8 x n = 1 M, where a round's full scan gathers 100 M node flags to find a dozen nodes).
+// ------------------------------------------------------------------------------------------------
+struct FullScan {
+    template <typename Fn> __device__ __forceinline__ void clauses(const KArgs& A, int, Fn fn) const {
+        WARP_STRIDED(a, A.g.F) { if (a < A.g.F) fn((int)a); }
+    }
+    template <typename Fn> __device__ __forceinline__ void units(const KArgs& A, int, Fn fn) const {
+        WARP_STRIDED(i, A.g.V) { if (i < A.g.V) fn((int)i); }
+    }
+    template <typename Fn> __device__ __forceinline__ void vars(const KArgs& A, int round, Fn fn) const { units(A, round, fn); }
+    __device__ __forceinline__ void unit(const pdp_state&, int, int) const {}
+    __device__ __forceinline__ NoQueue up_queue(int) const { return {}; }
+    __device__ __forceinline__ NoQueue peel_queue(int) const { return {}; }
+    __device__ __forceinline__ bool up_round(const pdp_state&, int) const { return true; }
+    __device__ __forceinline__ bool peel_round(const pdp_state&, int) const { return true; }
+};
+
+// Ping-pong lists, entries unique per epoch (stamps):
+//   clause lists 0/1 (by UP round)    : clauses to test for unit-ness
+//   variable lists 2/3 (by peel round): variables to test for purity; list 2 is filled during the whole UP stage
+//   unit lists 0/1 (by UP round)      : variables some unit clause of the round points at (at most one per clause of the
+//                                       round's list: they cannot overflow)
+template <typename Fn>
+__device__ __forceinline__ void fr_each(const pdp_state& s, int slot, const int32_t* list, Fn fn) {
+    const int n = s.ctrl[slot] < s.fr_cap ? s.ctrl[slot] : s.fr_cap;
+    WARP_STRIDED(x, n) { if (x < n) fn(list[x]); }
+}
+struct Frontier {
+    int epc, epv;   // epochs of the clause list and of the variable list the current round reads
+    template <typename Fn> __device__ __forceinline__ void clauses(const KArgs& A, int round, Fn fn) const {
+        fr_each(A.s, CTRL_FR_N + (round & 1), A.s.fr_list[round & 1], fn);
+    }
+    template <typename Fn> __device__ __forceinline__ void units(const KArgs& A, int round, Fn fn) const {
+        fr_each(A.s, CTRL_FR_NU + (round & 1), A.s.fr_unit[round & 1], fn);
+    }
+    template <typename Fn> __device__ __forceinline__ void vars(const KArgs& A, int round, Fn fn) const {
+        fr_each(A.s, CTRL_FR_N + 2 + (round & 1), A.s.fr_list[2 + (round & 1)], fn);
+    }
+    __device__ __forceinline__ void unit(const pdp_state& s, int round, int j) const {
+        fr_append(s, CTRL_FR_NU + (round & 1), s.fr_unit[round & 1], j);
+    }
+    // UP round r queues clauses for round r + 1 and variables for peel round 0; peel round r queues variables for
+    // peel round r + 1
+    __device__ __forceinline__ ListQueue up_queue(int round) const { return {(round & 1) ^ 1, epc + 1, 2, epv}; }
+    __device__ __forceinline__ ListQueue peel_queue(int round) const { return {-1, 0, 2 + ((round & 1) ^ 1), epv + 1}; }
+    // the top of a round, by all threads: the epoch of the round's list; thread 0 empties the lists the round fills.
+    // False when a list has overflowed (uniform: written before the last barrier).
+    __device__ __forceinline__ bool up_round(const pdp_state& s, int round) {
+        if (round > 0) ++epc;
+        if (s.ctrl[CTRL_FR_OVER]) return false;
+        if (gtid() == 0) { s.ctrl[CTRL_FR_N + ((round & 1) ^ 1)] = 0; s.ctrl[CTRL_FR_NU + ((round & 1) ^ 1)] = 0; }
+        return true;
+    }
+    __device__ __forceinline__ bool peel_round(const pdp_state& s, int round) {
+        if (round > 0) ++epv;
+        if (s.ctrl[CTRL_FR_OVER]) return false;
+        if (gtid() == 0) s.ctrl[CTRL_FR_N + 2 + ((round & 1) ^ 1)] = 0;
+        return true;
+    }
+};
+
 // unit propagation round (solver.py:228-273), split at its data dependencies
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void up_find_units(const KArgs& A, int flag_slot) {
+template <typename Src>
+__device__ __forceinline__ void find_units(const KArgs& A, const Src& src, int round, int flag_slot) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    WARP_STRIDED(a, g.F) {
-        if (a >= g.F) continue;
-        if (!s.af[a]) continue;
-        const int b = g.bfm[a];
-        if (!s.dirty[b]) continue;
+    src.clauses(A, round, [&](int a) {
+        if (!s.af[a] || !s.dirty[g.bfm[a]]) return;
         int j; bool neg;
-        if (clause_unit(g.c_var, g.cl_ptr[a], g.cl_ptr[a + 1], s.av, j, neg)) {
-            s.single[a] = 1;
-            atomicAdd(&s.up_cnt[j], 1);
-            atomicAdd(&s.up_ev[j], neg ? -1 : 1);
-            s.ctrl[flag_slot] = 1;
-        }
-    }
+        if (!clause_unit(g.c_var, g.cl_ptr[a], g.cl_ptr[a + 1], s.av, j, neg)) return;
+        s.single[a] = 1;
+        if (atomicAdd(&s.up_cnt[j], 1) == 0) src.unit(s, round, j);
+        atomicAdd(&s.up_ev[j], neg ? -1 : 1);
+        s.ctrl[flag_slot] = 1;
+    });
 }
 
-__device__ __forceinline__ void up_find_conflicts(const KArgs& A) {
+// a problem's first conflict raises CTRL_UP_WIPE: one conflict may mean a wipe
+template <typename Src>
+__device__ __forceinline__ void find_conflicts(const KArgs& A, const Src& src, int round) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    WARP_STRIDED(i, g.V) {
-        if (i >= g.V) continue;
+    src.units(A, round, [&](int i) {
         const int cnt = s.up_cnt[i];
-        if (cnt > 0 && abs(s.up_ev[i]) != cnt) atomicAdd(&s.conflicts[g.bvm[i]], 1);
-    }
+        if (cnt > 0 && abs(s.up_ev[i]) != cnt && atomicAdd(&s.conflicts[g.bvm[i]], 1) == 0) s.ctrl[CTRL_UP_WIPE] = 1;
+    });
 }
 
-// quirk kept from the reference (solver.py:257,261): the problem is wiped only when its conflict
-// COUNT equals exactly one.  RB: conflict rollback of the fused loop's grid-wide step (rb_mark)
-template <bool RB>
-__device__ __forceinline__ void up_apply_conflicts(const KArgs& A) {
+// quirk kept from the reference (solver.py:257,261): the problem is wiped only when its conflict COUNT equals exactly one;
+// the wipe scans the whole batch (rare).  RB: conflict rollback of the fused loop's grid-wide step (rb_mark)
+template <bool RB, typename Src>
+__device__ __forceinline__ void apply_conflicts(const KArgs& A, const Src& src, int round) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    const int64_t n = g.V > g.F ? g.V : g.F;
-    WARP_STRIDED(i, n) {
-        if (i < g.F) {
-            if (s.single[i]) { deactivate_clause(g, s, (int)i); s.single[i] = 0; s.masked[g.bfm[i]] = 1; }
-            else if (s.af[i] && s.conflicts[g.bfm[i]] == 1) deactivate_clause(g, s, (int)i);
+    const auto q = src.up_queue(round);
+    src.clauses(A, round, [&](int a) {
+        if (s.single[a]) { deactivate_clause(g, s, a, q); s.single[a] = 0; s.masked[g.bfm[a]] = 1; }
+    });
+    if (s.ctrl[CTRL_UP_WIPE]) {
+        const int64_t n = g.V > g.F ? g.V : g.F;
+        WARP_STRIDED(i, n) {
+            if (i < g.F && s.af[i] && !s.single[i] && s.conflicts[g.bfm[i]] == 1) deactivate_clause(g, s, (int)i);
+            if (i < g.V && s.av[i] && s.conflicts[g.bvm[i]] == 1) deactivate_variable(g, s, (int)i);
         }
-        if (i < g.V) {
-            if (s.av[i] && s.conflicts[g.bvm[i]] == 1) deactivate_variable(g, s, (int)i);
-        }
-        if (i < g.B) {
-            if (s.conflicts[i] >= 1) { s.is_sat[i] = 0.f; s.flags[i] |= PDP_FLAG_UP_CONFLICT; s.masked[i] = 1; if (RB) rb_mark(A, (int)i); }
-        }
+    }
+    WARP_STRIDED(b, g.B) {
+        if (b < g.B && s.conflicts[b] >= 1) { s.is_sat[b] = 0.f; s.flags[b] |= PDP_FLAG_UP_CONFLICT; s.masked[b] = 1; if (RB) rb_mark(A, (int)b); }
     }
 }
 
-__device__ __forceinline__ void up_assign(const KArgs& A) {
+template <typename Src>
+__device__ __forceinline__ void assign_units(const KArgs& A, const Src& src, int round) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    const int64_t n = g.V > g.B ? g.V : g.B;
-    WARP_STRIDED(i, n) {
-        if (i < g.V) {
-            const int cnt = s.up_cnt[i];
-            if (cnt > 0) {
-                const int ev = s.up_ev[i];
-                s.up_cnt[i] = 0; s.up_ev[i] = 0;
-                if (s.av[i] && abs(ev) == cnt) fix_variable(g, s, (int)i, ev > 0 ? 1.f : -1.f);
-            }
+    const auto q = src.up_queue(round);
+    src.units(A, round, [&](int i) {
+        const int cnt = s.up_cnt[i];
+        if (cnt > 0) {
+            const int ev = s.up_ev[i];
+            s.up_cnt[i] = 0; s.up_ev[i] = 0;
+            if (s.av[i] && abs(ev) == cnt) fix_variable(g, s, i, ev > 0 ? 1.f : -1.f, q);
         }
-    }
+    });
+    WARP_STRIDED(b, g.B) { if (b < g.B) s.conflicts[b] = 0; }
+    if (gtid() == 0) s.ctrl[CTRL_UP_WIPE] = 0;
 }
 
-__device__ __forceinline__ void up_clear_conflicts(const KArgs& A) {
-    const pdp_state& s = A.s;
-    WARP_STRIDED(i, A.g.B) { if (i < A.g.B) s.conflicts[i] = 0; }
-}
-
-// ------------------------------------------------------------------------------------------------
 // pure-literal peeling round (solver.py:180-203)
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void peel_find(const KArgs& A, int flag_slot) {
+template <typename Src>
+__device__ __forceinline__ void peel_find(const KArgs& A, const Src& src, int round, int flag_slot) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    WARP_STRIDED(i, g.V) {
-        if (i >= g.V) continue;
-        if (!s.av[i]) continue;
-        const int b = g.bvm[i];
-        if (!s.dirty[b]) continue;
+    src.vars(A, round, [&](int i) {
+        if (!s.av[i] || !s.dirty[g.bvm[i]]) return;
         float val;
-        if (var_pure(g, s.af, (int)i, val)) {
-            s.pure[i] = 1;
-            s.sol[i] = val;
-            s.ctrl[flag_slot] = 1;
-        }
-    }
+        if (var_pure(g, s.af, i, val)) { s.pure[i] = 1; s.sol[i] = val; s.ctrl[flag_slot] = 1; }
+    });
 }
 
-__device__ __forceinline__ void peel_apply(const KArgs& A) {
+// a pure variable is fixed to the value the round gave it: every active clause holding it is satisfied (none holds it:
+// sol 0.5, sign 0, and it only leaves the problem), so the fix queues no clause
+template <typename Src>
+__device__ __forceinline__ void peel_fix(const KArgs& A, const Src& src, int round) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    WARP_STRIDED(i, g.V) {
-        if (i >= g.V) continue;
-        if (!s.pure[i]) continue;
+    const auto q = src.peel_queue(round);
+    src.vars(A, round, [&](int i) {
+        if (!s.pure[i]) return;
         s.pure[i] = 0;
-        const int beg = g.var_ptr[i], end = g.var_ptr[i + 1];
-        for (int p = beg; p < end; ++p) {
-            const int a = g.v_cls[p];
-            if (s.af[a]) deactivate_clause(g, s, a);
-        }
-        deactivate_variable(g, s, (int)i);
+        fix_variable(g, s, i, 2.f * s.sol[i] - 1.f, q);
         s.masked[g.bvm[i]] = 1;
-    }
+    });
 }
 
-// UP closure then peel closure for the dirty problems.  Called by ALL threads of the cooperative grid.
-// Flag slots alternate by round parity so a flag is never reset while it can still be read.
+// The rounds over node source src, by ALL threads of the cooperative grid; false when the source's lists overflowed (at
+// the top of a round: the per-round scratch is clean).  Flag slots alternate by round parity so a flag is never reset
+// while it can still be read; UP and peel use disjoint slots so a thread that has left one loop can never disturb a flag
+// another thread is still reading.  Every flag slot is zero again after a true return.
+template <bool RB, typename Src>
+__device__ __forceinline__ bool closure_rounds(const KArgs& A, cg::grid_group& grid, Src& src) {
+    const pdp_state& s = A.s;
+    for (int round = 0;; ++round) {   // solver.py:234-273
+        const int slot = CTRL_FLAG_A + (round & 1);
+        if (!src.up_round(s, round)) return false;
+        find_units(A, src, round, slot);
+        if (gtid() == 0) s.ctrl[CTRL_FLAG_A + ((round + 1) & 1)] = 0;
+        grid.sync();
+        if (!s.ctrl[slot]) break;
+        find_conflicts(A, src, round);
+        grid.sync();
+        apply_conflicts<RB>(A, src, round);
+        grid.sync();
+        assign_units(A, src, round);
+        grid.sync();
+    }
+    for (int round = 0;; ++round) {   // solver.py:188-203
+        const int slot = CTRL_FLAG_C + (round & 1);
+        if (!src.peel_round(s, round)) return false;
+        peel_find(A, src, round, slot);
+        if (gtid() == 0) s.ctrl[CTRL_FLAG_C + ((round + 1) & 1)] = 0;
+        grid.sync();
+        if (!s.ctrl[slot]) break;
+        peel_fix(A, src, round);
+        grid.sync();
+    }
+    return true;
+}
+
 template <bool RB = false>
 __device__ PDP_COLD void closure(const KArgs& A, cg::grid_group& grid) {
+    FullScan src;
+    closure_rounds<RB>(A, grid, src);
+}
+
+// the queue of the decimation fixes closure_frontier starts from: clause list 0 and variable list 2
+__device__ __forceinline__ ListQueue frontier_queue(const pdp_state& s) { return {0, s.ctrl[CTRL_FR_EPC], 2, s.ctrl[CTRL_FR_EPV]}; }
+
+// after those fixes and a grid barrier.  A list that overflows sends the rest of the closure through the full scans.
+template <bool RB = false>
+__device__ PDP_COLD void closure_frontier(const KArgs& A, cg::grid_group& grid) {
     const pdp_state& s = A.s;
-    int round = 0;
-    for (;;) {   // solver.py:234-273
-        const int slot = CTRL_FLAG_A + (round & 1);
-        const int other = CTRL_FLAG_A + ((round + 1) & 1);
-        up_find_units(A, slot);
-        if (gtid() == 0) s.ctrl[other] = 0;
-        grid.sync();
-        if (!s.ctrl[slot]) break;
-        up_find_conflicts(A);
-        grid.sync();
-        up_apply_conflicts<RB>(A);
-        grid.sync();
-        up_assign(A);
-        up_clear_conflicts(A);
-        grid.sync();
-        ++round;
+    Frontier src{s.ctrl[CTRL_FR_EPC], s.ctrl[CTRL_FR_EPV]};
+    const bool closed = closure_rounds<RB>(A, grid, src);
+    grid.sync();
+    if (gtid() == 0) {
+        s.ctrl[CTRL_FR_EPC] = src.epc + 1; s.ctrl[CTRL_FR_EPV] = src.epv + 1;
+        for (int i = 0; i < 4; ++i) s.ctrl[CTRL_FR_N + i] = 0;
+        s.ctrl[CTRL_FR_NU] = 0; s.ctrl[CTRL_FR_NU + 1] = 0; s.ctrl[CTRL_FR_OVER] = 0;
     }
-    round = 0;
-    for (;;) {   // solver.py:188-203
-        const int slot = CTRL_FLAG_C + (round & 1);
-        const int other = CTRL_FLAG_C + ((round + 1) & 1);
-        peel_find(A, slot);
-        if (gtid() == 0) s.ctrl[other] = 0;
+    if (!closed) {
+        if (gtid() == 0) { s.ctrl[CTRL_FLAG_A] = 0; s.ctrl[CTRL_FLAG_A + 1] = 0; s.ctrl[CTRL_FLAG_C] = 0; s.ctrl[CTRL_FLAG_C + 1] = 0; }
         grid.sync();
-        if (!s.ctrl[slot]) break;
-        peel_apply(A);
-        grid.sync();
-        ++round;
+        closure<RB>(A, grid);
     }
-    // every flag slot is zero again here; UP and peel use disjoint slots so a thread that has left one
-    // loop can never disturb a flag another thread is still reading
-}
-
-// ------------------------------------------------------------------------------------------------
-// Frontier closure (large problems, grid-wide).  Once every problem is closed under unit propagation and peeling
-// (after simplify()), fixing a variable can only create unit clauses among the clauses that hold a variable
-// de-activated in the previous round, and pure literals among the variables of clauses de-activated since: the
-// rounds below are the rounds of closure() -- same phases, same synchronous semantics, same helper arithmetic --
-// run over those lists instead of over all F clauses and V variables (8.9 -> ms per decimation iteration at
-// 8 x n = 1 M, where a round's full scan gathers 100 M node flags to find a dozen nodes).
-//   clause list (ping-pong by UP round)   : clauses to test for unit-ness
-//   variable list (ping-pong by peel round): variables to test for purity; filled during the whole UP stage
-//   unit list (by UP round parity)         : variables some unit clause of the round points at
-// List entries are unique per epoch (stamps).  A list that overflows, or a problem wiped by the single-conflict
-// quirk, sends the rest of the closure through the full scans.
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void fr_push(const pdp_state& s, int list, int32_t* stamp, int id, int epoch) {
-    if (atomicExch(&stamp[id], epoch) == epoch) return;
-    const int k = atomicAdd(&s.ctrl[CTRL_FR_N + list], 1);
-    if (k < s.fr_cap) s.fr_list[list][k] = id; else s.ctrl[CTRL_FR_OVER] = 1;
-}
-__device__ __forceinline__ int fr_len(const pdp_state& s, int slot) {
-    const int n = s.ctrl[slot];
-    return n < s.fr_cap ? n : s.fr_cap;
-}
-// de-activate clause a and queue its still-active variables for the purity test
-__device__ __forceinline__ void fr_deactivate_clause(const pdp_graph& g, const pdp_state& s, int a, int vlist, int epv) {
-    deactivate_clause(g, s, a);
-    for (int c = g.cl_ptr[a]; c < g.cl_ptr[a + 1]; ++c) {
-        const int j = (int)(g.c_var[c] & PDP_IDX_MASK);
-        if (s.av[j]) fr_push(s, vlist, s.stamp_v, j, epv);
-    }
-}
-// fix_variable that also queues: clauses made true -> their variables (purity); the other clauses of i -> unit test
-__device__ __forceinline__ void fr_fix_variable(const pdp_graph& g, const pdp_state& s, int i, float sg, int clist, int epc,
-                                                int vlist, int epv) {
-    const int beg = g.var_ptr[i], end = g.var_ptr[i + 1];
-    for (int p = beg; p < end; ++p) {
-        const float lit = (g.v_cedge[p] & PDP_SIGN_BIT) ? -1.f : 1.f;
-        const int a = g.v_cls[p];
-        if (!s.af[a]) continue;
-        if (lit * sg > 0.f) fr_deactivate_clause(g, s, a, vlist, epv);
-        else fr_push(s, clist, s.stamp_c, a, epc);
-    }
-    deactivate_variable(g, s, i);
-    s.sol[i] = (sg + 1.f) / 2.0f;
-}
-
-// fix_variable / fr_fix_variable by the 32 lanes of a warp (lanes over the variable's edges): the decimation step of a
-// large problem fixes ONE variable, and a single thread walking its ~40 dependent global updates was 0.4 ms
-__device__ __forceinline__ void warp_fix_variable(const pdp_graph& g, const pdp_state& s, int i, float sg, bool frontier, int epc, int epv) {
-    const int beg = g.var_ptr[i], end = g.var_ptr[i + 1];
-    for (int p = beg + lane_id(); p < end; p += 32) {
-        const float lit = (g.v_cedge[p] & PDP_SIGN_BIT) ? -1.f : 1.f;
-        const int a = g.v_cls[p];
-        if (s.af[a]) {
-            if (lit * sg > 0.f) { if (frontier) fr_deactivate_clause(g, s, a, 2, epv); else deactivate_clause(g, s, a); }
-            else if (frontier) fr_push(s, 0, s.stamp_c, a, epc);
-        }
-        mask_edge(g, g.p_vpos[p], g.p_qpos[p]);
-    }
-    if (lane_id() == 0) { s.av[i] = 0; s.sol[i] = (sg + 1.f) / 2.0f; }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -977,165 +1028,6 @@ __device__ __forceinline__ void sel_grid(const KArgs& A, cg::grid_group& grid, c
             if (st > 0 && lane_id() == 0) s.ctrl[CTRL_SEL + ((pass + 1) & 1)] = 1;
         }
         grid.sync();
-    }
-}
-
-__device__ __forceinline__ void fr_find_units(const KArgs& A, int clist, int ulist, int flag_slot) {
-    const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    const int n = fr_len(s, CTRL_FR_N + clist);
-    WARP_STRIDED(x, n) {
-        if (x >= n) continue;
-        const int a = s.fr_list[clist][x];
-        if (!s.af[a]) continue;
-        int j; bool neg;
-        if (clause_unit(g.c_var, g.cl_ptr[a], g.cl_ptr[a + 1], s.av, j, neg)) {
-            s.single[a] = 1;
-            if (atomicAdd(&s.up_cnt[j], 1) == 0) {
-                const int k = atomicAdd(&s.ctrl[CTRL_FR_NU + ulist], 1);
-                if (k < s.fr_cap) s.fr_unit[ulist][k] = j; else s.ctrl[CTRL_FR_OVER] = 1;
-            }
-            atomicAdd(&s.up_ev[j], neg ? -1 : 1);
-            s.ctrl[flag_slot] = 1;
-        }
-    }
-}
-__device__ __forceinline__ void fr_find_conflicts(const KArgs& A, int ulist) {
-    const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    const int n = fr_len(s, CTRL_FR_NU + ulist);
-    WARP_STRIDED(x, n) {
-        if (x >= n) continue;
-        const int i = s.fr_unit[ulist][x];
-        const int cnt = s.up_cnt[i];
-        if (cnt > 0 && abs(s.up_ev[i]) != cnt) {
-            if (atomicAdd(&s.conflicts[g.bvm[i]], 1) == 0) s.ctrl[CTRL_FR_WIPE] = 1;   // one conflict may mean a wipe
-        }
-    }
-}
-// up_apply_conflicts over the lists; the wipe of single-conflict problems scans their nodes (rare)
-template <bool RB>
-__device__ __forceinline__ void fr_apply_conflicts(const KArgs& A, int clist, int vlist, int epv) {
-    const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    const int n = fr_len(s, CTRL_FR_N + clist);
-    WARP_STRIDED(x, n) {
-        if (x >= n) continue;
-        const int a = s.fr_list[clist][x];
-        if (s.single[a]) { fr_deactivate_clause(g, s, a, vlist, epv); s.single[a] = 0; s.masked[g.bfm[a]] = 1; }
-    }
-    if (s.ctrl[CTRL_FR_WIPE]) {
-        const int64_t m = g.V > g.F ? g.V : g.F;
-        WARP_STRIDED(i, m) {
-            if (i < g.F && s.af[i] && !s.single[i] && s.conflicts[g.bfm[i]] == 1) deactivate_clause(g, s, (int)i);
-            if (i < g.V && s.av[i] && s.conflicts[g.bvm[i]] == 1) deactivate_variable(g, s, (int)i);
-        }
-    }
-    WARP_STRIDED(b, g.B) {
-        if (b < g.B && s.conflicts[b] >= 1) { s.is_sat[b] = 0.f; s.flags[b] |= PDP_FLAG_UP_CONFLICT; s.masked[b] = 1; if (RB) rb_mark(A, (int)b); }
-    }
-}
-__device__ __forceinline__ void fr_assign(const KArgs& A, int ulist, int clist_next, int epc, int vlist, int epv) {
-    const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    const int n = fr_len(s, CTRL_FR_NU + ulist);
-    WARP_STRIDED(x, n) {
-        if (x >= n) continue;
-        const int i = s.fr_unit[ulist][x];
-        const int cnt = s.up_cnt[i];
-        if (cnt > 0) {
-            const int ev = s.up_ev[i];
-            s.up_cnt[i] = 0; s.up_ev[i] = 0;
-            if (s.av[i] && abs(ev) == cnt) fr_fix_variable(g, s, i, ev > 0 ? 1.f : -1.f, clist_next, epc, vlist, epv);
-        }
-    }
-}
-__device__ __forceinline__ void fr_peel_find(const KArgs& A, int vlist, int flag_slot) {
-    const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    const int n = fr_len(s, CTRL_FR_N + vlist);
-    WARP_STRIDED(x, n) {
-        if (x >= n) continue;
-        const int i = s.fr_list[vlist][x];
-        if (!s.av[i]) continue;
-        float val;
-        if (var_pure(g, s.af, i, val)) {
-            s.pure[i] = 1;
-            s.sol[i] = val;
-            s.ctrl[flag_slot] = 1;
-        }
-    }
-}
-__device__ __forceinline__ void fr_peel_apply(const KArgs& A, int vlist, int vlist_next, int epv) {
-    const pdp_graph& g = A.g; const pdp_state& s = A.s;
-    const int n = fr_len(s, CTRL_FR_N + vlist);
-    WARP_STRIDED(x, n) {
-        if (x >= n) continue;
-        const int i = s.fr_list[vlist][x];
-        if (!s.pure[i]) continue;
-        s.pure[i] = 0;
-        const int beg = g.var_ptr[i], end = g.var_ptr[i + 1];
-        for (int p = beg; p < end; ++p) {
-            const int a = g.v_cls[p];
-            if (s.af[a]) fr_deactivate_clause(g, s, a, vlist_next, epv);
-        }
-        deactivate_variable(g, s, i);
-        s.masked[g.bvm[i]] = 1;
-    }
-}
-
-// Called by ALL threads of the cooperative grid after select_and_fix_phase<frontier> and a grid barrier: clause list 0
-// and variable list 2 hold what the fixes touched (epochs epc0 / epv0, both already stored in the control block).
-template <bool RB = false>
-__device__ PDP_COLD void closure_frontier(const KArgs& A, cg::grid_group& grid) {
-    const pdp_state& s = A.s;
-    int epc = s.ctrl[CTRL_FR_EPC], epv = s.ctrl[CTRL_FR_EPV];
-    int round = 0, cur = 0;
-    bool fallback = false;
-    for (;;) {   // unit propagation (solver.py:234-273)
-        const int slot = CTRL_FLAG_A + (round & 1), other = CTRL_FLAG_A + ((round + 1) & 1);
-        const int ul = round & 1;
-        if (s.ctrl[CTRL_FR_OVER]) { fallback = true; break; }        // uniform: written before the last barrier
-        fr_find_units(A, cur, ul, slot);
-        if (gtid() == 0) { s.ctrl[other] = 0; s.ctrl[CTRL_FR_N + (cur ^ 1)] = 0; s.ctrl[CTRL_FR_NU + (ul ^ 1)] = 0; }
-        grid.sync();
-        if (!s.ctrl[slot]) break;
-        fr_find_conflicts(A, ul);
-        grid.sync();
-        fr_apply_conflicts<RB>(A, cur, 2, epv);
-        grid.sync();
-        ++epc;
-        fr_assign(A, ul, cur ^ 1, epc, 2, epv);
-        up_clear_conflicts(A);
-        if (gtid() == 0) s.ctrl[CTRL_FR_WIPE] = 0;
-        grid.sync();
-        cur ^= 1;
-        ++round;
-    }
-    if (!fallback && s.ctrl[CTRL_FR_OVER]) fallback = true;
-    if (!fallback) {
-        int vc = 2;
-        round = 0;
-        for (;;) {   // peeling (solver.py:188-203)
-            const int slot = CTRL_FLAG_C + (round & 1), other = CTRL_FLAG_C + ((round + 1) & 1);
-            if (s.ctrl[CTRL_FR_OVER]) { fallback = true; break; }
-            fr_peel_find(A, vc, slot);
-            if (gtid() == 0) { s.ctrl[other] = 0; s.ctrl[CTRL_FR_N + (vc ^ 1)] = 0; }
-            grid.sync();
-            if (!s.ctrl[slot]) break;
-            ++epv;
-            fr_peel_apply(A, vc, vc ^ 1, epv);
-            grid.sync();
-            vc ^= 1;
-            ++round;
-        }
-    }
-    grid.sync();
-    if (gtid() == 0) {
-        s.ctrl[CTRL_FR_EPC] = epc + 1; s.ctrl[CTRL_FR_EPV] = epv + 1;
-        for (int i = 0; i < 4; ++i) s.ctrl[CTRL_FR_N + i] = 0;
-        s.ctrl[CTRL_FR_NU] = 0; s.ctrl[CTRL_FR_NU + 1] = 0; s.ctrl[CTRL_FR_OVER] = 0; s.ctrl[CTRL_FR_WIPE] = 0;
-    }
-    if (fallback) {
-        // per-round scratch is clean at a round boundary; the full scans finish the closure from the current masks
-        if (gtid() == 0) { s.ctrl[CTRL_FLAG_A] = 0; s.ctrl[CTRL_FLAG_A + 1] = 0; s.ctrl[CTRL_FLAG_C] = 0; s.ctrl[CTRL_FLAG_C + 1] = 0; }
-        grid.sync();
-        closure<RB>(A, grid);
     }
 }
 

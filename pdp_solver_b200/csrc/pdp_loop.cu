@@ -72,7 +72,7 @@ __device__ __forceinline__ void decide_phase(const KArgs& A, int iter, const pdp
 __device__ __forceinline__ void select_and_fix_phase(const KArgs& A, int iter, bool frontier) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
     const int slot = CTRL_FIX + (iter & 1);
-    const int epc = s.ctrl[CTRL_FR_EPC], epv = s.ctrl[CTRL_FR_EPV];
+    const ListQueue q = frontier_queue(s);
     // warp per problem: every lane takes the same decisions, the fix itself is spread over the lanes
     for (int64_t b = gwarp(); b < g.B; b += gwarps()) {
         if (!s.conv[b]) continue;
@@ -81,7 +81,8 @@ __device__ __forceinline__ void select_and_fix_phase(const KArgs& A, int iter, b
             const float sg = sgnf(s.score[i]);
             if (sg != 0.f && s.av[i]) {
                 __syncwarp();     // everybody has read av[i] before lane 0 clears it
-                warp_fix_variable(g, s, i, sg, frontier, epc, epv);   // + the touched nodes, for closure_frontier
+                if (frontier) fix_variable<32>(g, s, i, sg, q);
+                else fix_variable<32>(g, s, i, sg);
                 if (lane_id() == 0) {
                     s.masked[b] = 1; s.dirty[b] = 1;
                     s.ctrl[slot] = 1; s.ctrl[CTRL_ANY_DIRTY] = 1;
@@ -95,7 +96,7 @@ __device__ __forceinline__ void select_and_fix_phase(const KArgs& A, int iter, b
 }
 
 // the fix step of the fused loop with a fraction: the arg-max fixes (K_b == 1) and the top-K fixes of the other problems,
-// one warp per taken variable (warp_fix_variable, + the frontier lists).  Fixes of one step commute: a clause is
+// one warp per taken variable (fix_variable<32>, + the frontier lists).  Fixes of one step commute: a clause is
 // de-activated iff it holds a newly true literal (_set_variable_core, solver.py:205-226).
 __device__ __forceinline__ void frac_select_and_fix(const KArgs& A, cg::grid_group& grid, int iter, bool frontier) {
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
@@ -105,7 +106,7 @@ __device__ __forceinline__ void frac_select_and_fix(const KArgs& A, cg::grid_gro
     select_and_fix_phase(A, iter, frontier);
     if (rb) grid.sync();   // the snapshots are complete before the top-K fixes
     const int slot = CTRL_FIX + (iter & 1);
-    const int epc = s.ctrl[CTRL_FR_EPC], epv = s.ctrl[CTRL_FR_EPV];
+    const ListQueue q = frontier_queue(s);
     for (int64_t base = gwarp() * 32; base < g.V; base += gwarps() * 32) {
         const int64_t i = base + lane_id();
         bool take = false;
@@ -123,7 +124,8 @@ __device__ __forceinline__ void frac_select_and_fix(const KArgs& A, cg::grid_gro
             m &= m - 1;
             const int vi = (int)__shfl_sync(0xffffffffu, i, src);
             const float vsg = __shfl_sync(0xffffffffu, sg, src);
-            warp_fix_variable(g, s, vi, vsg, frontier, epc, epv);
+            if (frontier) fix_variable<32>(g, s, vi, vsg, q);
+            else fix_variable<32>(g, s, vi, vsg);
             if (lane_id() == 0) {
                 const int b = g.bvm[vi];
                 s.masked[b] = 1; s.dirty[b] = 1;
@@ -306,8 +308,8 @@ k_sp_run(const __grid_constant__ KArgs A, const __grid_constant__ pdp_sp_params 
     }
 }
 
-// SATProblem.simplify on every problem (solver.py:281-285)
-__global__ void __launch_bounds__(256) k_simplify(const __grid_constant__ KArgs A) {
+// SATProblem.simplify on every problem (solver.py:281-285).  (256, 4): coop_blocks launches at most 4 CTAs per SM
+__global__ void __launch_bounds__(256, 4) k_simplify(const __grid_constant__ KArgs A) {
     cg::grid_group grid = cg::this_grid();
     const pdp_state& s = A.s;
     WARP_STRIDED(b, A.g.B) { if (b < A.g.B) s.dirty[b] = 1; }
@@ -318,7 +320,7 @@ __global__ void __launch_bounds__(256) k_simplify(const __grid_constant__ KArgs 
 }
 
 // SATProblem.set_variables (solver.py:275-279): assignment [V] float in {-1,0,1}
-__global__ void __launch_bounds__(256) k_set_variables(const __grid_constant__ KArgs A, const float* __restrict__ asg) {
+__global__ void __launch_bounds__(256, 4) k_set_variables(const __grid_constant__ KArgs A, const float* __restrict__ asg) {
     cg::grid_group grid = cg::this_grid();
     const pdp_graph& g = A.g; const pdp_state& s = A.s;
     WARP_STRIDED(b, g.B) { if (b < g.B) s.dirty[b] = 1; }
