@@ -224,6 +224,30 @@ size_t pdp_rollback_scratch_bytes(int64_t V, int64_t F, int64_t B);
 int pdp_set_conflict_rollback(pdp_ctx* ctx, void* d_scratch, size_t bytes);
 int pdp_get_rollbacks(pdp_ctx* ctx, int32_t* d_count, int32_t* d_last_iter, void* stream);
 
+/* Model type `reinforce` (SP with the reinforcement term, Chavas, Furtlehner, Mezard, Zecchina, J. Stat. Mech. 2005;
+ * reference ReinforceSurveyPropagatorSolver, solver.py:598-610) in pdp_sp_run.  With the mode on, iteration k of the runs
+ * since pdp_set_reinforce (k = 0, 1, ...) is, in the reference's order (solver.py:355-386):
+ *   1. the SP sweep with params->pi and the external forces ext = function_state[:,1] as input (as without the mode);
+ *   2. with check_termination, previous surveys and at least one active variable in the batch: a still-active problem whose
+ *      sparse_max(smooth-max_i(|eta_prev - eta| * em) * av) (per-problem min, the p-d-p convergence statistic) is <= 0.01
+ *      retires (ReinforceDecimator, pdp_decimate.py:204-215); its freeze iteration is recorded;
+ *   3. if d_coins[k] < decimation_probability: every variable is scored (SurveyScorer with pi, pdp_score) from the new
+ *      surveys and the current forces, and every edge of variable i takes ext = sign(score_i): on all edges without
+ *      check_termination, else as m * sign + (1 - m) * ext with m = 1 iff the problem is active after step 2;
+ *   4. with check_termination: an active variable's solution becomes [sum of its forces > 0] (ReinforcePredictor +
+ *      _update_solution) -- on the run's first iteration and where step 3 ran, the only iterations it can change;
+ *   5. with check_termination and flags bit 3 clear: the termination check of the p-d-p loop (trainer.py:150-162, a solved
+ *      replica retires its problem) on the problems step 4 touched.
+ * No variable is fixed; tolerance, t_max, the decimation fraction and conflict rollback are not used.  Without full_state
+ * the run takes the blocked passes where the batch allows them, with the pi terms per variable: this needs the forces
+ * loaded by pdp_load_state to be the same on all edges of each variable (step 3 keeps them so); when they are not, the
+ * runs take the generic passes until the next load.  Without full_state, pdp_store_state re-derives q_s and q_* with the
+ * forces the last sweep read (before that iteration's coin).  d_coins: device fp32, n_coins of them, owned by the caller
+ * until the mode is turned off; NULL turns the mode off.  Off after pdp_create; pdp_reset keeps the mode and the coin
+ * index k.  pdp_sp_run returns PDP_ERR_ARG when the iterations of the runs since pdp_set_reinforce, each run counted with
+ * all of its params->iterations, would exceed n_coins. */
+int pdp_set_reinforce(pdp_ctx* ctx, const float* d_coins, int32_t n_coins, float decimation_probability);
+
 /* IdentityPredictor.forward(last_call=True), reference pdp/nn/pdp_predict.py:118-128.
  * pdp_count_active_variables syncs the stream.  d_draws holds >= n_active uniform draws that are
  * consumed by the active variables in batch-global variable order (like torch.rand(n_active)). */

@@ -64,6 +64,7 @@ SIGNATURES = {
     "pdp_decimation_select": (ctypes.c_int, [P, P, P, P, F32, P, P]),
     "pdp_rollback_scratch_bytes": (ctypes.c_size_t, [I64, I64, I64]),
     "pdp_set_conflict_rollback": (ctypes.c_int, [P, P, ctypes.c_size_t]),
+    "pdp_set_reinforce": (ctypes.c_int, [P, P, I32, F32]),
     "pdp_get_rollbacks": (ctypes.c_int, [P, P, P, P]),
     "pdp_debug_check_edge_mask": (ctypes.c_int, [P, P, P]),
     "pdp_set_trace_buffer": (ctypes.c_int, [P, P, I32]),

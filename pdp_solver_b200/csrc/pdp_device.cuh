@@ -32,6 +32,8 @@ struct KArgs {
     // conflict rollback (pdp_set_conflict_rollback): the snapshot of the problems a step decimates, indexed like the state
     // (all null: rollback off)
     struct { float* sol; float* is_sat; uint8_t* av; uint8_t* af; } rb;
+    // reinforce (pdp_set_reinforce): the coins, decimation_probability, and whether this run starts at coin 0
+    struct { const float* coins; float p; float pi; int32_t fresh; } rf;
 };
 
 __device__ __forceinline__ int lane_id() { return threadIdx.x & 31; }
@@ -275,6 +277,25 @@ __device__ __forceinline__ void sp_var_prepare(float P, float N, float s, float&
 }
 __device__ __forceinline__ float sp_var_finish(float same_base, float opp, float O, float y) {
     const float same = same_base - y;
+    const float S = X30(same);
+    const float dc = X30(same + opp);
+    const float u = S * (1.f - O), v = O * (1.f - S);
+    const float total = u + v + dc;
+    return pdp_divf(u, total);
+}
+
+// the same with the two pi terms of a variable whose external force is the same on all its edges (reinforce on the
+// blocked passes): l_same / l_opp = log(max(1 - pi [ext == s], 1e-40)) / log(max(1 - pi [ext == -s], 1e-40)), added in
+// the order of sp_var_update
+__device__ __forceinline__ void sp_var_prepare_pi(float P, float N, float s, float l_opp, float& same_base, float& opp, float& O) {
+    same_base = 0.5f * (1.f + s) * P + 0.5f * (1.f - s) * N;
+    opp = 0.5f * (1.f - s) * P + 0.5f * (1.f + s) * N;
+    opp += l_opp;
+    O = X30(opp);
+}
+__device__ __forceinline__ float sp_var_finish_pi(float same_base, float l_same, float opp, float O, float y) {
+    float same = same_base - y;
+    same += l_same;
     const float S = X30(same);
     const float dc = X30(same + opp);
     const float u = S * (1.f - O), v = O * (1.f - S);

@@ -129,6 +129,7 @@ void carve(pdp_ctx* c, Carver& k, int64_t E, int64_t V, int64_t F, int64_t B) {
     s.want_score = k.take<uint8_t>(B);
     s.have_score = k.take<uint8_t>(B);
     s.last_d = k.take<float>(B);
+    s.rf_coin_iter = k.take<int32_t>(B);
     s.stamp_c = k.take<int32_t>(F);
     s.stamp_v = k.take<int32_t>(V);
     s.sel_hist = k.take<uint32_t>(B * PDP_SEL_BINS);
@@ -254,14 +255,15 @@ __global__ void k_reset_state(pdp_graph g, pdp_state s, int64_t V, int64_t F, in
         if (i < B) {
             s.is_sat[i] = 0.5f; s.active[i] = 1; s.counters[i] = 0; s.freeze_iter[i] = -1; s.flags[i] = 0;
             s.masked[i] = 0; s.dirty[i] = 1; s.conv[i] = 0; s.nanflag[i] = 0; s.nanpend[i] = 0; s.n_unsat[i] = 0; s.conflicts[i] = 0;
-            s.nav[i] = 0; s.arg_idx[i] = 0x7fffffff; s.energy[i] = 0; s.want_score[i] = 0; s.have_score[i] = 0; s.last_d[i] = 0.f;
+            s.nav[i] = 0; s.arg_idx[i] = 0x7fffffff; s.energy[i] = 0; s.want_score[i] = 0; s.have_score[i] = 0; s.rf_coin_iter[i] = 0; s.last_d[i] = 0.f;
             s.st_max[2 * i] = 0u; s.st_max[2 * i + 1] = 0u; s.st_min[2 * i] = 0x7f800000u; s.st_min[2 * i + 1] = 0x7f800000u;
             s.st_nan[i] = 0u; s.c_max[i] = 0u; s.c_min[i] = 0x7f800000u; s.c_nan[i] = 0u;
             s.sel_need[i] = -1; s.sel_sh[i] = 0; s.sel_pref[i] = 0ull;
             s.rb_h[i] = 0; s.rb_count[i] = 0; s.rb_last[i] = 0; s.rb_snap[i] = 0;
             for (int j = 0; j < PDP_SEL_BINS; ++j) s.sel_hist[i * PDP_SEL_BINS + j] = 0u;
         }
-        if (i < CTRL_SIZE) s.ctrl[i] = (i == CTRL_NUM_ACTIVE) ? (int32_t)B
+        // (the reinforce coin index and the uniformity of the loaded forces survive a reset: pdp_set_reinforce / the load set them)
+        if (i < CTRL_SIZE && i != CTRL_RF_K && i != CTRL_RF_MIXED) s.ctrl[i] = (i == CTRL_NUM_ACTIVE) ? (int32_t)B
                                        : ((i == CTRL_ANY_DIRTY || i == CTRL_FR_EPC || i == CTRL_FR_EPV || i == CTRL_NATIVE) ? 1 : 0);
     }
 }

@@ -162,10 +162,82 @@ __device__ __forceinline__ void termination_phase(const KArgs& A, int iter, int 
     if (gtid() == 0) s.ctrl[CTRL_ANY_DIRTY] = 0;
 }
 
+// ------------------------------------------------------------------------------------------------
+// model type `reinforce` (pdp_set_reinforce): ReinforceDecimator (pdp_decimate.py:204-233) and ReinforcePredictor +
+// _update_solution (pdp_predict.py:221-226, solver.py:388-399) in place of the SequentialDecimator phases
+// ------------------------------------------------------------------------------------------------
+// retire test: with the active-mask semantics on, previous surveys and some active variable in the batch, a problem whose
+// statistic sparse_max(smooth-max(|eta_prev - eta| * em) * av) -- the decimator statistic of the p-d-p passes -- is <= 0.01
+// is retired
+__device__ __forceinline__ void rf_decide_phase(const KArgs& A, int iter, const pdp_sp_params& prm, bool has_prev) {
+    const pdp_state& s = A.s;
+    const bool test = prm.check_termination && has_prev && s.ctrl[CTRL_RF_NAV] > 0;
+    WARP_STRIDED(b, A.g.B) {
+        if (b >= A.g.B) continue;
+        if (s.nanpend[b]) { s.nanpend[b] = 0; s.nanflag[b] = 1; s.ctrl[CTRL_ANY_NAN] = 1; }
+        if (!s.active[b]) continue;
+        const uint32_t nanb = s.st_nan[b];
+        if (test) {
+            const uint32_t mx1 = s.st_max[2 * b + 1], mn1 = s.st_min[2 * b + 1];
+            const bool seen1 = (mn1 != 0x7f800000u) || (mx1 != 0u);
+            const float D = (nanb & 2u) ? __int_as_float(0x7fc00000) : (seen1 ? sparse_max_round(u2f(mx1), u2f(mn1)) : -1.f);
+            if (D <= 0.01f) {
+                s.active[b] = 0;
+                s.freeze_iter[b] = iter;
+                atomicSub(&s.ctrl[CTRL_NUM_ACTIVE], 1);
+            }
+        }
+        if (nanb) s.flags[b] |= PDP_FLAG_CONTRADICTION;
+        s.st_max[2 * b] = 0u; s.st_max[2 * b + 1] = 0u;
+        s.st_min[2 * b] = 0x7f800000u; s.st_min[2 * b + 1] = 0x7f800000u;
+        s.st_nan[b] = 0u; s.nav[b] = 0;
+    }
+}
+
+// coin: every variable is scored from the new surveys and its current forces (SurveyScorer with pi), then its edges take
+// sign(score) -- with the active-mask semantics (blend) through the reference's arithmetic blend m * sign + (1 - m) * ext,
+// m = the problem is still active.  update: an active variable's solution becomes [sum of its forces > 0] (ascending edge
+// order) and the active problems are queued for the CNF check.  Both are per variable: no barrier between them.
+// stash (a run without the full [E,3] state): the forces a coin changes (those of the problems still active) keep their old
+// values in s.qs by edge slot p, unused in such a run, and the problem the iteration (rf_coin_iter), so that
+// pdp_store_state re-derives q_s and q_* of a problem's last sweep with the forces that sweep read
+__device__ __forceinline__ void rf_force_phase(const KArgs& A, int iter, int w, float pi, bool coin, bool blend, bool update,
+                                               bool stash) {
+    const pdp_graph& g = A.g; const pdp_state& s = A.s;
+    WARP_STRIDED(i, g.V) {
+        if (i >= g.V) continue;
+        const int beg = g.var_ptr[i], end = g.var_ptr[i + 1];
+        if (coin) {
+            const float sg = sgnf(score_variable(g, s, s.eta[w], (int)i, pi));
+            const float m = (float)s.active[g.bvm[i]];
+            const bool changes = !blend || m != 0.f;
+            for (int p = beg; p < end; ++p) {
+                const float e = s.ext[p];
+                if (stash && changes) s.qs[p] = e;
+                s.ext[p] = blend ? m * sg + (1.f - m) * e : sg;
+            }
+        }
+        if (update && s.av[i]) {
+            float f = 0.f;
+            for (int p = beg; p < end; ++p) f += s.ext[p];
+            s.sol[i] = (f > 0.f) ? 1.f : 0.f;
+        }
+    }
+    if (coin && stash) WARP_STRIDED(b, g.B) { if (b < g.B && (!blend || s.active[b])) s.rf_coin_iter[b] = iter; }
+    if (update) {
+        WARP_STRIDED(b, g.B) { if (b < g.B && s.active[b]) s.dirty[b] = 1; }
+        // active variables now carry values: an active clause may be satisfied (CTRL_NATIVE)
+        if (gtid() == 0) { s.ctrl[CTRL_ANY_DIRTY] = 1; s.ctrl[CTRL_NATIVE] = 0; }
+    }
+}
+
 // FAST: the blocked shared-memory passes (pi == 0, q_u only); otherwise the generic passes.
 // FRAC: a decimation fraction is set (pdp_set_decimation_fraction); a separate instance, so that the top-K selection
-// takes nothing from the registers of the instance the reference's rule runs in
-template <bool FAST, bool FULL, int CTAS, bool FRAC>
+// takes nothing from the registers of the instance the reference's rule runs in.
+// REINF: model type `reinforce` (pdp_set_reinforce): the retire test, the coin-driven external forces and the predictor
+// replace the decimation phases; separate instances for the same reason.  With FAST the sweep takes the blocked passes
+// with per-variable pi terms, unless the loaded forces are not uniform over some variable's edges (CTRL_RF_MIXED)
+template <bool FAST, bool FULL, int CTAS, bool FRAC, bool REINF = false>
 __global__ void __launch_bounds__(FAST ? SweepCfg<CTAS>::kThreads : 256, FAST ? CTAS : 1)
 k_sp_run(const __grid_constant__ KArgs A, const __grid_constant__ pdp_sp_params prm, int32_t* d_iters_done) {
     extern __shared__ __align__(128) unsigned char smem_dyn[];
@@ -176,6 +248,7 @@ k_sp_run(const __grid_constant__ KArgs A, const __grid_constant__ pdp_sp_params 
     bool use_mask = s.ctrl[CTRL_USE_MASK] != 0;
     bool em_set = s.ctrl[CTRL_EM_SET] != 0;
     int gen_left = FAST ? s.ctrl[CTRL_GEN_ITERS] : 0;
+    const bool rf_mixed = REINF && s.ctrl[CTRL_RF_MIXED] != 0;
     const int rep = prm.batch_replication > 1 ? prm.batch_replication : 1;
     const bool local_ok = A.g.contiguous_problems && rep == 1 && !(prm.flags & 2);
     const bool frontier = s.ctrl[CTRL_CLOSED] != 0 && !(prm.flags & 4);   // flags bit 2: full-scan closure (A/B, tests)
@@ -200,6 +273,11 @@ k_sp_run(const __grid_constant__ KArgs A, const __grid_constant__ pdp_sp_params 
         sm_rank = sm_rank_s;
     }
     if (gtid() == 0) { s.ctrl[CTRL_NEXT_CBLK] = 0; s.ctrl[CTRL_NEXT_VBLK] = 0; s.ctrl[CTRL_LOC_COUNT] = 0; s.ctrl[CTRL_LOC_NEXT] = 0; }
+    int rk = 0;   // REINF: index of this iteration's coin
+    if (REINF) {
+        rk = A.rf.fresh ? 0 : s.ctrl[CTRL_RF_K];
+        if (gtid() == 0) s.ctrl[CTRL_RF_NAV] = 0;
+    }
 #ifdef PDP_PHASE_TIMING
 #define GRID_SYNC() do { const long long _g0 = clock64(); grid.sync(); if (threadIdx.x == 0 && A.trace) atomicAdd(&A.trace[7], (int)((clock64() - _g0) >> 10)); } while (0)
 #else
@@ -209,6 +287,12 @@ k_sp_run(const __grid_constant__ KArgs A, const __grid_constant__ pdp_sp_params 
     const long long _kernel_t0 = clock64();
 #endif
     grid.sync();   // everybody has read the control block before anyone may change it
+    if (REINF) {   // `_active_variables.sum() > 0` of the retire test is batch-global (read three barriers later)
+        WARP_STRIDED(i, A.g.V) {
+            const unsigned m = __ballot_sync(0xffffffffu, i < A.g.V && s.av[i]);
+            if (lane_id() == 0 && m) atomicAdd(&s.ctrl[CTRL_RF_NAV], __popc(m));
+        }
+    }
 #ifdef PDP_PHASE_TIMING
     long long _lt = clock64();
 #define LOOP_T(slot_) do { if (threadIdx.x == 0 && A.trace) { const long long _n = clock64(); atomicAdd(&A.trace[slot_], (int)((_n - _lt) >> 10)); _lt = _n; } } while (0)
@@ -219,7 +303,7 @@ k_sp_run(const __grid_constant__ KArgs A, const __grid_constant__ pdp_sp_params 
         ++iter;
         const int r = (iter - 1) & 1, w = iter & 1;
         LOOP_T(23);
-        const bool blocked = FAST && gen_left <= 0;
+        const bool blocked = FAST && gen_left <= 0 && !rf_mixed;
         if (gen_left > 0) --gen_left;
         // ---- propagate, clause side: eta(t) from q(t-1)   (pdp_propagate.py:161-175)
         if (blocked) {
@@ -235,20 +319,30 @@ k_sp_run(const __grid_constant__ KArgs A, const __grid_constant__ pdp_sp_params 
         // ---- propagate, variable side: q(t) from eta(t-1) (pdp_propagate.py:184-218), fused with the
         //      decimator statistics of eta(t) against eta(t-1) (pdp_decimate.py:127-143)
         if (blocked) {
-            blk_var_pass<CTAS>(A, r, use_mask, has_prev, em_set, smem_dyn, sm_rank, bb);
+            blk_var_pass<CTAS, REINF>(A, r, use_mask, has_prev, em_set, smem_dyn, sm_rank, bb);
         } else {
             gen_var_side<GEN_ALL, FULL>(A, r, use_mask, prm.pi);
-            gen_stats<GEN_ALL>(A, w, has_prev, em_set);
+            // (reinforce reads the statistics only in its retire test)
+            if (!REINF || (prm.check_termination && has_prev)) gen_stats<GEN_ALL>(A, w, has_prev, em_set);
         }
         LOOP_T(18);
         GRID_SYNC();
         if (gtid() == 0) s.ctrl[CTRL_NEXT_CBLK] = 0;   // the variable pass is over; the next clause pass is a barrier away
         LOOP_T(19);
         // ---- decimate: decisions -> (score, argmax, fix, simplify)
-        decide_phase(A, iter, prm, has_prev, local_ok, blocked);
+        if (REINF) rf_decide_phase(A, iter, prm, has_prev);
+        else decide_phase(A, iter, prm, has_prev, local_ok, blocked);
         GRID_SYNC();
         LOOP_T(20);
-        if (local_ok && s.ctrl[CTRL_CONV + (iter & 1)]) {
+        if (REINF) {
+            // the prediction changes only where the forces do, and on a run's first iteration
+            const bool coin = A.rf.coins[rk++] < A.rf.p;
+            const bool update = prm.check_termination && (coin || it == 0);
+            if (coin || update) {
+                rf_force_phase(A, iter, w, prm.pi, coin, prm.check_termination != 0, update, !FULL);
+                GRID_SYNC();
+            }
+        } else if (local_ok && s.ctrl[CTRL_CONV + (iter & 1)]) {
             // converged problems one CTA can walk: scoring, arg-max, fix, closure, CNF check, termination, CTA-local
             loc_decimate_all<FRAC>(A, iter, w, prm.pi, prm.check_termination != 0, FAST ? smem_dyn : nullptr,
                                    FAST ? SweepCfg<CTAS>::kSmem : 0);
@@ -256,7 +350,7 @@ k_sp_run(const __grid_constant__ KArgs A, const __grid_constant__ pdp_sp_params 
             GRID_SYNC();
             LOOP_T(22);
         }
-        if (s.ctrl[local_ok ? (CTRL_CONVBIG + (iter & 1)) : (CTRL_CONV + (iter & 1))]) {
+        if (!REINF && s.ctrl[local_ok ? (CTRL_CONVBIG + (iter & 1)) : (CTRL_CONV + (iter & 1))]) {
             LOOP_T(23);
             score_phase(A, w, prm.pi);
             GRID_SYNC();
@@ -304,6 +398,7 @@ k_sp_run(const __grid_constant__ KArgs A, const __grid_constant__ pdp_sp_params 
         s.ctrl[CTRL_ITER] = iter; s.ctrl[CTRL_HAS_PREV] = has_prev; s.ctrl[CTRL_USE_MASK] = use_mask;
         s.ctrl[CTRL_EM_SET] = em_set; s.ctrl[CTRL_ITERS_THIS_RUN] = executed;
         if (FAST) s.ctrl[CTRL_GEN_ITERS] = gen_left;
+        if (REINF) s.ctrl[CTRL_RF_K] = rk;
         if (d_iters_done) *d_iters_done = executed;
     }
 }
@@ -425,6 +520,7 @@ static KArgs make_args(pdp_ctx* ctx) {
     A.g = ctx->g; A.s = ctx->s; A.trace = ctx->trace; A.trace_cap = ctx->trace_cap;
     A.stagger_c = PDP_STAGGER_C; A.stagger_v = PDP_STAGGER_V;
     A.dec_fraction = ctx->dec_fraction;
+    A.rf.coins = ctx->rf_coins; A.rf.p = ctx->rf_p; A.rf.pi = 0.f; A.rf.fresh = ctx->rf_fresh;
     A.rb.sol = nullptr; A.rb.is_sat = nullptr; A.rb.av = nullptr; A.rb.af = nullptr;
     if (ctx->rb_scratch) {
         const RbLayout l = rb_layout(ctx->g.V, ctx->g.F, ctx->g.B);
@@ -442,18 +538,32 @@ extern "C" int pdp_sp_run(pdp_ctx* ctx, const pdp_sp_params* params, int32_t* d_
     if (params->iterations < 0 || params->t_max < 0 || params->batch_replication < 0) { pdp_set_error("pdp_sp_run: negative parameter"); return PDP_ERR_ARG; }
     const int rep = params->batch_replication > 1 ? params->batch_replication : 1;
     if (ctx->g.B % rep != 0) { pdp_set_error("pdp_sp_run: batch size %lld not divisible by replication %d", (long long)ctx->g.B, rep); return PDP_ERR_ARG; }
+    const bool reinf = ctx->rf_coins != nullptr;
+    if (reinf && ctx->rf_upper + params->iterations > ctx->rf_n) {
+        pdp_set_error("pdp_sp_run: reinforce: %lld + %d iterations may read past the %d coins", (long long)ctx->rf_upper,
+                      params->iterations, ctx->rf_n);
+        return PDP_ERR_ARG;
+    }
     cudaStream_t stream = (cudaStream_t)stream_;
     KArgs A = make_args(ctx);
     pdp_sp_params prm = *params;
+    A.rf.pi = prm.pi;
     ctx->full_state_tracked = prm.full_state ? 1 : 0;
     ctx->last_pi = prm.pi;
     void* args[] = {&A, &prm, &d_iters_done};
     const bool frac = ctx->dec_fraction > 0.f;
-    const bool fast = ctx->g.blocked_ok && !prm.full_state && prm.pi == 0.f && !(prm.flags & 1);
-    if (fast) {
+    // (reinforce: the pi terms of the blocked passes are per variable, see k_sp_run)
+    const bool fast = ctx->g.blocked_ok && !prm.full_state && (prm.pi == 0.f || reinf) && !(prm.flags & 1);
+    if (reinf && !fast) {
+        void* kern = prm.full_state ? (void*)k_sp_run<false, true, 1, false, true> : (void*)k_sp_run<false, false, 1, false, true>;
+        int blocks = coop_blocks(ctx, kern);
+        if (blocks < 1) { pdp_set_error("pdp_sp_run: occupancy query failed"); return PDP_ERR_CUDA; }
+        PDP_CUDA_CHECK(cudaLaunchCooperativeKernel(kern, dim3(blocks), dim3(256), args, 0, stream));
+    } else if (fast) {
         // one or two CTAs per SM holding the whole shared memory: co-residency of the cooperative grid is guaranteed
         const int two = (ctx->g.ctas == 2) ? 1 : 0;
-        void* kern = frac ? (two ? (void*)k_sp_run<true, false, 2, true> : (void*)k_sp_run<true, false, 1, true>)
+        void* kern = reinf ? (two ? (void*)k_sp_run<true, false, 2, false, true> : (void*)k_sp_run<true, false, 1, false, true>)
+                   : frac ? (two ? (void*)k_sp_run<true, false, 2, true> : (void*)k_sp_run<true, false, 1, true>)
                           : (two ? (void*)k_sp_run<true, false, 2, false> : (void*)k_sp_run<true, false, 1, false>);
         const int smem = two ? SweepCfg<2>::kSmem : SweepCfg<1>::kSmem;
         const int threads = two ? SweepCfg<2>::kThreads : SweepCfg<1>::kThreads;
@@ -470,6 +580,7 @@ extern "C" int pdp_sp_run(pdp_ctx* ctx, const pdp_sp_params* params, int32_t* d_
         PDP_CUDA_CHECK(cudaLaunchCooperativeKernel(kern, dim3(blocks), dim3(256), args, 0, stream));
     }
     PDP_LAUNCH_CHECK(ctx);
+    if (reinf) { ctx->rf_upper += prm.iterations; ctx->rf_fresh = 0; }
     return PDP_OK;
 }
 
@@ -502,6 +613,18 @@ extern "C" int pdp_set_decimation_fraction(pdp_ctx* ctx, float fraction) {
     if (!ctx) { pdp_set_error("pdp_set_decimation_fraction: null context"); return PDP_ERR_ARG; }
     if (!valid_fraction(fraction)) { pdp_set_error("pdp_set_decimation_fraction: fraction %g not in [0, 1)", (double)fraction); return PDP_ERR_ARG; }
     ctx->dec_fraction = fraction;
+    return PDP_OK;
+}
+
+// model type `reinforce` in pdp_sp_run (pdp_b200.h)
+extern "C" int pdp_set_reinforce(pdp_ctx* ctx, const float* d_coins, int32_t n_coins, float decimation_probability) {
+    if (!ctx) { pdp_set_error("pdp_set_reinforce: null context"); return PDP_ERR_ARG; }
+    if (d_coins && (n_coins < 0 || decimation_probability != decimation_probability)) {
+        pdp_set_error("pdp_set_reinforce: %d coins, decimation probability %g", n_coins, (double)decimation_probability);
+        return PDP_ERR_ARG;
+    }
+    ctx->rf_coins = d_coins; ctx->rf_n = d_coins ? n_coins : 0; ctx->rf_p = decimation_probability;
+    ctx->rf_upper = 0; ctx->rf_fresh = 1;
     return PDP_OK;
 }
 

@@ -178,7 +178,11 @@ __global__ void k_load_state(pdp_graph g, pdp_state s, const float* __restrict__
         const int qp = g.p_qpos[p];
         s.qu[qp] = dq3[3 * e]; s.qs[qp] = dq3[3 * e + 1]; s.qd[qp] = dq3[3 * e + 2];
         const float eta = dfs2[2 * e];
-        s.eta[buf][g.p_vpos[p]] = eta; s.ext[p] = dfs2[2 * e + 1];
+        const float ext = dfs2[2 * e + 1];
+        s.eta[buf][g.p_vpos[p]] = eta; s.ext[p] = ext;
+        // reinforce runs the blocked passes only on forces that are uniform over each variable's edges (NaN counts as equal)
+        const float e0 = dfs2[2 * (int64_t)g.v_orig[g.var_ptr[g.c_var[g.v_cedge[p] & PDP_IDX_MASK] & PDP_IDX_MASK]] + 1];
+        if (!(ext == e0 || (ext != ext && e0 != e0))) s.ctrl[CTRL_RF_MIXED] = 1;
         // the blocked passes borrow the sign bits of the messages they read and write: messages that arrive with one (not
         // a probability) go through the generic passes until no message can carry a sign any more -- the first iteration
         // reads them, the second reads the q the first derived from them (a survey below 0 makes exp(opp) > 1 and q < 0);
@@ -206,6 +210,7 @@ __global__ void k_store_state(pdp_graph g, pdp_state s, float* out_q3, float* ou
         const int buf = last & 1;
         const int beg = g.var_ptr[i], end = g.var_ptr[i + 1];
         const bool rebuild = (!tracked) && last >= 1;
+        const bool stashed = last == s.rf_coin_iter[b];   // reinforce: the coin after the sweep of `last` changed the forces
         float P = 0.f, N = 0.f;
         const bool um = (last >= 2) && s.masked[b];
         const float avi = (float)s.av[i];
@@ -226,7 +231,7 @@ __global__ void k_store_state(pdp_graph g, pdp_state s, float* out_q3, float* ou
                 float y = L40_1m(s.eta[buf ^ 1][vp]);
                 if (um) y = y * (avi * (float)s.af[g.v_cls[p]]);
                 float uu;
-                sp_var_update(P, N, y, (g.v_cedge[p] & PDP_SIGN_BIT) ? -1.f : 1.f, s.ext[p], pi, uu, v, d);
+                sp_var_update(P, N, y, (g.v_cedge[p] & PDP_SIGN_BIT) ? -1.f : 1.f, stashed ? s.qs[p] : s.ext[p], pi, uu, v, d);
             }
             if (out_q3) { out_q3[3 * e] = u; out_q3[3 * e + 1] = v; out_q3[3 * e + 2] = d; }
             if (out_fs2) { out_fs2[2 * e] = s.eta[buf][vp]; out_fs2[2 * e + 1] = s.ext[p]; }
@@ -455,6 +460,7 @@ extern "C" int pdp_load_state(pdp_ctx* ctx, const float* d_prop_q3, const float*
     NEED(ctx, (d_dec_q3 && d_dec_fs2) || ctx->g.E == 0, "pdp_load_state: null argument");
     cudaStream_t stream = (cudaStream_t)stream_;
     PDP_CUDA_CHECK(cudaMemsetAsync(ctx->s.ctrl + CTRL_GEN_ITERS, 0, sizeof(int32_t), stream));
+    PDP_CUDA_CHECK(cudaMemsetAsync(ctx->s.ctrl + CTRL_RF_MIXED, 0, sizeof(int32_t), stream));
     if (ctx->g.E > 0) { k_load_state<<<GRID(ctx->g.E)>>>(ctx->g, ctx->s, d_dec_q3, d_dec_fs2, 0); PDP_LAUNCH_CHECK(ctx); }
     return PDP_OK;
 }
@@ -463,6 +469,7 @@ extern "C" int pdp_load_state_const(pdp_ctx* ctx, float qu, float qs, float qd, 
     NEED(ctx, true, "");
     cudaStream_t stream = (cudaStream_t)stream_;
     PDP_CUDA_CHECK(cudaMemsetAsync(ctx->s.ctrl + CTRL_GEN_ITERS, 0, sizeof(int32_t), stream));
+    PDP_CUDA_CHECK(cudaMemsetAsync(ctx->s.ctrl + CTRL_RF_MIXED, 0, sizeof(int32_t), stream));
     if (ctx->g.E > 0) { k_load_state_const<<<GRID(ctx->g.E)>>>(ctx->g, ctx->s, qu, qs, qd, eta, ext, 0); PDP_LAUNCH_CHECK(ctx); }
     return PDP_OK;
 }

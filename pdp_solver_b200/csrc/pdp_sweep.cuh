@@ -434,10 +434,12 @@ __device__ __forceinline__ void ph_var_score(int t, const pdp_graph& g, const pd
 // own sign NaN, and every message of the variable reads both sums -- `same` the one of its sign, `opp` the other.)
 // MULTI: the block holds several problems: frozen ones are left alone (PDP_SLOT_SKIP), those on the sticky-NaN path get
 // the sticky sign.
-template <int G, bool MULTI, bool MASKED, bool PREV>
+// REINF: reinforce (pdp_set_reinforce) with the external force uniform over each variable's edges: its pi terms are two
+// per-variable constants, read from the variable's first edge
+template <int G, bool MULTI, bool MASKED, bool PREV, bool REINF>
 __device__ __forceinline__ void ph_var_node(int t, const pdp_graph& g, const pdp_state& s, const BlkGeo& B, bool use_mask,
                                             bool em_set, float* __restrict__ PA, float* __restrict__ PB, uint32_t stk_blk,
-                                            KeyedReducer<StatAcc>& red, BlkStats& sm_st, bool local_stats) {
+                                            KeyedReducer<StatAcc>& red, BlkStats& sm_st, bool local_stats, float pi) {
     const int lane = t & 31;
     // shared-window address of plane PA / distance to PB, pinned in registers (left to itself the compiler re-derives the
     // window base from %cgaid at every use)
@@ -521,9 +523,17 @@ __device__ __forceinline__ void ph_var_node(int t, const pdp_graph& g, const pdp
                 }
             }
         }
-        float sb_pos, opp_pos, O_pos, sb_neg, opp_neg, O_neg;
-        sp_var_prepare(P, N, 1.f, sb_pos, opp_pos, O_pos);
-        sp_var_prepare(P, N, -1.f, sb_neg, opp_neg, O_neg);
+        float sb_pos, opp_pos, O_pos, sb_neg, opp_neg, O_neg, l_pos = 0.f, l_neg = 0.f;
+        if (REINF) {
+            const float e = s.ext[g.var_ptr[V.i]];
+            l_pos = L40(1.0f - pi * ((e == 1.f) ? 1.f : 0.f));    // same of s = +1, opp of s = -1
+            l_neg = L40(1.0f - pi * ((e == -1.f) ? 1.f : 0.f));   // same of s = -1, opp of s = +1
+            sp_var_prepare_pi(P, N, 1.f, l_neg, sb_pos, opp_pos, O_pos);
+            sp_var_prepare_pi(P, N, -1.f, l_pos, sb_neg, opp_neg, O_neg);
+        } else {
+            sp_var_prepare(P, N, 1.f, sb_pos, opp_pos, O_pos);
+            sp_var_prepare(P, N, -1.f, sb_neg, opp_neg, O_neg);
+        }
         bool made_nan = false;
 #pragma unroll
         for (int k = 0; k < 2; ++k) eq[k] = (k < npair) ? fw[32 * k] : 0u;
@@ -532,6 +542,7 @@ __device__ __forceinline__ void ph_var_node(int t, const pdp_graph& g, const pdp
         uint32_t nan_or = 0u;
         auto fin_row = [&](uint32_t en, float y) {
             const bool neg = (en >> 15) != 0u;
+            if (REINF) return sp_var_finish_pi(neg ? sb_neg : sb_pos, neg ? l_neg : l_pos, neg ? opp_neg : opp_pos, neg ? O_neg : O_pos, y);
             return sp_var_finish(neg ? sb_neg : sb_pos, neg ? opp_neg : opp_pos, neg ? O_neg : O_pos, y);
         };
         for (int k0 = 0; k0 < npair; k0 += 2) {
@@ -713,7 +724,7 @@ __device__ __forceinline__ void blk_clause_pass(const KArgs& A, int r, bool use_
 
 // variable pass of iteration t: the decimator statistics of eta(t) [buffer r^1] against eta(t-1)
 // [buffer r], and q(t) [C-layout, in place] from eta(t-1)
-template <int CTAS>
+template <int CTAS, bool REINF>
 __device__ __forceinline__ void blk_var_pass(const KArgs& A, int r, bool use_mask, bool has_prev, bool em_set, unsigned char* smem, int sm_rank, BulkBar& bb) {
     using Cfg = SweepCfg<CTAS>;
     constexpr int NT = Cfg::kThreads, CAP = Cfg::kAdjCap;
@@ -772,7 +783,7 @@ __device__ __forceinline__ void blk_var_pass(const KArgs& A, int r, bool use_mas
         if (local_stats) stats_slots_reset(sm_st, tid, B.b1 - B.b0 + 1);
         const bool masked = (use_mask || em_set) && (B.multi() || s.masked[B.b0]);
         const uint32_t stk_blk = (!B.multi() && s.nanflag[B.b0]) ? 0x80000000u : 0u;
-        const bool scoring = s.want_score[B.b0] || s.want_score[B.b1];
+        const bool scoring = !REINF && (s.want_score[B.b0] || s.want_score[B.b1]);
         MaskWords MW; MW.m0 = 0u; MW.m1 = 0u;
         if (masked) MW = ph_mask_fetch<NT>(tid, g.vmask, B);
         mbar_wait_cta(bb.bar, bb.parity);
@@ -784,7 +795,7 @@ __device__ __forceinline__ void blk_var_pass(const KArgs& A, int r, bool use_mas
         // overwrites them); its own loop, so that the node phase's code is the same with and without it
         if (scoring) { ph_var_score<NT>(tid, g, s, B, PA); __syncthreads(); }
         {
-#define VN_CALL(MU, MA, PR) ph_var_node<NT, MU, MA, PR>(tid, g, s, B, use_mask, em_set, PA, PB, stk_blk, red, sm_st, local_stats)
+#define VN_CALL(MU, MA, PR) ph_var_node<NT, MU, MA, PR, REINF>(tid, g, s, B, use_mask, em_set, PA, PB, stk_blk, red, sm_st, local_stats, A.rf.pi)
             if (B.multi()) { if (has_prev) VN_CALL(true, true, true); else VN_CALL(true, true, false); }
             else if (masked) { if (has_prev) VN_CALL(false, true, true); else VN_CALL(false, true, false); }
             else { if (has_prev) VN_CALL(false, false, true); else VN_CALL(false, false, false); }

@@ -279,6 +279,20 @@ class Context(object):
         self._check(self._L.pdp_set_conflict_rollback(self._h, _ptr(scratch), nbytes), "pdp_set_conflict_rollback")
         self._rb_scratch = scratch
 
+    def set_reinforce(self, coins, decimation_probability=0.5):
+        """Model type `reinforce` in sp_run (include/pdp_b200.h, pdp_set_reinforce): iteration k of the runs from here on
+        draws coins[k] (fp32 [n] on the device) and, when it is < decimation_probability, sets every active problem's
+        external forces to the signs of its SP biases; the retire test and the predictor replace the decimation.  coins=None
+        turns the mode off.  The context keeps a reference to the coins while the mode is on."""
+        if coins is None:
+            self._check(self._L.pdp_set_reinforce(self._h, None, 0, 0.0), "pdp_set_reinforce")
+            self._rf_coins = None
+            return
+        c = _f32(coins, self.device).reshape(-1).contiguous()
+        self._check(self._L.pdp_set_reinforce(self._h, _ptr(c), int(c.numel()), float(decimation_probability)),
+                    "pdp_set_reinforce")
+        self._rf_coins = c
+
     def rollbacks(self):
         """(count int32 [B], iteration of the last rollback int32 [B], 0 = none) since pdp_reset"""
         count, last = self._new(self.B, dtype=torch.int32), self._new(self.B, dtype=torch.int32)

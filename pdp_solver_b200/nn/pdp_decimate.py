@@ -58,6 +58,30 @@ def check_conflict_rollback(conflict_rollback, fraction):
     return conflict_rollback
 
 
+def draw_coins(T, device):
+    """The coins of T reinforce iterations drawn before a fused run: T separate torch.rand(1) draws on `device`, the values
+    the step loop draws one per iteration (ReinforceDecimator._coin).  Returns (coins [T], the generator state before the
+    draws) for settle_coins."""
+    device = torch.device(device)
+    state = torch.cuda.get_rng_state(device) if device.type == "cuda" else torch.get_rng_state()
+    coins = torch.empty(int(T), dtype=torch.float32, device=device)
+    for t in range(int(T)):
+        torch.rand(1, out=coins[t:t + 1])
+    return coins, state
+
+
+def settle_coins(state, done, device):
+    """Leaves the generator of `device` where a step loop that ran `done` iterations leaves it: back to `state` (from
+    draw_coins), then `done` single draws again.  The draws that follow the run (WalkSAT) are then the step loop's."""
+    device = torch.device(device)
+    if device.type == "cuda":
+        torch.cuda.set_rng_state(state, device)
+    else:
+        torch.set_rng_state(state)
+    for _ in range(int(done)):
+        torch.rand(1, device=device)
+
+
 class NeuralDecimator(nn.Module):
     """The neural (non-greedy) decimator of `p-nd-np` / `np-nd-np` (reference pdp_decimate.py:21-100): one GRU
     cell per message direction over the edges; same sub-module names (state-dict compatible).  The GRU cells run on the
@@ -218,7 +242,11 @@ class ReinforceDecimator(nn.Module):
     """The (distributed) Reinforce decimator of model type `reinforce` (reference pdp_decimate.py:189-250): no variable
     is fixed; with probability `decimation_probability` per iteration (one batch-global coin, pdp_decimate.py:218)
     every edge's external force becomes the sign of its variable's SP bias, which the propagator and scorer feed
-    back through their pi terms.  Problems whose surveys moved by at most 0.01 are retired."""
+    back through their pi terms.  Problems whose surveys moved by at most 0.01 are retired.
+
+    Inside ReinforceSurveyPropagatorSolver.forward the whole loop runs in the persistent kernel (pdp_set_reinforce) with
+    coins drawn beforehand (draw_coins / settle_coins), unless `_coin_source` is set or the caller's termination callback
+    is its own: then forward() below runs once per iteration."""
 
     _draws_per_iteration = True       # one coin per iteration: the solver loop must stop exactly where the reference stops
 

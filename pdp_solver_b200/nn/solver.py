@@ -5,8 +5,9 @@ the reference; underneath, the batch lives in a device `Context` (CSR/CSC instea
 matrices) and the whole propagate -> decimate -> predict loop, the CNF check, unit propagation /
 peeling and WalkSAT run as hand-written sm_100a kernels behind the C ABI of libpdp_b200.so.
 
-Scope (SURVEY.md section 8): the classical model types `p-d-p` (SurveyPropagatorSolver) and `walk-sat`
-(WalkSATSolver) run entirely in the library's kernels (one persistent launch for the whole loop).  The neural
+Scope (SURVEY.md section 8): the classical model types `p-d-p` (SurveyPropagatorSolver), `walk-sat` (WalkSATSolver) and
+`reinforce` (ReinforceSurveyPropagatorSolver) run entirely in the library's kernels (one persistent launch for the whole
+loop).  The neural
 model types `p-nd-np` (NeuralSurveyPropagatorSolver) and `np-nd-np` (NeuralPropagatorDecimatorSolver) run the
 reference's iteration structure step by step: message arithmetic, segmented sums, CNF check, simplification and
 WalkSAT are the library's kernels, the dense layers (Linear adaptors, GRU cells, MLPs) are library GEMMs through
@@ -219,9 +220,14 @@ class PropagatorDecimatorSolverBase(nn.Module):
 
         propagator_state = decimator_state = None
         if self._propagator is not None and self._decimator is not None:
+            fused = check_termination is None or _is_standard_termination(check_termination)
             if isinstance(self._decimator, pdp_decimate.SequentialDecimator) and \
                     isinstance(self._decimator._scorer, pdp_predict.SurveyScorer):
                 propagator_state, decimator_state = self._forward_core(
+                    init_propagator_state, init_decimator_state, sat_problem, iteration_num, check_termination)
+            elif isinstance(self._decimator, pdp_decimate.ReinforceDecimator) and fused and \
+                    self._decimator._coin_source is None:
+                propagator_state, decimator_state = self._forward_core_reinforce(
                     init_propagator_state, init_decimator_state, sat_problem, iteration_num, check_termination)
             else:
                 propagator_state, decimator_state = self._forward_core_stepwise(
@@ -287,6 +293,29 @@ class PropagatorDecimatorSolverBase(nn.Module):
             self.last_iterations = torch.tensor([done], dtype=torch.int32, device=ctx.device)
         sat_problem._edge_mask_set = iteration_num > 0
         # the final message states are exported on first use (the predict path never looks at them)
+        state = _DeferredState(ctx)
+        return state, state
+
+    def _forward_core_reinforce(self, init_propagator_state, init_decimator_state, sat_problem, iteration_num,
+                                check_termination):
+        """reference solver.py:355-386 for model type `reinforce` in one persistent kernel (pdp_set_reinforce): the coins
+        of all T iterations are drawn before the launch, and the generator is left where the step loop leaves it."""
+        ctx = sat_problem._ctx
+        dec = self._decimator
+        ctx.load_state(init_propagator_state, init_decimator_state[:2])
+        T = int(iteration_num)
+        coins, rng_state = pdp_decimate.draw_coins(T, ctx.device)
+        ctx.set_reinforce(coins, dec._decimation_probability)
+        try:
+            # the blocked passes where the batch allows; the returned [E,3] state is re-derived on export with the forces the
+            # last sweep read (pdp_set_reinforce)
+            done = ctx.sp_run(T, 0.0, 0, check_termination is not None, sat_problem._batch_replication,
+                              self._propagator.pi_value(), sync=True)
+        finally:
+            ctx.set_reinforce(None)
+        pdp_decimate.settle_coins(rng_state, done, ctx.device)
+        self.last_iterations = torch.tensor([done], dtype=torch.int32, device=ctx.device)
+        sat_problem._edge_mask_set = T > 0
         state = _DeferredState(ctx)
         return state, state
 
@@ -442,8 +471,10 @@ class NeuralSurveyPropagatorSolver(PropagatorDecimatorSolverBase):
 
 class ReinforceSurveyPropagatorSolver(PropagatorDecimatorSolverBase):
     """The classical Reinforce solver, model type `reinforce` (reference solver.py:598-610): SP with the pi
-    reinforcement term, external forces set from the SP biases under a batch-global coin, no variable fixing.  Runs
-    step by step on the library's stateless operators (pdp_sp_step, pdp_score, pdp_edge_aggregate, pdp_cnf_eval)."""
+    reinforcement term, external forces set from the SP biases under a batch-global coin, no variable fixing.  With no
+    termination callback or the trainer's, the whole loop runs in one persistent kernel (pdp_set_reinforce); a caller's own
+    callback, or a coin source set on the decimator, runs it step by step on the library's stateless operators
+    (pdp_sp_step, pdp_score, pdp_edge_aggregate, pdp_cnf_eval)."""
 
     def __init__(self, device, name, pi=0.1, decimation_probability=0.5, local_search_iterations=0, epsilon=0.05):
         super(ReinforceSurveyPropagatorSolver, self).__init__(
