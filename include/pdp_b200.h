@@ -117,7 +117,9 @@ int pdp_edge_aggregate(pdp_ctx* ctx, int32_t by_variable, const float* d_state, 
  *   of MessageAggregator.forward, reference pdp/nn/util.py:51-77, and of the classifiers (act = 0).
  * pdp_edge_gru_forward: out[rows, hidden] = torch.nn.GRUCell([x1|x2], h), blended with h where row_mask is 0 -- the two cells of
  *   NeuralDecimator.forward, reference pdp/nn/pdp_decimate.py:51-87.  A pass holds n_blk * n_mma / 4 hidden units, four
- *   accumulator columns each (r, z, W_in x, W_hn h of the unit side by side; bias in the same order).  out must not alias h. */
+ *   accumulator columns each (r, z, W_in x, W_hn h of the unit side by side; bias in the same order).  out must not alias h.
+ * Alignment: d_x1, d_x2, d_x3, d_h, d_out and d_row_mask need only be 4-byte (float) aligned; rows and arrays that are 8- or
+ * 16-byte aligned take wider accesses, the others element-by-element ones.  d_w_img must be 16-byte aligned (PDP_ERR_ARG). */
 int pdp_edge_nn_swizzle(void);   /* 1: the weight images use the 64-byte swizzled operand layout (nn/tensor_ops.py follows) */
 int pdp_edge_nn_chunk_k(void);   /* K elements per chunk of the weight images (16): the host side tiles W accordingly */
 int pdp_edge_mlp_forward(const float* d_x1, int32_t k1, const float* d_x2, int32_t k2, const float* d_x3, int32_t k3, int64_t rows,

@@ -424,12 +424,14 @@ __global__ void __launch_bounds__(kThreads, 1) k_edge_nn(const __grid_constant__
     if (warp >= 8 && warp < 16) {
         // ---------------- epilogue: thread <-> accumulator lane = row of the tile; two warps per lane quadrant, each takes
         //                  every other group of 16 columns.  A thread's 16 results are contiguous in its output row: 64-bit
-        //                  accesses (rows are 8-byte aligned when their length is even), two full sectors per thread
+        //                  accesses (rows are 8-byte aligned when their length is even and the array starts 8-byte aligned),
+        //                  two full sectors per thread.  The caller's arrays need only be 4-byte aligned: a view that starts
+        //                  one float into its storage takes the element-by-element path.  (h_old is null for LINEAR.)
         const int q = warp & 3;                      // lane quadrant this warp may read (warp index mod 4)
         const int hh = (warp - 8) >> 2;              // which half of the column groups
         const int r = q * 32 + lane;
         const uint32_t tlane0 = tmem_base + ((uint32_t)(q * 32) << 16);
-        const bool vec2 = !(P.n_out & 1);
+        const bool vec2 = !(P.n_out & 1) && !(((uintptr_t)P.out | (uintptr_t)P.h_old) & 7);
         uint32_t acc_ph[2] = {0u, 0u};
         int ab = 0;
         // LINEAR: a tile's output rows are consecutive in global memory, so the warps collect them in a shared-memory image of
